@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the TensoFlow hot path on B200 (see the contract in DESIGN.md).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Default workload = BASELINE.json configs[1]: shape stage, VM field 512^3 (C=36, H=256,
 A=128, 3 mip levels), 8192-ray batch x 512 samples, forward + backward
@@ -134,7 +134,7 @@ def build_shape(cfg, device, seed=0):
 
 
 def shape_step(field, variance, rays, cfg, loss_scale=1.0):
-    """fwd + bwd of the shape-stage hot path on one ray batch (already on the device)."""
+    """fwd + bwd of the shape-stage hot path on one ray batch (already on the device): (loss, samples, render outputs)."""
     from tensoflow_b200 import synthetic
     from tensoflow_b200.shape_renderer import render_core, charbonnier
     t0, t1, idx = synthetic.uniform_samples(rays["rays_o"], rays["dirs"], field.aabb, cfg["samples"])
@@ -142,7 +142,29 @@ def shape_step(field, variance, rays, cfg, loss_scale=1.0):
                       t0, t1, idx, cos_anneal_ratio=1.0)
     loss = charbonnier(out["ray_rgb"], rays["rgbs"]).mean() + 0.1 * out["gradient_error"].mean()
     (loss * loss_scale).backward()
-    return loss.detach(), int(idx.shape[0])
+    return loss.detach(), int(idx.shape[0]), out
+
+
+DUMP_SAMPLE = 1 << 18      # elements written of a larger array
+
+
+def dump_array(t):
+    """`t` as a float32 host array: whole when it has at most DUMP_SAMPLE elements, otherwise DUMP_SAMPLE elements of its
+    flattened values at sorted indices drawn from a fixed seed (the same indices in every run of the same configuration)."""
+    t = t.detach()
+    if t.numel() > DUMP_SAMPLE:
+        idx = torch.randint(t.numel(), (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(0)).sort().values
+        t = t.reshape(-1)[idx.to(t.device)]
+    return t.float().cpu().numpy()
+
+
+def step_outputs(loss, out, field, variance):
+    """What one training step hands its caller: the loss, the render outputs and the parameter gradients (host arrays)."""
+    arrays = {"loss": dump_array(loss)}
+    arrays.update({k: dump_array(v) for k, v in out.items() if torch.is_tensor(v)})
+    arrays.update({f"grad.{n}": dump_array(p.grad) for n, p in field.named_parameters() if p.grad is not None})
+    arrays["grad.variance"] = dump_array(variance.grad)
+    return arrays
 
 
 def cpu_baseline_shape(cfg, n_rays, iters, threads):
@@ -352,7 +374,7 @@ def run_ours(args):
     # ---- warm-up ----
     for i in range(max(args.warmup, 3)):
         zero_grads()
-        _, n_samples = shape_step(field, variance, resident[i % n_batches], cfg, 1.0 / world)
+        _, n_samples, _ = shape_step(field, variance, resident[i % n_batches], cfg, 1.0 / world)
         allreduce_grads()
     torch.cuda.synchronize()
 
@@ -400,12 +422,19 @@ def run_ours(args):
         return ms, clocks, launches, tot, kern
 
     # ---- device-resident timing (value) ----
+    last = {}
+
     def step_resident(i):
         zero_grads()
-        shape_step(field, variance, resident[i % n_batches], cfg, 1.0 / world)
+        loss, _, out = shape_step(field, variance, resident[i % n_batches], cfg, 1.0 / world)
         allreduce_grads()
+        if args.dump_outputs and i == args.steps - 1:     # only the last step's outputs are kept alive past their step
+            last.update(loss=loss, out=out)
 
     ms, clocks, launches, ktimes, kern = timed(step_resident, True)
+    # copied out before the next timed window overwrites the gradients (in place in the flat bucket when world > 1)
+    dumped = step_outputs(last["loss"], last["out"], field, variance) if (args.dump_outputs and rank == 0) else None
+    last.clear()
 
     # ---- end-to-end timing: pinned host rays -> H2D -> step -> D2H loss ----
     losses = []
@@ -413,7 +442,7 @@ def run_ours(args):
     def step_e2e(i):
         zero_grads()
         rays = step_device(i)
-        loss, _ = shape_step(field, variance, rays, cfg, 1.0 / world)
+        loss, _, _ = shape_step(field, variance, rays, cfg, 1.0 / world)
         allreduce_grads()
         losses.append(float(loss.cpu()))   # D2H read of the step's result
 
@@ -487,6 +516,11 @@ def run_ours(args):
         "gpu_launches": launches, "clocks": clocks, "loss": losses[-1] if losses else None,
         "check": check, "secondary": secondary,
     }
+    if dumped is not None:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -505,7 +539,14 @@ def main():
     ap.add_argument("--check-rays", type=int, default=64, help="rays of the parity check against the oracle (0 = off)")
     ap.add_argument("--no-secondary", action="store_true", help="skip the config-3 / module-path lines of `secondary`")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the loss, render outputs and parameter gradients of the last timed step "
+                         "as DIR/<name>.npy (float32; an array of more than 2^18 elements as a fixed seeded sample of them)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -3,6 +3,9 @@
 
     python oracle/build_ref.py [--force]
 
+The package build (__graft_entry__.build) does not run this: run it by hand before oracle/gen_golden_prefilter.py, which
+loads whatever library oracle/_ref/ holds.
+
 oracle/_ref/libref_cubemap.so = oracle/ref_cubemap_shim.cu (C-ABI launchers, ours)
                                 + /root/reference/network/renderutils/c_src/{cubemap.cu (included by the shim), common.cpp}
 built with plain nvcc for sm_100a (the reference's own build goes through torch.utils.cpp_extension and its torch binding,

@@ -11,8 +11,10 @@ torch_scatter / raytracing) are the shim's restatements: that part stays "parity
 """
 from __future__ import annotations
 
+import glob
 import os
 import sys
+import zlib
 
 import numpy as np
 import torch
@@ -26,14 +28,35 @@ def _np(d):
     return {k: v.detach().cpu().numpy() for k, v in d.items()}
 
 
+PART_BYTES = 900_000       # a fixture larger than this is written as <stem>.0.npz, <stem>.1.npz, ... (each file below 1 MB)
+
+
 def _save(name, **groups):
     flat = {}
     for g, d in groups.items():
         for k, v in d.items():
             flat[f"{g}/{k}"] = v
+    write_fixture(name, flat)
+
+
+def write_fixture(name, flat):
+    """Compressed arrays in one file, or in parts of at most ~PART_BYTES each (tests/test_golden.py load() joins them)."""
     os.makedirs(GOLD, exist_ok=True)
-    np.savez_compressed(os.path.join(GOLD, name), **flat)
-    print(name, f"{os.path.getsize(os.path.join(GOLD, name)) / 1e6:.2f} MB", len(flat), "arrays")
+    stem = os.path.join(GOLD, name[:-4])
+    for old in glob.glob(stem + ".npz") + glob.glob(stem + ".[0-9].npz"):
+        os.remove(old)
+    parts, size = [{}], 0
+    for k, v in flat.items():
+        n = len(zlib.compress(np.ascontiguousarray(v).tobytes()))
+        if parts[-1] and size + n > PART_BYTES:
+            parts.append({})
+            size = 0
+        parts[-1][k] = v
+        size += n
+    paths = [stem + ".npz"] if len(parts) == 1 else [f"{stem}.{i}.npz" for i in range(len(parts))]
+    for path, part in zip(paths, parts):
+        np.savez_compressed(path, **part)
+        print(os.path.basename(path), f"{os.path.getsize(path) / 1e6:.2f} MB", len(part), "arrays")
 
 
 def gen_tensosdf():

@@ -3,6 +3,7 @@ REFERENCE's own classes (network/fields.py TensoSDF + MCShadingNetwork, network/
 TensoFlow) in the build container.  CPU tests pin the oracle to them; GPU tests pin the CUDA
 path (through the C ABI) to the same reference outputs.  Tolerances: outputs 1e-4 relative,
 parameter gradients 1e-3 relative (BASELINE.json north star), rel err = max|a-b|/max|b|."""
+import glob
 import os
 
 import numpy as np
@@ -16,11 +17,14 @@ GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 def load(name):
-    z = np.load(os.path.join(GOLD, name))
+    """name.npz, or its parts name.0.npz, name.1.npz, ... (oracle/gen_golden.py splits fixtures into files below 1 MB)."""
+    stem = os.path.join(GOLD, name[:-4])
     out = {}
-    for k in z.files:
-        g, key = k.split("/", 1)
-        out.setdefault(g, {})[key] = torch.from_numpy(z[k])
+    for path in sorted(glob.glob(stem + ".[0-9].npz")) or [stem + ".npz"]:
+        z = np.load(path)
+        for k in z.files:
+            g, key = k.split("/", 1)
+            out.setdefault(g, {})[key] = torch.from_numpy(z[k])
     return out
 
 

@@ -1,10 +1,10 @@
-"""CPU tests of the oracle itself: texture semantics, autograd consistency, and (where the
-reference tree is present) agreement with the reference's own classes through the shim."""
-import pytest
+"""CPU tests of the oracle itself: texture semantics, autograd consistency, values pinned to stored outputs of seeded inputs
+(tests/golden/pins_oracle_cpu.npz, oracle/golden_pins.py) and, where the original project's source tree is present,
+agreement with its own classes through the shim."""
 import torch
 import torch.nn.functional as F
 
-from oracle import torch_oracle as O, ref_shim
+from oracle import golden_pins, torch_oracle as O, ref_shim
 from conftest import rel_err
 
 
@@ -58,8 +58,10 @@ def test_sphere_init_is_a_sphere():
     assert abs(float(g.norm(dim=-1).mean()) - 0.99) < 0.05
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present")
 def test_oracle_matches_reference_tensosdf():
+    golden_pins.check("test_oracle_cpu", "tensosdf", PINS["tensosdf"]())
+    if not ref_shim.available():
+        return
     ref_shim.install()
     import network.fields as RF
     torch.manual_seed(0)
@@ -86,11 +88,13 @@ def test_oracle_matches_reference_tensosdf():
         assert rel_err(q.grad, p.grad) < 1e-5, n
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present")
 def test_surface_refine_matches_reference_material_renderer():
     """oracle surface_refine == the reference's own MaterialRenderer.trace_sdf_with_mesh (materialRenderer.py:315-343) driven by
     a stand-in tracer (the mesh depth is an input of both)."""
     import types
+    golden_pins.check("test_oracle_cpu", "surface_refine", PINS["surface_refine"]())
+    if not ref_shim.available():
+        return
     ref_shim.install()
     import network.fields as RF
     import network.materialRenderer as MR
@@ -126,3 +130,42 @@ def test_surface_refine_matches_reference_material_renderer():
     assert rel_err(dep, depth[hit]) < 1e-6
     assert rel_err(pts, inters[hit]) < 1e-6
     assert float((n - normals[hit]).abs().max()) < 1e-4
+
+
+# ------------------------------------------------------------------ pinned values (seeded oracle fields and inputs)
+def _tensosdf_values():
+    torch.manual_seed(0)
+    G = torch.tensor([16, 16, 16]); aabb = torch.tensor([[-1., -1, -1], [1, 1, 1]])
+    f = O.TensoSDF(G, aabb, sdf_n_comp=8, sdf_dim=32, app_dim=16, init_n_levels=1)
+    f.upsample_volume_grid(torch.tensor([33, 33, 33])); f.upsample_volume_grid(torch.tensor([66, 66, 66]))
+    with torch.no_grad():
+        for p in list(f.sdf_plane) + list(f.sdf_line):
+            p.add_(0.05 * torch.randn_like(p))
+    x = torch.rand(777, 3) * 2.2 - 1.1
+    lv = torch.rand(777, 1) * 4 - 1
+    out = f(x, lv)
+    g, h = f.gradient(x, lv, training=True, sdf=out[:, :1])
+    (out.sum() + g.sum()).backward()
+    return [("out", out, 1e-6), ("grad", g, 1e-5), ("hess", h, 1e-4)] + [(f"d_{n}", p.grad, 1e-5) for n, p in f.named_parameters()]
+
+
+def _surface_refine_values():
+    from oracle import torch_oracle_renderer as RR
+    torch.manual_seed(0)
+    G = torch.tensor([32, 32, 32]); aabb = torch.tensor([[-1., -1, -1], [1, 1, 1]])
+    f = O.TensoSDF(G, aabb, sdf_n_comp=8, sdf_dim=32, app_dim=16, init_n_levels=1)
+    with torch.no_grad():
+        for p in list(f.sdf_plane) + list(f.sdf_line):
+            p.add_(5e-3 * torch.randn_like(p))
+    pn = 200
+    o = F.normalize(torch.randn(pn, 3), dim=-1) * 2.0
+    d = F.normalize((torch.rand(pn, 3) - 0.5) * 0.2 - o, dim=-1)
+    m_depth = 2.0 - 0.22 + 0.05 * torch.randn(pn, 1)
+    hit = torch.rand(pn) < 0.8
+    unit = torch.mean((aabb[1] - aabb[0]) / (G - 1))
+    radius = (aabb[1] - aabb.mean(0)).mean()
+    dep, pts, n = RR.surface_refine(f, 20.0, o[hit], d[hit], m_depth[hit], float(unit), float(radius), 32, 9)
+    return [("depth", dep, 1e-6), ("points", pts, 1e-6), ("normals", n, 1e-4)]
+
+
+PINS = {"tensosdf": _tensosdf_values, "surface_refine": _surface_refine_values}

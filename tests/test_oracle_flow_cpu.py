@@ -1,10 +1,11 @@
 """CPU tests of the TensoFlow oracle: self-consistency identities (the reference's only
-known-answer material for the flow, SURVEY 8c) and, where the reference tree is present,
-exact agreement with the reference's own network/flow.py through the shim."""
+known-answer material for the flow, SURVEY 8c), values pinned to stored outputs of seeded inputs
+(tests/golden/pins_oracle_flow_cpu.npz, oracle/golden_pins.py) and, where the original project's source tree is present,
+exact agreement with its own network/flow.py through the shim."""
 import pytest
 import torch
 
-from oracle import torch_oracle_mat as OM, ref_shim
+from oracle import golden_pins, torch_oracle_mat as OM, ref_shim
 
 
 def test_spline_round_trip_and_unit_mass():
@@ -39,8 +40,10 @@ def test_sample_density_consistency():
     assert float((lj + lq).abs().max()) < 2e-2           # reference: <= 8e-3 (SURVEY appendix D-5)
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present")
 def test_oracle_matches_reference_tensoflow():
+    golden_pins.check("test_oracle_flow_cpu", "tensoflow", PINS["tensoflow"]())
+    if not ref_shim.available():
+        return
     ref_shim.install()
     import network.flow as RFL
     torch.manual_seed(0)
@@ -81,13 +84,15 @@ def test_oracle_matches_reference_tensoflow():
             assert torch.allclose(p.grad, gm[n].grad, rtol=0, atol=0), n
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present")
 @pytest.mark.parametrize("version", ["direction", "sphere_direction"])
 def test_oracle_outer_mlp_lights_match_reference(version):
     """MLP outer lights (reference fields.py:716-721, 913-928; `outer_light_version: direction` is the reference default and the
     setting of 8 shipped material configs): oracle predict_outer_lights == the reference class's, same weights."""
     import torch.nn.functional as F
     from conftest import rel_err
+    golden_pins.check("test_oracle_flow_cpu", f"outer_lights_{version}", PINS[f"outer_lights_{version}"]())
+    if not ref_shim.available():
+        return
     ref_shim.install()
     import network.fields as RF
     from oracle import torch_oracle_mc as MC
@@ -108,3 +113,42 @@ def test_oracle_outer_mlp_lights_match_reference(version):
     a = ref.predict_outer_lights(pts, dirs)
     b = mine.predict_outer_lights(pts, dirs)
     assert a.shape == (n, 3) and rel_err(b, a) < 1e-6
+
+
+# ------------------------------------------------------------------ pinned values (seeded oracle modules and inputs)
+def _tensoflow_values():
+    torch.manual_seed(0)
+    f = OM.TensoFlow(torch.tensor([[-1., -1, -1], [1, 1, 1]]), gridSize=(16, 16, 16))
+    with torch.no_grad():
+        for p in f.nis_plane:
+            p.mul_(1000)
+    pn, sn = 30, 64
+    pts, va, rough = torch.rand(pn, 3) * 1.8 - 0.9, torch.rand(pn, 2), torch.rand(pn, 1)
+    a_eval, la_eval = f.sample(pts, va, rough, sn, None)
+    shift = torch.rand(pn, sn, 1)
+    a, la = f.sample(pts, va, rough, sn, shift)
+    rid = torch.sort(torch.randint(0, pn, (200,)))[0]
+    z, lq = f(pts, va, rough, torch.rand(200, 2), rays_id=rid)
+    lq.sum().backward()
+    return ([("angles_eval", a_eval, 0), ("logj_eval", la_eval, 0), ("angles", a, 0), ("logj", la, 0), ("z", z, 0), ("logq", lq, 0)]
+            + [(f"d_{n}", p.grad, 0) for n, p in f.named_parameters() if p.grad is not None])
+
+
+def _outer_light_values(version):
+    import torch.nn.functional as F
+    from oracle import torch_oracle_mc as MC
+    torch.manual_seed(3)
+    m = MC.MCShadingNetwork(MC.analytic_sphere_tracer(0.45), torch.tensor([[-1., -1, -1], [1, 1, 1]]), gridSize=(8, 8, 8),
+                            flow_grid=(16, 16, 16), outer_light_version=version)
+    with torch.no_grad():
+        for p in m.outer_light.parameters():
+            p.add_(0.1 * torch.randn_like(p))
+    n = 500
+    pts = F.normalize(torch.randn(n, 3), dim=-1) * torch.rand(n, 1)
+    pts[:20] = F.normalize(pts[:20], dim=-1) * (0.999 + 0.0019 * torch.rand(20, 1))
+    dirs = F.normalize(torch.randn(n, 3), dim=-1)
+    return [("lights", m.predict_outer_lights(pts, dirs), 1e-6)]
+
+
+PINS = {"tensoflow": _tensoflow_values, "outer_lights_direction": lambda: _outer_light_values("direction"),
+        "outer_lights_sphere_direction": lambda: _outer_light_values("sphere_direction")}
