@@ -146,7 +146,10 @@ class ShapeRenderer(nn.Module):
         w = alpha * torch.cumprod(torch.cat([torch.ones_like(alpha[:, :1]), 1. - alpha + 1e-7], -1), -1)[:, :-1]
         return sample_pdf_det(z, w, n_imp).detach()
 
-    def sample_ray(self, o, d, near, far, radiis, rays_cos, t_rand=None):     # shapeRenderer.py:871-932
+    def sample_ray(self, o, d, near, far, radiis, rays_cos, t_rand=None, rounds=None):     # shapeRenderer.py:871-932
+        """rounds: optional list; (t, sdf) of the depth lists is appended to it after the coarse samples and after every
+        upsampling round (sdf None after the last round, whose SDF the reference does not query).  The return value does
+        not depend on it."""
         c = self.cfg
         f = self.sdf_network
         ns = c['n_samples']
@@ -161,6 +164,8 @@ class ShapeRenderer(nn.Module):
             pts = o[:, None, :] + d[:, None, :] * t[..., :, None]
             lvl = torch.log2(O.compute_ball_radii(t[..., :, None], radiis[:, None, :], rays_cos[:, None, :]) / self.base_radii)
             sdf = f.sdf(pts.reshape(-1, 3), lvl.reshape(-1, 1)).reshape(t.shape)
+            if rounds is not None:
+                rounds.append((t.detach().clone(), sdf.clone()))
             for i in range(c['up_sample_steps']):
                 if c['clip_sample_variance']:
                     inv_s = torch.clamp(self.inv_s(), max=64 * 2 ** i)
@@ -174,6 +179,8 @@ class ShapeRenderer(nn.Module):
                     new_sdf = f.sdf(pts.reshape(-1, 3), lvl.reshape(-1, 1)).reshape(new_t.shape)
                     sdf = torch.gather(torch.cat([sdf, new_sdf], dim=-1), 1, index)
                 t = t_all
+                if rounds is not None:
+                    rounds.append((t.detach().clone(), sdf.clone() if i + 1 != c['up_sample_steps'] else None))
         dists = t[..., 1:] - t[..., :-1]
         dists = torch.cat([dists, dists[..., -1:]], -1)
         mid = t + dists * 0.5

@@ -7,7 +7,9 @@
 //   sampler_merge    : warp per ray: the last merge (the reference skips the SDF of the last round)
 //   sampler_finalize : warp per ray: interval ends, mid points, inside-box mask -> per-ray counts, then (second call) the
 //                      packed t_starts / t_ends / ray_indices in ray order
-// Depth lists live in [R, S_max] rows (sorted, first n valid).  HBM-bound: ~ (8 n + 100) B per ray and round.
+// Depth lists live in [R, S_max] rows (first n valid), ascending after every merge.  Before the first merge a ray that misses
+// the box holds a descending coarse list (tmin > tmax after the [near, far] clip), as the reference does; round 0 upsamples
+// it in that order.  HBM-bound: ~ (8 n + 100) B per ray and round.
 #include "common.cuh"
 
 namespace {
@@ -58,29 +60,37 @@ __global__ void __launch_bounds__(256) sampler_init_kernel(InitParams p) {
     p.level[i] = mip_level(z, p.radiis[r], p.rays_cos[r], p.base_radii);
 }
 
-// ---- merge of two sorted lists held in shared memory (stable: ties keep the old sample first) ------------------
-// zs / ss [0, n) old, zn / sn [0, m) new -> out_z / out_s [0, n + m)
+// ---- merge of two monotone lists held in shared memory into one ascending list (stable: ties keep the old sample first) --
+// zs / ss [0, n) old, zn / sn [0, m) new -> out_z / out_s [0, n + m), n >= 1, m >= 1.  Each input may ascend or descend
+// (first > last): a ray that misses the box has tmin > tmax once both are clipped to [near, far], so its coarse list
+// descends, and so do the importance samples drawn from it in round 0.  A descending list is read from its end; the
+// output is what torch.sort gives the reference.
 __device__ __forceinline__ void warp_merge(const float* zs, const float* ss, int n, const float* zn, const float* sn, int m, float* out_z,
                                            float* out_s, int lane) {
+    const bool old_desc = zs[0] > zs[n - 1], new_desc = zn[0] > zn[m - 1];
+    auto old_at = [&](int k) { return old_desc ? n - 1 - k : k; };       // storage index of the k-th smallest
+    auto new_at = [&](int j) { return new_desc ? m - 1 - j : j; };
     for (int k = lane; k < n; k += 32) {
-        const float v = zs[k];
+        const int i = old_at(k);
+        const float v = zs[i];
         int lo = 0, hi = m;                       // #(new < v)
-        while (lo < hi) { const int mid = (lo + hi) >> 1; if (zn[mid] < v) lo = mid + 1; else hi = mid; }
+        while (lo < hi) { const int mid = (lo + hi) >> 1; if (zn[new_at(mid)] < v) lo = mid + 1; else hi = mid; }
         out_z[k + lo] = v;
-        if (out_s) out_s[k + lo] = ss[k];
+        if (out_s) out_s[k + lo] = ss[i];
     }
     for (int j = lane; j < m; j += 32) {
-        const float v = zn[j];
+        const int i = new_at(j);
+        const float v = zn[i];
         int lo = 0, hi = n;                       // #(old <= v)
-        while (lo < hi) { const int mid = (lo + hi) >> 1; if (zs[mid] <= v) lo = mid + 1; else hi = mid; }
+        while (lo < hi) { const int mid = (lo + hi) >> 1; if (zs[old_at(mid)] <= v) lo = mid + 1; else hi = mid; }
         out_z[j + lo] = v;
-        if (out_s) out_s[j + lo] = sn ? sn[j] : 0.f;
+        if (out_s) out_s[j + lo] = sn ? sn[i] : 0.f;
     }
 }
 
 struct UpParams {
     const float* rays_o; const float* dirs; const float* radiis; const float* rays_cos;
-    float* z; float* sdf;        // [R, stride] sorted lists (n valid), updated in place by the merge
+    float* z; float* sdf;        // [R, stride] lists (n valid), updated in place by the merge (ascending afterwards)
     const float* new_z_in;       // [R, m_in] samples of the previous round (NULL: nothing to merge)
     const float* new_sdf_in;     // [R * m_in] their SDF values
     const float* u;              // [m] = linspace(0.5/m, 1-0.5/m, m)

@@ -51,6 +51,38 @@ def test_oracle_renderer_golden():
             assert rel_err(p.grad, g["grads"][n]) < 1e-4, n
 
 
+def test_oracle_sample_ray_rounds():
+    """sample_ray(rounds=...) records the depth / SDF lists after the coarse samples and after every round without changing
+    what it returns.  A ray that misses the box keeps the descending coarse list of the reference until the first sort."""
+    g = load("renderer.npz")
+    i = g["inputs"]
+    m = _oracle(g, torch.float64)
+    o = torch.cat([i["rays_o"][:5], torch.tensor([[2.0, 1.2, 0.0]])]).double()          # last ray: misses the unit box
+    d = torch.cat([i["dirs"][:5], F.normalize(torch.tensor([[-1.0, 0.1, 0.05]]), dim=-1)]).double()
+    near, far = RR.near_far_from_sphere(o, d)
+    args = (o, d, near, far, torch.full((6, 1), 1e-3, dtype=torch.float64), torch.ones(6, 1, dtype=torch.float64),
+            torch.rand(6, 1, generator=torch.Generator().manual_seed(2), dtype=torch.float64))
+    want = m.sample_ray(*args)
+    rounds = []
+    got = m.sample_ray(*args, rounds=rounds)
+    assert all(torch.equal(a, b) for a, b in zip(got, want))
+    steps, n = m.cfg['up_sample_steps'], m.cfg['n_samples']
+    assert len(rounds) == steps + 1
+    for r, (t, sdf) in enumerate(rounds):
+        assert t.shape == (6, n + r * (m.cfg['n_importance'] // steps))
+        assert (sdf is None) == (r == steps)
+        if r > 0:
+            assert bool((t[:, 1:] >= t[:, :-1]).all())
+        if sdf is not None:
+            pts = o[:, None, :] + d[:, None, :] * t[..., None]
+            lvl = torch.log2(RR.O.compute_ball_radii(t[..., None], args[4][:, None, :], args[5][:, None, :]) / m.base_radii)
+            assert torch.allclose(sdf, m.sdf_network.sdf(pts.reshape(-1, 3), lvl.reshape(-1, 1)).reshape(t.shape), atol=1e-12)
+    t_coarse = rounds[0][0]
+    assert bool((t_coarse[-1, 1:] < t_coarse[-1, :-1]).all()) and bool((t_coarse[:5, 1:] > t_coarse[:5, :-1]).all())
+    ts, _, idx = got                                   # the packed starts come from the last list of their ray
+    assert all(bool(torch.isin(ts[idx == r], rounds[-1][0][r]).all()) for r in range(6))
+
+
 @pytest.mark.gpu
 def test_cuda_renderer_golden():
     if not torch.cuda.is_available():
