@@ -444,6 +444,25 @@ TF_API int tf_occ_march_write(const float* rays_o, const float* rays_d, const fl
                               const int32_t* offsets, int64_t* ray_indices, float* t_starts, float* t_ends,
                               tf_stream_t stream);
 
+/* ---- isosurface extraction (marching cubes) ---------------------------------------------------------
+ * mcubes.marching_cubes(u, threshold) as extract_mesh.py calls it on the shape stage's SDF lattice, GPU-resident.
+ * u [nx][ny][nz] fp32, z fastest, nx, ny, nz >= 2, nx*ny*nz < 2^31; a point is inside iff u < threshold.  Rows are the
+ * nx*ny (i, j) lines of points.
+ *   vertices: one per crossed lattice edge, owned by the edge's lower point p = (i*ny + j)*nz + k, ordered by (p, axis x/y/z),
+ *             at index coordinate a_axis + (threshold - u_a) / (u_b - u_a) (each op one fp32 rounding);
+ *   triangles int32 [T,3]: cells in order (i*ny + j)*nz + k, then in the order of the generated case table
+ *             (tensoflow_b200/isosurface_table.py); (v1 - v0) x (v2 - v0) points toward increasing u.
+ * tf_iso_count writes per row the owned crossed edges (vert_count[nx*ny]) and the triangles of the row's cells
+ * (tri_count[nx*ny]).  The caller takes the exclusive prefix sums (int64, totals < 2^31), then tf_iso_vertices writes
+ * vertices [V,3] and index_volume [nx*ny*nz] (int32 vertices owned by the points before p, every p), and
+ * tf_iso_triangles reads index_volume and writes triangles [T,3].  No atomics: the output is bit-reproducible. */
+TF_API int tf_iso_count(const float* u, int32_t nx, int32_t ny, int32_t nz, float threshold, int32_t* vert_count,
+                        int32_t* tri_count, tf_stream_t stream);
+TF_API int tf_iso_vertices(const float* u, int32_t nx, int32_t ny, int32_t nz, float threshold, const int64_t* vert_offsets,
+                           float* vertices, int32_t* index_volume, tf_stream_t stream);
+TF_API int tf_iso_triangles(const float* u, int32_t nx, int32_t ny, int32_t nz, float threshold, const int64_t* tri_offsets,
+                            const int32_t* index_volume, int32_t* triangles, tf_stream_t stream);
+
 /* ---- optimizer step ------------------------------------------------------------------------------
  * torch.optim.Adam(grad_vars, betas=(0.9, 0.99)).step() of the reference trainer (train/trainer_inv.py:112,212; one
  * learning rate per parameter group, :247-248) as ONE streaming pass: for tensor t (numel[t] fp32 elements in any

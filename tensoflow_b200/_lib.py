@@ -68,6 +68,9 @@ _SIGNATURES = {
                                         _P, _P, _P, _P, _P]),
     "tf_neus_composite_bwd": (C.c_int, [_P, _P, _P, _P, _P, C.c_int32, _P, C.c_float, _P, C.c_int32,
                                         _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
+    "tf_iso_count": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, C.c_float, _P, _P, _P]),
+    "tf_iso_vertices": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, C.c_float, _P, _P, _P, _P]),
+    "tf_iso_triangles": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, C.c_float, _P, _P, _P, _P]),
 }
 
 # later sections of the ABI (small MLP layers, flow sampler, MC shading, BVH)

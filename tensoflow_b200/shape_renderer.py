@@ -499,6 +499,43 @@ class ShapeRenderer(torch.nn.Module):
             res[k] = full.reshape(h, w, -1).cpu().numpy()
         return res
 
+    # ---- mesh export (the reference's NeRO-derived extract_fields / extract_geometry, used by extract_mesh.py) ---------------
+    EXTRACT_SLAB_POINTS = 1 << 24          # lattice points per field-evaluation slab (bounds the temporary xyz to 192 MB)
+
+    @torch.no_grad()
+    def extract_fields(self, bound_min, bound_max, resolution: int) -> torch.Tensor:
+        """u [R,R,R] fp32 on the device: TensoSDF.sdf(x, None) on the lattice linspace(bound_min[a], bound_max[a], R) per axis
+        (z fastest), +1.0 (the outside value) where ||x|| >= 1.  Evaluated in slabs of x-planes."""
+        if torch.device(self.device).type != 'cuda':
+            raise RuntimeError("extract_fields runs on the CUDA kernels (tensoflow_b200 has no CPU path)")
+        R = int(resolution)
+        lo = torch.as_tensor(bound_min, dtype=torch.float32).reshape(3).cpu()
+        hi = torch.as_tensor(bound_max, dtype=torch.float32).reshape(3).cpu()
+        axes = [torch.linspace(float(lo[a]), float(hi[a]), R).to(self.device) for a in range(3)]
+        yy, zz = torch.meshgrid(axes[1], axes[2], indexing='ij')
+        yz = torch.stack([yy, zz], -1).reshape(1, R * R, 2)
+        u = torch.empty(R, R, R, device=self.device, dtype=torch.float32)
+        planes = max(1, self.EXTRACT_SLAB_POINTS // (R * R))
+        for i0 in range(0, R, planes):
+            xs = axes[0][i0:i0 + planes]
+            pts = torch.cat([xs[:, None, None].expand(-1, R * R, 1), yz.expand(xs.shape[0], -1, -1)], -1).reshape(-1, 3)
+            val = self.sdf_network.sdf(pts, None).reshape(-1)
+            val = torch.where(torch.norm(pts, dim=-1) >= 1.0, torch.ones_like(val), val)
+            u[i0:i0 + xs.shape[0]] = val.reshape(xs.shape[0], R, R)
+        return u
+
+    @torch.no_grad()
+    def extract_geometry(self, bound_min, bound_max, resolution: int, threshold: float = 0.0):
+        """Zero level set of the SDF as a triangle mesh -> (vertices [V,3] world fp32, triangles [T,3] int32) on the device,
+        winding out of the object: marching cubes (tensoflow_b200.isosurface) on extract_fields, vertices rescaled as
+        v / (R - 1) * (bound_max - bound_min) + bound_min.  `MaterialRenderer(cfg, *shape.extract_geometry(...))` takes it."""
+        from .isosurface import marching_cubes
+        u = self.extract_fields(bound_min, bound_max, resolution)
+        verts, tris = marching_cubes(u, threshold)
+        lo = torch.as_tensor(bound_min, dtype=torch.float32).reshape(1, 3).to(verts.device)
+        hi = torch.as_tensor(bound_max, dtype=torch.float32).reshape(1, 3).to(verts.device)
+        return verts / (int(resolution) - 1.0) * (hi - lo) + lo, tris
+
     # ---- alpha mask (reference shapeRenderer.py:257-325) --------------------------------------------
     @torch.no_grad()
     def compute_grid_alpha(self, xyz_locs, length):
