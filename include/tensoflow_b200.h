@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define TF_ABI_VERSION 1
+#define TF_ABI_VERSION 2
 
 #if defined(__GNUC__)
 #define TF_API __attribute__((visibility("default")))
@@ -120,25 +120,21 @@ TF_API int tf_sdf_only_fwd(const tf_vm_field_t* f, const tf_sdf_mlp_t* m, const 
 TF_API int tf_sdf_point_fwd(const tf_vm_field_t* f, const tf_sdf_mlp_t* m, const float* xyz, const float* level,
                             int64_t n, float* sdf, float* feat, void* workspace, size_t ws_bytes, tf_stream_t stream);
 
+/* Byte offset of the centre hidden activations [n, hidden] inside the workspace that was passed to tf_sdf_stencil_fwd (with
+ * feat != NULL); (size_t)-1 exactly when the tensor-core forward does not apply to this decoder shape (then neither
+ * tf_sdf_point_fwd nor the block exists). */
+TF_API size_t tf_sdf_stencil_fwd_hidden_offset(const tf_vm_field_t* f, const tf_sdf_mlp_t* m);
+
 /* Backward of tf_sdf_stencil_fwd.  g_sdf[n], g_feat[n,A], g_grad[n,3], g_hess[n] are the
  * upstream gradients (each may be NULL = zero); sdf7 is the forward output.
+ * hidden_centre[n, hidden] is the block at tf_sdf_stencil_fwd_hidden_offset(f, m) of the forward's workspace, which the caller
+ * keeps alive until this call (it feeds the weight gradient of the appearance head and is not recomputed).  It is required when
+ * g_feat != NULL and the offset is not (size_t)-1 (tensor-core path): the call returns an error without it.  Otherwise it is
+ * ignored and may be NULL.
  * Any workspace size >= tf_sdf_stencil_bwd_workspace(.., 1) works; larger is faster
  * (the call processes the n samples in slices that fit). */
 TF_API size_t tf_sdf_stencil_bwd_workspace(const tf_vm_field_t* f, const tf_sdf_mlp_t* m, int64_t n_slice);
 TF_API int tf_sdf_stencil_bwd(const tf_vm_field_t* f, const tf_sdf_mlp_t* m, const float* xyz,
-                       const float* level, int64_t n, const float units[3], const float* sdf7,
-                       const float* g_sdf, const float* g_feat, const float* g_grad,
-                       const float* g_hess, const tf_vm_mut_t* g_field,
-                       const tf_sdf_mlp_grad_t* g_mlp, void* workspace, size_t ws_bytes,
-                       tf_stream_t stream);
-
-/* The same with the centre hidden activations KEPT from the forward call: hidden_centre[n, hidden] = the block at byte offset
- * tf_sdf_stencil_fwd_hidden_offset(f, m) of the workspace that was passed to tf_sdf_stencil_fwd (with feat != NULL), which the
- * caller then has to keep alive until the backward call.  The backward kernel does not recompute / store them (they feed the
- * weight gradient of the appearance head).  hidden_centre == NULL behaves like tf_sdf_stencil_bwd; the offset is (size_t)-1
- * when the forward path for this decoder shape does not produce the block. */
-TF_API size_t tf_sdf_stencil_fwd_hidden_offset(const tf_vm_field_t* f, const tf_sdf_mlp_t* m);
-TF_API int tf_sdf_stencil_bwd_kept(const tf_vm_field_t* f, const tf_sdf_mlp_t* m, const float* xyz,
                        const float* level, int64_t n, const float units[3], const float* sdf7, const float* hidden_centre,
                        const float* g_sdf, const float* g_feat, const float* g_grad,
                        const float* g_hess, const tf_vm_mut_t* g_field,
@@ -246,10 +242,10 @@ TF_API int tf_cube_light_bwd(int32_t res, const float* dirs, const uint8_t* mask
  * c = cond (0 / 1), t = 1 - c; feat[pn, feat_dim] holds one conditioning vector per point (sn >= 16 consecutive pairs share
  * it; feat_dim <= 40); W1[64, 7 + feat_dim], W2/W3[64, 64], W4[21, 64] are the nn.Linear weights (row-major [out, in]);
  * scale / offset are the Reshift constants (2, -1).  The [M, 64] activations stay on chip.
- * save_h[M, 3, 64] / save_st[M, 24] (both or none; NULL = not kept): the tensor-core forward stores the three hidden activations
- * and the spline parameters there, and tf_flow_block_bwd given them (saved_h / saved_st) runs its adjoint chain on the tensor
- * cores without recomputing the forward; with NULL it recomputes on the FP32 pipe.  tf_flow_block_uses_tensor_cores() tells
- * which forward kernel is active (TF_FLOW_SIMT=1 in the environment selects the FP32-pipe kernels for A/B runs).
+ * Both directions run on the tensor cores (tcgen05).
+ * save_h[M, 3, 64] / save_st[M, 24] (both or none; NULL = not kept): the forward stores the three hidden activations and the
+ * spline parameters there.  tf_flow_block_bwd requires them (saved_h / saved_st, from a forward with inverse = 0): its adjoint
+ * chain reads them and does not recompute the forward; without them it returns an error and launches nothing.
  * bwd (forward spline only): g_y_out[M,2] / g_logj[M] (each may be NULL) -> g_y_in[M,2]; d_feat[pn, feat_dim] and the weight
  * / bias gradients are ACCUMULATED (atomics; the caller zero-initialises).  The gradient of logj_in equals g_logj. */
 TF_API int tf_flow_block_fwd(const float* y_in, const float* logj_in, const float* feat, int32_t feat_dim, int32_t sn,
@@ -257,7 +253,6 @@ TF_API int tf_flow_block_fwd(const float* y_in, const float* logj_in, const floa
                              const float* b3, const float* W4, const float* b4, float scale, float offset, int32_t cond,
                              int32_t inverse, int64_t M, float* y_out, float* logj_out, float* save_h, float* save_st,
                              tf_stream_t stream);
-TF_API int tf_flow_block_uses_tensor_cores(void);
 TF_API int tf_flow_block_bwd(const float* y_in, const float* feat, int32_t feat_dim, int32_t sn, const float* W1,
                              const float* b1, const float* W2, const float* b2, const float* W3, const float* b3,
                              const float* W4, const float* b4, float scale, float offset, int32_t cond, int64_t M,
@@ -487,10 +482,10 @@ TF_API int tf_kernel_timing_read(const char* name, double* total_ms, int32_t* la
  * out[m][n] += sum_r X[r][m] * Y[r][n]  (X [rows,M], Y [rows,N], out [M,N], all row-major fp32).
  * This is the dW = dPre^T X product every nn.Linear backward of the path ends with
  * (torch autograd's addmm in the reference: network/fields.py:192-198 decoder, other/material MLPs).
- * Shapes with M in {128,256}, N % 16 == 0, N <= 256 run on tcgen05 (3xTF32, fp32-level accuracy);
- * anything else on the FFMA kernel.  force_simt != 0 selects the FFMA kernel (A/B testing). */
+ * Shapes with M % 16 == 0, N % 16 == 0, both in [16, 256], and 16-byte aligned X / Y run on tcgen05 (3xTF32, fp32-level
+ * accuracy); anything else on the FFMA kernel. */
 TF_API int tf_xty_accumulate(const float* X, const float* Y, int64_t rows, int32_t M, int32_t N, float* out,
-                             int32_t force_simt, tf_stream_t stream);
+                             tf_stream_t stream);
 
 #ifdef __cplusplus
 }

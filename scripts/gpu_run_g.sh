@@ -5,5 +5,3 @@ mkdir -p gpurun_out
 timeout 600 python -m pytest tests/test_flow_gpu.py tests/test_golden.py tests/test_mc_gpu.py -q -m gpu -x 2>&1 | tail -40 > gpurun_out/r2g_pytest.log
 tail -25 gpurun_out/r2g_pytest.log
 timeout 300 python scripts/bench_material.py --steps 5 > gpurun_out/r2g_bench_material.json 2> gpurun_out/r2g_bench_material.err; tail -c 1700 gpurun_out/r2g_bench_material.json; tail -3 gpurun_out/r2g_bench_material.err
-TF_FLOW_SIMT=1 timeout 300 python scripts/bench_material.py --steps 5 > gpurun_out/r2g_bench_material_simt.json 2>/dev/null; python -c "
-import json; d=json.load(open('gpurun_out/r2g_bench_material_simt.json')); print('simt', d['ms_per_step'], d['calls_ms_per_step'].get('flow_block_fwd'))"

@@ -5,15 +5,12 @@ set -u
 mkdir -p gpurun_out
 rm -f gpurun_out/gpu_test_errors.json
 python -m pytest tests/ -q -m gpu 2>&1 | tail -30 > gpurun_out/r2i_pytest.log; tail -8 gpurun_out/r2i_pytest.log
-TF_FLOW_SIMT=1 python -m pytest tests/test_flow_gpu.py tests/test_golden.py tests/test_mc_gpu.py -q -m gpu 2>&1 | tail -5 > gpurun_out/r2i_pytest_flow_simt.log; tail -3 gpurun_out/r2i_pytest_flow_simt.log
 timeout 1200 compute-sanitizer --tool memcheck --error-exitcode 1 python -m pytest tests/test_shape_gpu.py tests/test_renderer.py tests/test_shader.py -q -x \
     -k "vm_feature or neus_composite or tv_loss or gaussian or sampler or probe or alpha_mask or cuda_shader" > gpurun_out/r2i_sanitizer_memcheck.log 2>&1
 echo "memcheck rc=$?" | tee -a gpurun_out/r2i_sanitizer_memcheck.log
 timeout 1200 compute-sanitizer --tool racecheck --error-exitcode 1 python -m pytest tests/test_shape_gpu.py tests/test_renderer.py -q -x \
     -k "neus_composite or tv_loss or gaussian or sampler or probe" > gpurun_out/r2i_sanitizer_racecheck.log 2>&1
 echo "racecheck rc=$?" | tee -a gpurun_out/r2i_sanitizer_racecheck.log
-TF_FLOW_SIMT=1 timeout 1200 compute-sanitizer --tool memcheck --error-exitcode 1 python -m pytest tests/test_flow_gpu.py -q -x -k "logq or sample" > gpurun_out/r2i_sanitizer_memcheck_flow_simt.log 2>&1
-echo "memcheck flow (FP32 pipe) rc=$?" | tee -a gpurun_out/r2i_sanitizer_memcheck_flow_simt.log
 python bench.py 2> gpurun_out/r2i_bench.err | tee gpurun_out/r2i_bench.json | python -c "
 import json,sys
 d=json.loads(sys.stdin.read())

@@ -57,13 +57,10 @@ _SIGNATURES = {
                                   C.c_size_t, _P]),
     "tf_sdf_point_fwd": (C.c_int, [C.POINTER(VMField), C.POINTER(SdfMlp), _P, _P, C.c_int64, _P, _P, _P, C.c_size_t, _P]),
     "tf_sdf_stencil_bwd_workspace": (C.c_size_t, [C.POINTER(VMField), C.POINTER(SdfMlp), C.c_int64]),
-    "tf_sdf_stencil_bwd": (C.c_int, [C.POINTER(VMField), C.POINTER(SdfMlp), _P, _P, C.c_int64,
-                                     C.POINTER(C.c_float), _P, _P, _P, _P, _P, C.POINTER(VMMut),
-                                     C.POINTER(SdfMlpGrad), _P, C.c_size_t, _P]),
     "tf_sdf_stencil_fwd_hidden_offset": (C.c_size_t, [C.POINTER(VMField), C.POINTER(SdfMlp)]),
-    "tf_sdf_stencil_bwd_kept": (C.c_int, [C.POINTER(VMField), C.POINTER(SdfMlp), _P, _P, C.c_int64,
-                                          C.POINTER(C.c_float), _P, _P, _P, _P, _P, _P, C.POINTER(VMMut),
-                                          C.POINTER(SdfMlpGrad), _P, C.c_size_t, _P]),
+    "tf_sdf_stencil_bwd": (C.c_int, [C.POINTER(VMField), C.POINTER(SdfMlp), _P, _P, C.c_int64,
+                                     C.POINTER(C.c_float), _P, _P, _P, _P, _P, _P, C.POINTER(VMMut),
+                                     C.POINTER(SdfMlpGrad), _P, C.c_size_t, _P]),
     "tf_neus_composite_fwd": (C.c_int, [_P, _P, _P, _P, _P, C.c_int32, _P, C.c_float, _P, C.c_int32,
                                         _P, _P, _P, _P, _P]),
     "tf_neus_composite_bwd": (C.c_int, [_P, _P, _P, _P, _P, C.c_int32, _P, C.c_float, _P, C.c_int32,
@@ -93,7 +90,6 @@ _OPTIONAL_SIGNATURES = {
                                      _P, _P, _P, _P, _P, _P, _P, _P]),
     "tf_flow_block_fwd": (C.c_int, [_P, _P, _P, C.c_int32, C.c_int32, _P, _P, _P, _P, _P, _P, _P, _P, C.c_float, C.c_float, C.c_int32, C.c_int32,
                                     C.c_int64, _P, _P, _P, _P, _P]),
-    "tf_flow_block_uses_tensor_cores": (C.c_int, []),
     "tf_flow_block_bwd": (C.c_int, [_P, _P, C.c_int32, C.c_int32, _P, _P, _P, _P, _P, _P, _P, _P, C.c_float, C.c_float, C.c_int32, C.c_int64,
                                     _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "tf_shader_encode_fwd": (C.c_int, [_P, _P, _P, _P, _P, C.c_int32, C.c_int32, C.c_int64, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
@@ -122,7 +118,7 @@ _OPTIONAL_SIGNATURES = {
     "tf_kernel_timing_enable": (None, [C.c_int32]),
     "tf_kernel_timing_reset": (None, []),
     "tf_kernel_timing_read": (C.c_int, [C.c_char_p, C.POINTER(C.c_double), C.POINTER(C.c_int32)]),
-    "tf_xty_accumulate": (C.c_int, [_P, _P, C.c_int64, C.c_int32, C.c_int32, _P, C.c_int32, _P]),
+    "tf_xty_accumulate": (C.c_int, [_P, _P, C.c_int64, C.c_int32, C.c_int32, _P, _P]),
 }
 
 
@@ -149,7 +145,7 @@ def load():
         fn = getattr(lib, name)
         fn.restype = res
         fn.argtypes = args
-    if lib.tf_abi_version() != 1:
+    if lib.tf_abi_version() != 2:
         raise RuntimeError("libtensoflow_b200.so ABI version mismatch")
     _lib = lib
     return lib

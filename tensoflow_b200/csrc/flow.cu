@@ -1,7 +1,6 @@
 // Piecewise-quadratic coupling transform of the TensoFlow sampler, one thread per
 // (surface point, direction) pair.  Restates ElementWisePWQuadraticTransform
 // (reference network/flow.py:314-525) for K = 10 bins: st = 11 vertex heights + 10 widths.
-#include <stdlib.h>
 #include "common.cuh"
 #include "flow_spline.cuh"
 
@@ -38,372 +37,11 @@ __global__ void __launch_bounds__(128) pwquad_bwd_kernel(const float* __restrict
     for (int i = 0; i < NST; ++i) d_st[r * NST + i] = ds[i];
 }
 
-// =====================================================================================================================
-// Fused coupling block (reference network/flow.py:549-641): conditioner MLP [PE(y_c) (7) | feature (F)] -> 64 -> 64 -> 64 -> 21
-// (Reshift on the whole input, LeakyReLU between the layers) + the piecewise-quadratic spline of the other coordinate, one
-// thread per (point, direction) pair.  The feature part of the first layer is shared by all directions of a point and is
-// evaluated once per point; the [M, 64] activations never leave the SM (the unfused path writes and re-reads them per layer).
-// Weights sit in shared memory transposed ([in][out]) so that a broadcast LDS.128 feeds 4 FMAs.
-// FLOP-bound on the FP32 pipe: 2 * (7*64 + 2*64*64 + 64*21) = 20.2 kFLOP per pair and block forward, ~3x that backward.
-// =====================================================================================================================
-constexpr int FH = 64, FPE = 7, FSTP = 24, FTILE = 128, FMAXF = 40, FMAXP = 10;
+// Fused coupling block (reference network/flow.py:549-641): input checks shared by both directions; the kernels are in flow_tc.cu
+constexpr int FMAXF = 40;          // widest per-point feature the tensor-core kernels take (their shared-memory tiles)
 
-struct FlowW { const float *W1, *b1, *W2, *b2, *W3, *b3, *W4, *b4; int F; float scale, offset; };
+struct FlowW { const float *W1, *b1, *W2, *b2, *W3, *b3, *W4, *b4; int F; };
 
-struct FlowSm {            // shared-memory views (floats)
-    float *w1a, *w2, *w3, *w4, *b1, *b2, *b3, *b4;
-};
-__device__ __forceinline__ float* flow_carve(float*& p, int n) { float* r = p; p += n; return r; }
-__device__ __forceinline__ void flow_load_weights(const FlowW& w, FlowSm& m, float*& sp, int tid, int nth) {
-    m.w1a = flow_carve(sp, FPE * FH + FH);      // 7 rows + one pad row (16-byte aligned rows)
-    m.w2 = flow_carve(sp, FH * FH); m.w3 = flow_carve(sp, FH * FH); m.w4 = flow_carve(sp, FH * FSTP);
-    m.b1 = flow_carve(sp, FH); m.b2 = flow_carve(sp, FH); m.b3 = flow_carve(sp, FH); m.b4 = flow_carve(sp, FSTP);
-    const int K1 = FPE + w.F;
-    for (int i = tid; i < FPE * FH; i += nth) { const int k = i / FH, j = i % FH; m.w1a[i] = w.W1[j * K1 + k]; }
-    for (int i = tid; i < FH * FH; i += nth) { const int k = i / FH, j = i % FH; m.w2[i] = w.W2[j * FH + k]; m.w3[i] = w.W3[j * FH + k]; }
-    for (int i = tid; i < FH * FSTP; i += nth) { const int k = i / FSTP, j = i % FSTP; m.w4[i] = j < NST ? w.W4[j * FH + k] : 0.f; }
-    for (int i = tid; i < FH; i += nth) { m.b1[i] = w.b1[i]; m.b2[i] = w.b2[i]; m.b3[i] = w.b3[i]; }
-    for (int i = tid; i < FSTP; i += nth) m.b4[i] = i < NST ? w.b4[i] : 0.f;
-}
-
-__device__ __forceinline__ float leaky(float x) { return x > 0.f ? x : 0.01f * x; }
-__device__ __forceinline__ void flow_posenc(float y, float scale, float offset, float x[FPE]) {
-    x[0] = y;
-    x[1] = sinf(y); x[2] = cosf(y);
-    x[3] = sinf(y * 2.f); x[4] = cosf(y * 2.f);
-    x[5] = sinf(y * 4.f); x[6] = cosf(y * 4.f);
-#pragma unroll
-    for (int k = 0; k < FPE; ++k) x[k] = x[k] * scale + offset;            // Reshift (flow.py:146-164) on the whole input
-}
-// out[j] = act(base[j] + sum_k WT[k][j] in[k]),  WT [KIN][64] in shared memory
-template <int KIN, bool ACT>
-__device__ __forceinline__ void flow_dense(const float* __restrict__ WT, const float* __restrict__ base, const float* in, float* out) {
-#pragma unroll
-    for (int j4 = 0; j4 < FH / 4; ++j4) {
-        const float4 b = *reinterpret_cast<const float4*>(base + 4 * j4);
-        out[4 * j4] = b.x; out[4 * j4 + 1] = b.y; out[4 * j4 + 2] = b.z; out[4 * j4 + 3] = b.w;
-    }
-#pragma unroll
-    for (int k = 0; k < KIN; ++k) {
-        if ((k & 7) == 0) asm volatile("" ::: "memory");        // keeps ptxas from hoisting hundreds of LDS ahead (register spills)
-        const float x = in[k];
-#pragma unroll
-        for (int j4 = 0; j4 < FH / 4; ++j4) {
-            const float4 w = *reinterpret_cast<const float4*>(WT + k * FH + 4 * j4);
-            out[4 * j4] = fmaf(w.x, x, out[4 * j4]); out[4 * j4 + 1] = fmaf(w.y, x, out[4 * j4 + 1]);
-            out[4 * j4 + 2] = fmaf(w.z, x, out[4 * j4 + 2]); out[4 * j4 + 3] = fmaf(w.w, x, out[4 * j4 + 3]);
-        }
-    }
-    if (ACT) {
-#pragma unroll
-        for (int j = 0; j < FH; ++j) out[j] = leaky(out[j]);
-    }
-}
-// st[j < 24] = b4[j] + sum_k W4T[k][j] h3[k]
-__device__ __forceinline__ void flow_head(const float* __restrict__ W4T, const float* __restrict__ b4, const float* h3, float* st) {
-#pragma unroll
-    for (int j = 0; j < FSTP; ++j) st[j] = b4[j];
-#pragma unroll
-    for (int k = 0; k < FH; ++k) {
-        if ((k & 7) == 0) asm volatile("" ::: "memory");
-        const float x = h3[k];
-#pragma unroll
-        for (int j4 = 0; j4 < FSTP / 4; ++j4) {
-            const float4 w = *reinterpret_cast<const float4*>(W4T + k * FSTP + 4 * j4);
-            st[4 * j4] = fmaf(w.x, x, st[4 * j4]); st[4 * j4 + 1] = fmaf(w.y, x, st[4 * j4 + 1]);
-            st[4 * j4 + 2] = fmaf(w.z, x, st[4 * j4 + 2]); st[4 * j4 + 3] = fmaf(w.w, x, st[4 * j4 + 3]);
-        }
-    }
-}
-// din[k] = sum_j WT[k][j] dout[j]  (NOUT = 64 or 24 columns per row)
-template <int KIN, int NOUT>
-__device__ __forceinline__ void flow_dense_T(const float* __restrict__ WT, const float* dout, float* din) {
-#pragma unroll
-    for (int k = 0; k < KIN; ++k) {
-        if ((k & 3) == 0) asm volatile("" ::: "memory");
-        float a0 = 0.f, a1 = 0.f, a2 = 0.f, a3 = 0.f;
-#pragma unroll
-        for (int j4 = 0; j4 < NOUT / 4; ++j4) {
-            const float4 w = *reinterpret_cast<const float4*>(WT + k * NOUT + 4 * j4);
-            a0 = fmaf(w.x, dout[4 * j4], a0); a1 = fmaf(w.y, dout[4 * j4 + 1], a1);
-            a2 = fmaf(w.z, dout[4 * j4 + 2], a2); a3 = fmaf(w.w, dout[4 * j4 + 3], a3);
-        }
-        din[k] = (a0 + a1) + (a2 + a3);
-    }
-}
-// per-point part of the first layer for the points of a tile: h1p[lp][j] = b1[j] + sum_k W1[j][7+k] (scale feat[p][k] + offset)
-__device__ __forceinline__ void flow_point_partials(const FlowW& w, const float* __restrict__ b1s, const float* __restrict__ feat, int64_t p_first,
-                                                    int np, float* h1p, int tid, int nth) {
-    const int K1 = FPE + w.F;
-    for (int e = tid; e < np * FH; e += nth) {
-        const int lp = e / FH, j = e % FH;
-        const float* f = feat + (p_first + lp) * w.F;
-        const float* wr = w.W1 + (size_t)j * K1 + FPE;
-        float acc = b1s[j];
-        for (int k = 0; k < w.F; ++k) acc = fmaf(__ldg(wr + k), __ldg(f + k) * w.scale + w.offset, acc);
-        h1p[lp * FH + j] = acc;
-    }
-}
-
-struct FlowFwdParams {
-    FlowW w; const float* y_in; const float* logj_in; const float* feat; int sn, cond; int64_t M;
-    float* y_out; float* logj_out;
-};
-
-template <bool INVERSE>
-__global__ void __launch_bounds__(FTILE, 2) flow_block_fwd_kernel(FlowFwdParams p) {
-    extern __shared__ __align__(16) float fsm[];
-    float* sp = fsm;
-    FlowSm m;
-    const int tid = threadIdx.x;
-    flow_load_weights(p.w, m, sp, tid, FTILE);
-    float* h1p = flow_carve(sp, FMAXP * FH);
-    __syncthreads();
-    const int64_t ntiles = (p.M + FTILE - 1) / FTILE;
-    for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
-        const int64_t i0 = tile * FTILE;
-        const int64_t i_last = (i0 + FTILE - 1 < p.M ? i0 + FTILE - 1 : p.M - 1);
-        const int64_t p_first = i0 / p.sn;
-        const int np = (int)(i_last / p.sn - p_first) + 1;
-        flow_point_partials(p.w, m.b1, p.feat, p_first, np, h1p, tid, FTILE);
-        __syncthreads();
-        const int64_t i = i0 + tid;
-        if (i < p.M) {
-            const float y0 = p.y_in[i * 2], y1 = p.y_in[i * 2 + 1];
-            const float yc = p.cond ? y1 : y0, yt = p.cond ? y0 : y1;
-            float xin[FPE], ha[FH], hb[FH], st[FSTP];
-            flow_posenc(yc, p.w.scale, p.w.offset, xin);
-            flow_dense<FPE, true>(m.w1a, h1p + (int)(i / p.sn - p_first) * FH, xin, ha);
-            flow_dense<FH, true>(m.w2, m.b2, ha, hb);
-            flow_dense<FH, true>(m.w3, m.b3, hb, ha);
-            flow_head(m.w4, m.b4, ha, st);
-            float xt, lj;
-            if (INVERSE) pwquad_eval_inverse(st, yt, xt, lj);
-            else pwquad_eval_forward(st, yt, xt, lj);
-            p.y_out[i * 2 + p.cond] = yc;
-            p.y_out[i * 2 + 1 - p.cond] = xt;
-            p.logj_out[i] = (p.logj_in ? p.logj_in[i] : 0.f) + lj;
-        }
-        __syncthreads();
-    }
-}
-
-// ---- backward (density direction only: the sampling direction runs on frozen copies without autograd) ----------------
-constexpr int FLD = FH + 4;        // row stride of the activation tiles (bank spread for per-thread rows, 16-byte aligned)
-constexpr int FLDS = FSTP + 4;     // row stride of the d_st tile
-
-struct FlowBwdParams {
-    FlowW w; const float* y_in; const float* feat; int sn, cond; int64_t M;
-    const float* g_y_out;          // [M,2] or NULL
-    const float* g_logj;           // [M] or NULL
-    float* g_y_in;                 // [M,2]
-    float* d_feat;                 // [pn,F]   (+=, atomics)
-    float *dW1, *db1, *dW2, *db2, *dW3, *db3, *dW4, *db4;      // (+=, atomics at the end of the CTA)
-};
-
-// acc[j][k] += sum_p D[p][j] H[p][k] over the 128 rows of a tile; every thread owns a JP x KP patch of the accumulator
-template <int JP, int KP>
-__device__ __forceinline__ void flow_tile_xty(const float* __restrict__ D, int ldd, const float* __restrict__ H, int ldh, float* __restrict__ acc,
-                                              int ldacc, int j0, int k0) {
-    float a[JP][KP];
-#pragma unroll
-    for (int x = 0; x < JP; ++x)
-#pragma unroll
-        for (int y = 0; y < KP; ++y) a[x][y] = 0.f;
-    for (int p = 0; p < FTILE; ++p) {
-        float d[JP], h[KP];
-#pragma unroll
-        for (int x = 0; x < JP; ++x) d[x] = D[p * ldd + j0 + x];
-#pragma unroll
-        for (int y = 0; y < KP; ++y) h[y] = H[p * ldh + k0 + y];
-#pragma unroll
-        for (int x = 0; x < JP; ++x)
-#pragma unroll
-            for (int y = 0; y < KP; ++y) a[x][y] = fmaf(d[x], h[y], a[x][y]);
-    }
-#pragma unroll
-    for (int x = 0; x < JP; ++x)
-#pragma unroll
-        for (int y = 0; y < KP; ++y) acc[(j0 + x) * ldacc + k0 + y] += a[x][y];
-}
-// bias[j] += column sums of a tile
-__device__ __forceinline__ void flow_tile_colsum(const float* __restrict__ D, int ldd, int ncols, float* __restrict__ acc, int tid) {
-    if (tid < ncols) {
-        float s = 0.f;
-        for (int p = 0; p < FTILE; ++p) s += D[p * ldd + tid];
-        acc[tid] += s;
-    }
-}
-
-__global__ void __launch_bounds__(FTILE, 1) flow_block_bwd_kernel(FlowBwdParams p) {
-    extern __shared__ __align__(16) float fsm[];
-    float* sp = fsm;
-    FlowSm m;
-    const int tid = threadIdx.x;
-    flow_load_weights(p.w, m, sp, tid, FTILE);
-    const int F = p.w.F, K1 = FPE + F;
-    float* aW1a = flow_carve(sp, FH * 8);            // [64][8]
-    float* aW1b = flow_carve(sp, FH * FMAXF);        // [64][F]
-    float* aW2 = flow_carve(sp, FH * FH);            // [out j][in k]
-    float* aW3 = flow_carve(sp, FH * FH);
-    float* aW4 = flow_carve(sp, FSTP * FH);          // [24][64]
-    float* ab1 = flow_carve(sp, FH); float* ab2 = flow_carve(sp, FH); float* ab3 = flow_carve(sp, FH); float* ab4 = flow_carve(sp, FSTP);
-    float* Ta = flow_carve(sp, FTILE * FLD);
-    float* Tb = flow_carve(sp, FTILE * FLD);
-    float* Tc = flow_carve(sp, FTILE * FLD);
-    float* Td = flow_carve(sp, FTILE * FLDS);
-    float* Tx = flow_carve(sp, FTILE * 8);
-    float* h1p = flow_carve(sp, FMAXP * FH);
-    float* Sp = flow_carve(sp, FMAXP * FH);
-    for (int i = tid; i < FH * 8 + FH * FMAXF + 2 * FH * FH + FSTP * FH + 3 * FH + FSTP; i += FTILE) aW1a[i] = 0.f;   // contiguous accumulators
-    __syncthreads();
-    const int64_t ntiles = (p.M + FTILE - 1) / FTILE;
-    for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
-        const int64_t i0 = tile * FTILE;
-        const int64_t i_last = (i0 + FTILE - 1 < p.M ? i0 + FTILE - 1 : p.M - 1);
-        const int64_t p_first = i0 / p.sn;
-        const int np = (int)(i_last / p.sn - p_first) + 1;
-        flow_point_partials(p.w, m.b1, p.feat, p_first, np, h1p, tid, FTILE);
-        __syncthreads();
-        const int64_t i = i0 + tid;
-        const bool live = i < p.M;
-        const int lp = live ? (int)(i / p.sn - p_first) : 0;
-        float yc = 0.f, d_yt = 0.f;
-        float dv[FH];                                     // running adjoint vector of the chain
-        {   // ---- forward recompute: activations to the tiles, spline adjoint ------------------------------------
-            float xin[FPE], ha[FH], hb[FH], st[FSTP], dst[FSTP];
-#pragma unroll
-            for (int k = 0; k < FSTP; ++k) dst[k] = 0.f;
-            if (live) {
-                const float y0 = p.y_in[i * 2], y1 = p.y_in[i * 2 + 1];
-                yc = p.cond ? y1 : y0;
-                const float yt = p.cond ? y0 : y1;
-                flow_posenc(yc, p.w.scale, p.w.offset, xin);
-                flow_dense<FPE, true>(m.w1a, h1p + lp * FH, xin, ha);
-#pragma unroll
-                for (int j4 = 0; j4 < FH / 4; ++j4) *reinterpret_cast<float4*>(Ta + tid * FLD + 4 * j4) = make_float4(ha[4 * j4], ha[4 * j4 + 1], ha[4 * j4 + 2], ha[4 * j4 + 3]);
-                flow_dense<FH, true>(m.w2, m.b2, ha, hb);
-#pragma unroll
-                for (int j4 = 0; j4 < FH / 4; ++j4) *reinterpret_cast<float4*>(Tb + tid * FLD + 4 * j4) = make_float4(hb[4 * j4], hb[4 * j4 + 1], hb[4 * j4 + 2], hb[4 * j4 + 3]);
-                flow_dense<FH, true>(m.w3, m.b3, hb, ha);
-#pragma unroll
-                for (int j4 = 0; j4 < FH / 4; ++j4) *reinterpret_cast<float4*>(Tc + tid * FLD + 4 * j4) = make_float4(ha[4 * j4], ha[4 * j4 + 1], ha[4 * j4 + 2], ha[4 * j4 + 3]);
-                flow_head(m.w4, m.b4, ha, st);
-                const float gx = p.g_y_out ? p.g_y_out[i * 2 + 1 - p.cond] : 0.f;
-                const float gl = p.g_logj ? p.g_logj[i] : 0.f;
-                pwquad_adjoint(st, yt, gx, gl, d_yt, dst);
-            } else {
-#pragma unroll
-                for (int k = 0; k < FPE; ++k) xin[k] = 0.f;
-#pragma unroll
-                for (int j4 = 0; j4 < FH / 4; ++j4) {
-                    const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
-                    *reinterpret_cast<float4*>(Ta + tid * FLD + 4 * j4) = z; *reinterpret_cast<float4*>(Tb + tid * FLD + 4 * j4) = z;
-                    *reinterpret_cast<float4*>(Tc + tid * FLD + 4 * j4) = z;
-                }
-            }
-#pragma unroll
-            for (int k = 0; k < FSTP; ++k) Td[tid * FLDS + k] = dst[k];
-#pragma unroll
-            for (int k = 0; k < 8; ++k) Tx[tid * 8 + k] = k < FPE ? xin[k] : 0.f;
-            // dh3 = W4^T d_st
-            flow_dense_T<FH, FSTP>(m.w4, dst, dv);
-        }
-        __syncthreads();
-        // ---- layer 4: dW4 += d_st^T h3, db4 ------------------------------------------------------------------------
-        flow_tile_xty<3, 4>(Td, FLDS, Tc, FLD, aW4, FH, 3 * (tid >> 4), 4 * (tid & 15));
-        flow_tile_colsum(Td, FLDS, FSTP, ab4, tid);
-        __syncthreads();
-        {   // dpre3 = dh3 * leaky'(h3) -> Tc (own row), then dh2 = W3^T dpre3
-            float t[FH];
-#pragma unroll
-            for (int j = 0; j < FH; ++j) { dv[j] *= Tc[tid * FLD + j] > 0.f ? 1.f : 0.01f; Tc[tid * FLD + j] = dv[j]; }
-            flow_dense_T<FH, FH>(m.w3, dv, t);
-#pragma unroll
-            for (int j = 0; j < FH; ++j) dv[j] = t[j];
-        }
-        __syncthreads();
-        flow_tile_xty<4, 8>(Tc, FLD, Tb, FLD, aW3, FH, 4 * (tid >> 3), 8 * (tid & 7));
-        flow_tile_colsum(Tc, FLD, FH, ab3, tid);
-        __syncthreads();
-        {   // dpre2 -> Tb, dh1 = W2^T dpre2
-            float t[FH];
-#pragma unroll
-            for (int j = 0; j < FH; ++j) { dv[j] *= Tb[tid * FLD + j] > 0.f ? 1.f : 0.01f; Tb[tid * FLD + j] = dv[j]; }
-            flow_dense_T<FH, FH>(m.w2, dv, t);
-#pragma unroll
-            for (int j = 0; j < FH; ++j) dv[j] = t[j];
-        }
-        __syncthreads();
-        flow_tile_xty<4, 8>(Tb, FLD, Ta, FLD, aW2, FH, 4 * (tid >> 3), 8 * (tid & 7));
-        flow_tile_colsum(Tb, FLD, FH, ab2, tid);
-        __syncthreads();
-        {   // dpre1 -> Ta; d x_in -> d y_c
-#pragma unroll
-            for (int j = 0; j < FH; ++j) { dv[j] *= Ta[tid * FLD + j] > 0.f ? 1.f : 0.01f; Ta[tid * FLD + j] = dv[j]; }
-            float dx[8];
-            flow_dense_T<FPE, FH>(m.w1a, dv, dx);
-            if (live) {
-                const float sc = p.w.scale;
-                const float dyc = sc * (dx[0] + dx[1] * cosf(yc) - dx[2] * sinf(yc) + 2.f * (dx[3] * cosf(2.f * yc) - dx[4] * sinf(2.f * yc)) +
-                                        4.f * (dx[5] * cosf(4.f * yc) - dx[6] * sinf(4.f * yc)));
-                p.g_y_in[i * 2 + p.cond] = (p.g_y_out ? p.g_y_out[i * 2 + p.cond] : 0.f) + dyc;
-                p.g_y_in[i * 2 + 1 - p.cond] = d_yt;
-            }
-        }
-        __syncthreads();
-        // ---- layer 1: dW1a += dpre1^T x_in, db1, per-point sums S for the feature part --------------------------------
-        flow_tile_xty<1, 4>(Ta, FLD, Tx, 8, aW1a, 8, tid >> 1, 4 * (tid & 1));
-        flow_tile_colsum(Ta, FLD, FH, ab1, tid);
-        if (tid >= FH) {                                   // warps 2-3: S[lp][j] = sum of dpre1 over the tile's rows of point lp
-            const int j = tid - FH;
-            float s = 0.f;
-            int cur = 0;
-            for (int r = 0; r < FTILE; ++r) {
-                const int64_t ir = i0 + r;
-                const int lr = ir < p.M ? (int)(ir / p.sn - p_first) : cur;
-                if (lr != cur) { Sp[cur * FH + j] = s; s = 0.f; cur = lr; }
-                s += Ta[r * FLD + j];
-            }
-            Sp[cur * FH + j] = s;
-        }
-        __syncthreads();
-        // feature part: dW1b[j][k] += S[lp][j] xf[lp][k];  d_feat[p][k] += scale sum_j W1[j][7+k] S[lp][j]
-        for (int e = tid; e < np * F; e += FTILE) {
-            const int l = e / F, k = e % F;
-            const float xf = __ldg(p.feat + (p_first + l) * F + k) * p.w.scale + p.w.offset;
-            float g = 0.f;
-            for (int j = 0; j < FH; ++j) {
-                const float sj = Sp[l * FH + j];
-                g = fmaf(__ldg(p.w.W1 + (size_t)j * K1 + FPE + k), sj, g);
-                atomicAdd(&aW1b[j * FMAXF + k], sj * xf);
-            }
-            atomicAdd(p.d_feat + (p_first + l) * F + k, g * p.w.scale);
-        }
-        __syncthreads();
-    }
-    // ---- flush the CTA's weight-gradient partials ------------------------------------------------------------------------
-    for (int i = tid; i < FH * FPE; i += FTILE) { const int j = i / FPE, k = i % FPE; const float v = aW1a[j * 8 + k]; if (v != 0.f) atomicAdd(p.dW1 + (size_t)j * K1 + k, v); }
-    for (int i = tid; i < FH * F; i += FTILE) { const int j = i / F, k = i % F; const float v = aW1b[j * FMAXF + k]; if (v != 0.f) atomicAdd(p.dW1 + (size_t)j * K1 + FPE + k, v); }
-    for (int i = tid; i < FH * FH; i += FTILE) {
-        if (aW2[i] != 0.f) atomicAdd(p.dW2 + i, aW2[i]);
-        if (aW3[i] != 0.f) atomicAdd(p.dW3 + i, aW3[i]);
-    }
-    for (int i = tid; i < NST * FH; i += FTILE) if (aW4[i] != 0.f) atomicAdd(p.dW4 + i, aW4[i]);
-    for (int i = tid; i < FH; i += FTILE) {
-        if (ab1[i] != 0.f) atomicAdd(p.db1 + i, ab1[i]);
-        if (ab2[i] != 0.f) atomicAdd(p.db2 + i, ab2[i]);
-        if (ab3[i] != 0.f) atomicAdd(p.db3 + i, ab3[i]);
-    }
-    for (int i = tid; i < NST; i += FTILE) if (ab4[i] != 0.f) atomicAdd(p.db4 + i, ab4[i]);
-}
-
-size_t flow_fwd_smem() { return sizeof(float) * (size_t)(FPE * FH + FH + 2 * FH * FH + FH * FSTP + 3 * FH + FSTP + FMAXP * FH); }
-size_t flow_bwd_smem() {
-    return sizeof(float) * (size_t)(FPE * FH + FH + 2 * FH * FH + FH * FSTP + 3 * FH + FSTP                       // weights
-                                    + FH * 8 + FH * FMAXF + 2 * FH * FH + FSTP * FH + 3 * FH + FSTP                 // accumulators
-                                    + 3 * FTILE * FLD + FTILE * FLDS + FTILE * 8 + 2 * FMAXP * FH);                 // tiles
-}
 int flow_check(const FlowW& w, int sn, int cond, int64_t M) {
     TF_REQUIRE(w.W1 && w.b1 && w.W2 && w.b2 && w.W3 && w.b3 && w.W4 && w.b4, "flow block: NULL weight pointer");
     TF_REQUIRE(w.F >= 1 && w.F <= FMAXF, "flow block: feature width must be in [1, %d] (got %d)", FMAXF, w.F);
@@ -434,7 +72,7 @@ extern "C" TF_API int tf_pwquad_bwd(const float* y, const float* st, int64_t M, 
     return 0;
 }
 
-// tensor-core forward (flow_tc.cu)
+// tensor-core kernels (flow_tc.cu)
 int tf_internal_flow_block_fwd_tc(const float* y_in, const float* logj_in, const float* feat, int feat_dim, int sn, const float* W1,
                                   const float* b1, const float* W2, const float* b2, const float* W3, const float* b3, const float* W4,
                                   const float* b4, float scale, float offset, int cond, int inverse, int64_t M, float* y_out, float* logj_out,
@@ -443,42 +81,17 @@ int tf_internal_flow_block_bwd_tc(const float* y_in, const float* feat, int feat
                                   const float* W4, float scale, float offset, int cond, int64_t M, const float* saved_h, const float* saved_st,
                                   const float* g_y_out, const float* g_logj, float* g_y_in, float* d_feat, float* dW1, float* db1, float* dW2,
                                   float* db2, float* dW3, float* db3, float* dW4, float* db4, cudaStream_t stream);
-// TF_FLOW_SIMT=1 selects the FP32-pipe kernel below instead of the tcgen05 one (A/B runs; read once per process)
-static bool flow_use_simt() {
-    static int forced = -1;
-    if (forced < 0) { const char* e = getenv("TF_FLOW_SIMT"); forced = (e && e[0] == '1') ? 1 : 0; }
-    return forced == 1;
-}
-
 extern "C" TF_API int tf_flow_block_fwd(const float* y_in, const float* logj_in, const float* feat, int32_t feat_dim, int32_t sn,
                                         const float* W1, const float* b1, const float* W2, const float* b2, const float* W3, const float* b3,
                                         const float* W4, const float* b4, float scale, float offset, int32_t cond, int32_t inverse, int64_t M,
                                         float* y_out, float* logj_out, float* save_h, float* save_st, tf_stream_t stream) {
     if (M == 0) return 0;
-    FlowW w = {W1, b1, W2, b2, W3, b3, W4, b4, feat_dim, scale, offset};
-    if (int e = flow_check(w, sn, cond, M)) return e;
+    if (int e = flow_check({W1, b1, W2, b2, W3, b3, W4, b4, feat_dim}, sn, cond, M)) return e;
     TF_REQUIRE(y_in && feat && y_out && logj_out, "tf_flow_block_fwd: NULL pointer");
-    if (!flow_use_simt()) {
-        TF_REQUIRE((save_h == nullptr) == (save_st == nullptr), "tf_flow_block_fwd: pass both activation buffers or none");
-        tf_internal_flow_block_fwd_tc(y_in, logj_in, feat, feat_dim, sn, W1, b1, W2, b2, W3, b3, W4, b4, scale, offset, cond, inverse, M, y_out,
-                                      logj_out, save_h, save_st, (cudaStream_t)stream);
-        TF_CHECK_LAUNCH("tf_flow_block_fwd (tcgen05)");
-        return 0;
-    }
-    FlowFwdParams p = {w, y_in, logj_in, feat, sn, cond, M, y_out, logj_out};
-    const size_t smem = flow_fwd_smem();
-    const int64_t ntiles = (M + FTILE - 1) / FTILE;
-    const int64_t cap = (int64_t)tf_num_sms() * 2;
-    const int grid = (int)(ntiles < cap ? ntiles : cap);
-    if (inverse) {
-        cudaFuncSetAttribute(flow_block_fwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        flow_block_fwd_kernel<true><<<grid, FTILE, smem, (cudaStream_t)stream>>>(p);
-    } else {
-        cudaFuncSetAttribute(flow_block_fwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        flow_block_fwd_kernel<false><<<grid, FTILE, smem, (cudaStream_t)stream>>>(p);
-    }
-    tf_count_launches(1);
-    TF_CHECK_LAUNCH("tf_flow_block_fwd");
+    TF_REQUIRE((save_h == nullptr) == (save_st == nullptr), "tf_flow_block_fwd: pass both activation buffers or none");
+    if (int e = tf_internal_flow_block_fwd_tc(y_in, logj_in, feat, feat_dim, sn, W1, b1, W2, b2, W3, b3, W4, b4, scale, offset, cond, inverse, M,
+                                              y_out, logj_out, save_h, save_st, (cudaStream_t)stream)) return e;
+    TF_CHECK_LAUNCH("tf_flow_block_fwd (tcgen05)");
     return 0;
 }
 
@@ -488,26 +101,11 @@ extern "C" TF_API int tf_flow_block_bwd(const float* y_in, const float* feat, in
                                         const float* g_y_out, const float* g_logj, float* g_y_in, float* d_feat, float* dW1, float* db1,
                                         float* dW2, float* db2, float* dW3, float* db3, float* dW4, float* db4, tf_stream_t stream) {
     if (M == 0) return 0;
-    FlowW w = {W1, b1, W2, b2, W3, b3, W4, b4, feat_dim, scale, offset};
-    if (int e = flow_check(w, sn, cond, M)) return e;
+    if (int e = flow_check({W1, b1, W2, b2, W3, b3, W4, b4, feat_dim}, sn, cond, M)) return e;
     TF_REQUIRE(y_in && feat && g_y_in && d_feat && dW1 && db1 && dW2 && db2 && dW3 && db3 && dW4 && db4, "tf_flow_block_bwd: NULL pointer");
-    if (saved_h && saved_st) {          // activations kept by the tcgen05 forward: tensor-core adjoint chain, no recompute
-        if (int e = tf_internal_flow_block_bwd_tc(y_in, feat, feat_dim, sn, W1, W2, W3, W4, scale, offset, cond, M, saved_h, saved_st, g_y_out, g_logj,
-                                                  g_y_in, d_feat, dW1, db1, dW2, db2, dW3, db3, dW4, db4, (cudaStream_t)stream)) return e;
-        TF_CHECK_LAUNCH("tf_flow_block_bwd (tcgen05)");
-        return 0;
-    }
-    FlowBwdParams p = {w, y_in, feat, sn, cond, M, g_y_out, g_logj, g_y_in, d_feat, dW1, db1, dW2, db2, dW3, db3, dW4, db4};
-    const size_t smem = flow_bwd_smem();
-    TF_REQUIRE(smem <= 227 * 1024, "tf_flow_block_bwd: shared-memory budget exceeded (%zu bytes)", smem);
-    cudaFuncSetAttribute(flow_block_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    const int64_t ntiles = (M + FTILE - 1) / FTILE;
-    const int grid = (int)(ntiles < tf_num_sms() ? ntiles : tf_num_sms());
-    flow_block_bwd_kernel<<<grid, FTILE, smem, (cudaStream_t)stream>>>(p);
-    tf_count_launches(1);
-    TF_CHECK_LAUNCH("tf_flow_block_bwd");
+    TF_REQUIRE(saved_h && saved_st, "tf_flow_block_bwd: saved_h / saved_st are NULL (keep the activations in tf_flow_block_fwd)");
+    if (int e = tf_internal_flow_block_bwd_tc(y_in, feat, feat_dim, sn, W1, W2, W3, W4, scale, offset, cond, M, saved_h, saved_st, g_y_out, g_logj,
+                                              g_y_in, d_feat, dW1, db1, dW2, db2, dW3, db3, dW4, db4, (cudaStream_t)stream)) return e;
+    TF_CHECK_LAUNCH("tf_flow_block_bwd (tcgen05)");
     return 0;
 }
-
-/* 1 when tf_flow_block_fwd runs on the tcgen05 kernel (which can keep the activations for tf_flow_block_bwd), 0 for the FP32-pipe kernel */
-extern "C" TF_API int tf_flow_block_uses_tensor_cores(void) { return flow_use_simt() ? 0 : 1; }

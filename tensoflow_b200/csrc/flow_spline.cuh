@@ -1,6 +1,6 @@
 // Piecewise-quadratic coupling transform of the TensoFlow sampler (reference network/flow.py:314-525,
 // ElementWisePWQuadraticTransform, K = 10 bins: st = 11 vertex heights + 10 widths): device functions shared by the
-// element-wise kernels (flow.cu) and the fused coupling-block kernels (flow.cu, flow_tc.cu).
+// element-wise kernels (flow.cu) and the fused coupling-block kernels (flow_tc.cu).
 #pragma once
 #include <float.h>
 #include "common.cuh"

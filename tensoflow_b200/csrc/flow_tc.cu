@@ -1,14 +1,13 @@
 // Fused coupling block of the TensoFlow sampler on the 5th-gen tensor cores (tcgen05 + TMEM), sm_100a.
 //
-// Same contract as flow_block_fwd_kernel in flow.cu (reference network/flow.py:549-641), but the conditioner chain
-// [PE(y_c) | feature] -> 64 -> 64 -> 64 -> 21 of a tile of 128 (point, direction) pairs runs as four small GEMMs whose A operand
+// Contract: tf_flow_block_fwd / tf_flow_block_bwd (include/tensoflow_b200.h, reference network/flow.py:549-641).  The conditioner
+// chain [PE(y_c) | feature] -> 64 -> 64 -> 64 -> 21 of a tile of 128 (point, direction) pairs runs as four small GEMMs whose A operand
 // never leaves the SM: thread t owns pair t = TMEM lane t; after each layer the accumulator D [128 x 64] is read back
 // (tcgen05.ld), bias + LeakyReLU applied, split into tf32 hi | lo and written to TENSOR MEMORY (tcgen05.st) as the A
 // operand of the next layer's TS-mode MMAs (3xTF32: hi.hi + hi.lo + lo.hi, fp32-level accuracy).  The weights sit in shared
 // memory pre-split in the K-major no-swizzle UMMA layout for the whole kernel (84 KB), the per-point feature part of the first
 // layer is added as a per-row bias, the spline runs on the 21 outputs of the last layer in registers.
 // Two CTAs share an SM (256 TMEM columns each) so that one CTA's epilogue overlaps the other's MMAs.
-// The FFMA kernel this replaces spent its time on broadcast LDS.128 of the weights (one per 4 FMAs, ~21 % of the FP32 peak).
 #include "common.cuh"
 #include "tc_common.cuh"
 #include "flow_spline.cuh"

@@ -11,7 +11,6 @@
 //   hidden   : processed in chunks of NC=32 units; thread (s = tid/16, tx = tid%16) owns
 //              the 7 stencil rows of sample s x 2 hidden units -> the stencil is thread local
 //   GEMM2    : centre rows only ([16][NC] x [NC][A]); taps need output 0 only (a dot product)
-#include <stdlib.h>
 #include "common.cuh"
 
 namespace {
@@ -444,14 +443,15 @@ __global__ void __launch_bounds__(NT, 1) sdf_stencil_bwd_kernel(StencilParams p)
     if (threadIdx.x == 0 && accb1[0] != 0.f) atomicAdd(p.db1, accb1[0]);
 }
 
-struct Dims { int C, K, KP, KS, H, A; };
+struct Dims { int C, K, KP, KS, KT, H, A; };   // KT: K rounded up to the tensor-core K slice (16)
 
 int check_mlp(const tf_vm_field_t* f, const tf_sdf_mlp_t* m, Dims& d) {
     TF_REQUIRE(m && m->W0 && m->b0 && m->W1 && m->b1, "MLP descriptor / weights are NULL");
     TF_REQUIRE(m->hidden > 0 && m->hidden % NC == 0, "hidden must be a multiple of %d (got %d)", NC, m->hidden);
     TF_REQUIRE(m->app_dim >= 4 && m->app_dim % 4 == 0 && m->app_dim <= 128, "app_dim must be a multiple of 4 in [4,128] (got %d)", m->app_dim);
     TF_REQUIRE(f->n_comp <= 36, "n_comp <= 36 supported by the fused stencil (got %d)", f->n_comp);
-    d.C = f->n_comp; d.K = 3 * d.C + 3; d.KP = round_up4(d.K); d.KS = d.KP + 4; d.H = m->hidden; d.A = m->app_dim;
+    d.C = f->n_comp; d.K = 3 * d.C + 3; d.KP = round_up4(d.K); d.KS = d.KP + 4; d.KT = (d.K + 15) / 16 * 16;
+    d.H = m->hidden; d.A = m->app_dim;
     return 0;
 }
 
@@ -484,23 +484,32 @@ size_t tf_internal_linear_tc_ws_floats(int K, int N);
 int tf_internal_linear_tc(const float* X, const float* W, int ldw, int trans, const float* bias, int64_t M, int K, int N, int act, float act_p,
                           float* Y, float* wtc, cudaStream_t stream);
 // tensor-core forward (sdf_stencil_tc.cu)
-size_t tf_internal_tc_fwd_smem(int KT, int H);
+bool tf_internal_stencil_fwd_tc_ok(int KT, int H);
 size_t tf_internal_tc_w0_floats(int KT, int H);
 int tf_internal_stencil_fwd_tc(const tf_vm_field_t* f, const tf_sdf_mlp_t* m, const float* xyz, const float* level, int64_t n,
                                const float units[3], int nq, float* sdf7, float* grad, float* hess, float* sdf1, float* spc,
                                float* w0tc, cudaStream_t stream);
-// TF_STENCIL_SIMT=1 selects the fp32 FFMA kernels below instead of the tcgen05 path (A/B testing only)
-static bool use_simt_path(const Dims& d) {
-    static int forced = -1;
-    if (forced < 0) { const char* e = getenv("TF_STENCIL_SIMT"); forced = (e && e[0] == '1') ? 1 : 0; }
-    const int KT = (d.K + 15) / 16 * 16;
-    return forced == 1 || tf_internal_tc_fwd_smem(KT, d.H) > 227 * 1024 || KT > 128 || d.H > 256 || d.H % 32 != 0;
-}
+// tensor-core backward (sdf_stencil_bwd_tc.cu)
+size_t tf_internal_bwd_tc_smem(int KT, int H);
+size_t tf_internal_bwd_tc_wtc_floats(int KT, int H);
+int tf_internal_bwd_tc_prep(const float* W0, int K, int KT, int H, float* wtc, cudaStream_t stream);
+int tf_internal_bwd_tc_samples_per_tile();
+int tf_internal_bwd_tc_fold(const float* tmp, int H, int K, int KT, float* dW0, float* db0, cudaStream_t stream);
+int tf_internal_stencil_bwd_tc(const tf_vm_field_t* f, const tf_vm_mut_t* g, const tf_sdf_mlp_t* m, const float* wtc, const float* xyz,
+                               const float* level, int64_t n, const float units[3], const float* sdf7, const float* g_sdf,
+                               const float* g_grad, const float* g_hess, const float* dHc, float* dpre, float* arow,
+                               float* da_scratch, float* dW1r0, float* db1, cudaStream_t stream);
+size_t tf_internal_bwd_tc_scratch_floats(int KT);
+
+// Which decoder shapes run on the tcgen05 kernels; the FFMA kernels above take the others (hidden > 256).  check_mlp and
+// tf_check_field already bound the rest: hidden % 32 == 0, n_comp % 4 == 0 and n_comp <= 36, so KT <= 112.
+static bool fwd_on_tc(const Dims& d) { return tf_internal_stencil_fwd_tc_ok(d.KT, d.H); }
+// the tcgen05 backward reads the centre hidden activations that the tcgen05 forward kept
+static bool bwd_on_tc(const Dims& d) { return fwd_on_tc(d) && tf_internal_bwd_tc_smem(d.KT, d.H) <= 227 * 1024; }
 
 static size_t fwd_ws_floats(const Dims& d, int64_t n, bool with_feat) {
-    if (use_simt_path(d)) return weights_ws_floats(d);
-    const int KT = (d.K + 15) / 16 * 16;
-    return tf_internal_tc_w0_floats(KT, d.H) + (with_feat ? (size_t)(n < 1 ? 1 : n) * d.H + tf_internal_linear_tc_ws_floats(d.H, d.A) : 0);
+    if (!fwd_on_tc(d)) return weights_ws_floats(d);
+    return tf_internal_tc_w0_floats(d.KT, d.H) + (with_feat ? (size_t)(n < 1 ? 1 : n) * d.H + tf_internal_linear_tc_ws_floats(d.H, d.A) : 0);
 }
 
 extern "C" TF_API size_t tf_sdf_stencil_fwd_workspace(const tf_vm_field_t* f, const tf_sdf_mlp_t* m, int64_t n, int32_t with_feat) {
@@ -521,11 +530,10 @@ static int stencil_fwd_impl(int mode, const tf_vm_field_t* f, const tf_sdf_mlp_t
     TF_REQUIRE(((uintptr_t)workspace & 15) == 0, "workspace not 16-byte aligned");
     if (feat) TF_REQUIRE(((uintptr_t)feat & 15) == 0, "feat not 16-byte aligned");
     cudaStream_t stream = (cudaStream_t)stream_;
-    if (!use_simt_path(d)) {
+    if (fwd_on_tc(d)) {
         // tcgen05 path: first layer on the tensor cores, appearance head as one more linear layer
-        const int KT = (d.K + 15) / 16 * 16;
         float* w0tc = (float*)workspace;
-        float* spc = feat ? w0tc + tf_internal_tc_w0_floats(KT, d.H) : nullptr;
+        float* spc = feat ? w0tc + tf_internal_tc_w0_floats(d.KT, d.H) : nullptr;
         if (mode == 0) TF_REQUIRE(sdf7, "sdf7 is NULL"); else TF_REQUIRE(sdf1, "sdf is NULL");
         if (int e = tf_internal_stencil_fwd_tc(f, m, xyz, level, n, units, mode == 0 ? 7 : 1, sdf7, grad, hess, sdf1, spc, w0tc, stream)) return e;
         if (feat) {
@@ -581,8 +589,8 @@ extern "C" TF_API int tf_sdf_point_fwd(const tf_vm_field_t* f, const tf_sdf_mlp_
     if (!f || !m) { tf_set_error("tf_sdf_point_fwd: NULL descriptor"); return 1; }
     if (int e = check_mlp(f, m, d)) return e;
     TF_REQUIRE(feat, "tf_sdf_point_fwd: feat is NULL (use tf_sdf_only_fwd for the SDF alone)");
-    TF_REQUIRE(!use_simt_path(d), "tf_sdf_point_fwd: only the tensor-core path evaluates single queries with features "
-                                  "(hidden %% 32 == 0, hidden <= 256); use tf_sdf_stencil_fwd");
+    TF_REQUIRE(fwd_on_tc(d), "tf_sdf_point_fwd: only the tensor-core path evaluates single queries with features "
+                             "(hidden <= 256); use tf_sdf_stencil_fwd");
     return stencil_fwd_impl(1, f, m, xyz, level, n, nullptr, nullptr, feat, nullptr, nullptr, sdf, workspace, ws_bytes, stream);
 }
 
@@ -591,17 +599,6 @@ static size_t bwd_slice_floats(const Dims& d, int64_t n_slice) {
     return (size_t)tiles * ((size_t)R * d.H + (size_t)R * d.KP + (size_t)TS * d.H);
 }
 
-// tensor-core backward (sdf_stencil_bwd_tc.cu)
-size_t tf_internal_bwd_tc_wtc_floats(int KT, int H);
-size_t tf_internal_bwd_tc_smem(int KT, int H);
-int tf_internal_bwd_tc_prep(const float* W0, int K, int KT, int H, float* wtc, cudaStream_t stream);
-int tf_internal_bwd_tc_samples_per_tile();
-int tf_internal_bwd_tc_fold(const float* tmp, int H, int K, int KT, float* dW0, float* db0, cudaStream_t stream);
-int tf_internal_stencil_bwd_tc(const tf_vm_field_t* f, const tf_vm_mut_t* g, const tf_sdf_mlp_t* m, const float* wtc, const float* xyz,
-                               const float* level, int64_t n, const float units[3], const float* sdf7, const float* g_sdf,
-                               const float* g_grad, const float* g_hess, const float* dHc, float* dpre, float* arow, float* spc,
-                               float* da_scratch, float* dW1r0, float* db1, cudaStream_t stream);
-size_t tf_internal_bwd_tc_scratch_floats(int KT);
 int tf_internal_xty(const float* X, int ldx, const float* Y, int ldy, int64_t rows, int M, int N, float* out, int ldo, cudaStream_t stream);
 int tf_internal_colsum(const float* X, int ldx, int64_t rows, int cols, float* out, cudaStream_t stream);
 int tf_internal_matmul(const float* A, int lda, const float* W, int ldw, int64_t M, int Kred, int Nout, float* out, int ldo,
@@ -611,27 +608,21 @@ int tf_internal_xty_tc(const float* X, const float* Y, int64_t rows, int M, int 
 int tf_internal_xty_tc_tiled(const float* X, const float* Y, int64_t rows, int M, int N, float* out, int ldo, int n_valid, int x_tiled,
                              cudaStream_t stream);
 
-static bool use_simt_bwd(const Dims& d) {
-    const int KT = (d.K + 15) / 16 * 16;
-    return use_simt_path(d) || d.C % 4 != 0 || KT > 128 /* dA accumulator + TMEM chunk operands share 256 columns */ || tf_internal_bwd_tc_smem(KT, d.H) > 227 * 1024;
-}
 // tensor-core backward workspace: [W slices | dW0/db0 staging | per tile of 18 samples: dPre [128,H], A rows [128,KT],
-// centre hidden [18,H], dHidden(centre) [18,H]]
+// dHidden(centre) [18,H]]
 static size_t bwd_tc_fixed_floats(const Dims& d) {
-    const int KT = (d.K + 15) / 16 * 16;
-    return tf_internal_bwd_tc_wtc_floats(KT, d.H) + (size_t)d.H * KT + tf_internal_linear_tc_ws_floats(d.A, d.H) +
-           tf_internal_bwd_tc_scratch_floats(KT);
+    return tf_internal_bwd_tc_wtc_floats(d.KT, d.H) + (size_t)d.H * d.KT + tf_internal_linear_tc_ws_floats(d.A, d.H) +
+           tf_internal_bwd_tc_scratch_floats(d.KT);
 }
 static size_t bwd_tc_tile_floats(const Dims& d) {
-    const int KT = (d.K + 15) / 16 * 16, spt = tf_internal_bwd_tc_samples_per_tile();
-    return (size_t)128 * (d.H + KT) + 2 * (size_t)spt * d.H;
+    return (size_t)128 * (d.H + d.KT) + (size_t)tf_internal_bwd_tc_samples_per_tile() * d.H;
 }
 
 extern "C" TF_API size_t tf_sdf_stencil_bwd_workspace(const tf_vm_field_t* f, const tf_sdf_mlp_t* m, int64_t n_slice) {
     Dims d;
     if (!f || !m || check_mlp(f, m, d)) return 0;
     if (n_slice < 1) n_slice = 1;
-    if (!use_simt_bwd(d)) {
+    if (bwd_on_tc(d)) {
         const int spt = tf_internal_bwd_tc_samples_per_tile();
         return (bwd_tc_fixed_floats(d) + (size_t)((n_slice + spt - 1) / spt) * bwd_tc_tile_floats(d)) * sizeof(float);
     }
@@ -642,7 +633,7 @@ static int stencil_bwd_tc(const tf_vm_field_t* f, const tf_sdf_mlp_t* m, const D
                           const float units[3], const float* sdf7, const float* g_sdf, const float* g_feat, const float* g_grad,
                           const float* g_hess, const tf_vm_mut_t* g_field, const tf_sdf_mlp_grad_t* g_mlp, float* ws, size_t ws_floats,
                           const float* hidden_c, cudaStream_t stream) {
-    const int KT = (d.K + 15) / 16 * 16, H = d.H;
+    const int KT = d.KT, H = d.H;
     const int spt = tf_internal_bwd_tc_samples_per_tile();
     const size_t fixed = bwd_tc_fixed_floats(d), per_tile = bwd_tc_tile_floats(d);
     TF_REQUIRE(ws_floats >= fixed + per_tile, "workspace too small (%zu bytes)", ws_floats * sizeof(float));
@@ -655,8 +646,7 @@ static int stencil_bwd_tc(const tf_vm_field_t* f, const tf_sdf_mlp_t* m, const D
     float* da_scratch = wlin + tf_internal_linear_tc_ws_floats(d.A, H);
     float* dpre = da_scratch + tf_internal_bwd_tc_scratch_floats(KT);
     float* arow = dpre + (size_t)tiles_fit * 128 * H;
-    float* spc = arow + (size_t)tiles_fit * 128 * KT;
-    float* dHc = spc + (size_t)tiles_fit * spt * H;
+    float* dHc = arow + (size_t)tiles_fit * 128 * KT;
     tf_internal_bwd_tc_prep(m->W0, d.K, KT, H, wtc, stream);
     cudaMemsetAsync(tmp, 0, (size_t)H * KT * sizeof(float), stream);
     for (int64_t t0 = 0; t0 < ntiles_all; t0 += tiles_fit) {
@@ -671,7 +661,7 @@ static int stencil_bwd_tc(const tf_vm_field_t* f, const tf_sdf_mlp_t* m, const D
         }
         if (int e = tf_internal_stencil_bwd_tc(f, g_field, m, wtc, xyz + s0 * 3, level ? level + s0 : nullptr, ns, units, sdf7 + s0 * NQ,
                                                g_sdf ? g_sdf + s0 : nullptr, g_grad ? g_grad + s0 * 3 : nullptr,
-                                               g_hess ? g_hess + s0 : nullptr, gf ? dHc : nullptr, dpre, arow, (gf && !hidden_c) ? spc : nullptr,
+                                               g_hess ? g_hess + s0 : nullptr, gf ? dHc : nullptr, dpre, arow,
                                                da_scratch, g_mlp->W1, g_mlp->b1, stream))
             return e;
         // [dW0 | db0] staging += dPre^T [A | 1]; the kernel wrote dPre per tile as [H][128] (row fastest: coalesced stores there,
@@ -679,8 +669,8 @@ static int stencil_bwd_tc(const tf_vm_field_t* f, const tf_sdf_mlp_t* m, const D
         TF_REQUIRE(tf_internal_xty_tc_ok(dpre, arow, H, KT), "tensor-core X^T Y does not take this decoder shape (H=%d, KT=%d)", H, KT);
         if (int e = tf_internal_xty_tc_tiled(dpre, arow, nt * 128, H, KT, tmp, KT, d.K + 1, 1, stream)) return e;
         if (gf) {
-            // centre hidden activations: kept from the forward call when the caller has them, else recomputed by the kernel above
-            const float* hid = hidden_c ? hidden_c + s0 * H : spc;
+            // centre hidden activations kept from the forward call
+            const float* hid = hidden_c + s0 * H;
             if (tf_internal_xty_tc_ok(gf, hid, d.A, H)) tf_internal_xty_tc(gf, hid, ns, d.A, H, g_mlp->W1 + H, H, H, stream);
             else tf_internal_xty(gf, d.A, hid, H, ns, d.A, H, g_mlp->W1 + H, H, stream);
             tf_internal_colsum(gf, d.A, ns, d.A, g_mlp->b1 + 1, stream);
@@ -692,26 +682,17 @@ static int stencil_bwd_tc(const tf_vm_field_t* f, const tf_sdf_mlp_t* m, const D
 }
 
 // byte offset of the centre hidden activations [n, hidden] inside the workspace of tf_sdf_stencil_fwd(.., feat != NULL);
-// (size_t)-1 when the forward path for this shape does not produce them
+// (size_t)-1 exactly when the tcgen05 forward does not apply to this shape (the FFMA forward does not keep them)
 extern "C" TF_API size_t tf_sdf_stencil_fwd_hidden_offset(const tf_vm_field_t* f, const tf_sdf_mlp_t* m) {
     Dims d;
-    if (!f || !m || check_mlp(f, m, d) || use_simt_path(d)) return (size_t)-1;
-    const int KT = (d.K + 15) / 16 * 16;
-    return tf_internal_tc_w0_floats(KT, d.H) * sizeof(float);
+    if (!f || !m || check_mlp(f, m, d) || !fwd_on_tc(d)) return (size_t)-1;
+    return tf_internal_tc_w0_floats(d.KT, d.H) * sizeof(float);
 }
 
 extern "C" TF_API int tf_sdf_stencil_bwd(const tf_vm_field_t* f, const tf_sdf_mlp_t* m, const float* xyz, const float* level,
-                                  int64_t n, const float units[3], const float* sdf7, const float* g_sdf, const float* g_feat,
-                                  const float* g_grad, const float* g_hess, const tf_vm_mut_t* g_field,
+                                  int64_t n, const float units[3], const float* sdf7, const float* hidden_centre, const float* g_sdf,
+                                  const float* g_feat, const float* g_grad, const float* g_hess, const tf_vm_mut_t* g_field,
                                   const tf_sdf_mlp_grad_t* g_mlp, void* workspace, size_t ws_bytes, tf_stream_t stream_) {
-    return tf_sdf_stencil_bwd_kept(f, m, xyz, level, n, units, sdf7, nullptr, g_sdf, g_feat, g_grad, g_hess, g_field, g_mlp, workspace, ws_bytes,
-                                   stream_);
-}
-
-extern "C" TF_API int tf_sdf_stencil_bwd_kept(const tf_vm_field_t* f, const tf_sdf_mlp_t* m, const float* xyz, const float* level,
-                                       int64_t n, const float units[3], const float* sdf7, const float* hidden_centre, const float* g_sdf,
-                                       const float* g_feat, const float* g_grad, const float* g_hess, const tf_vm_mut_t* g_field,
-                                       const tf_sdf_mlp_grad_t* g_mlp, void* workspace, size_t ws_bytes, tf_stream_t stream_) {
     if (int e = tf_check_field(f, level != nullptr)) return e;
     Dims d;
     if (int e = check_mlp(f, m, d)) return e;
@@ -727,10 +708,13 @@ extern "C" TF_API int tf_sdf_stencil_bwd_kept(const tf_vm_field_t* f, const tf_s
     cudaStream_t stream = (cudaStream_t)stream_;
     float* ws = (float*)workspace;
     TF_REQUIRE(workspace, "workspace is NULL");
-    if (hidden_centre) TF_REQUIRE(((uintptr_t)hidden_centre & 15) == 0, "hidden_centre not 16-byte aligned");
-    if (!use_simt_bwd(d))
+    if (bwd_on_tc(d)) {
+        TF_REQUIRE(hidden_centre || !g_feat, "tf_sdf_stencil_bwd: hidden_centre is NULL (keep the forward workspace: "
+                                             "tf_sdf_stencil_fwd_hidden_offset)");
+        TF_REQUIRE(((uintptr_t)hidden_centre & 15) == 0, "hidden_centre not 16-byte aligned");
         return stencil_bwd_tc(f, m, d, xyz, level, n, units, sdf7, g_sdf, g_feat, g_grad, g_hess, g_field, g_mlp, ws,
                               ws_bytes / sizeof(float), hidden_centre, stream);
+    }
     const size_t wfl = weights_ws_floats(d);
     TF_REQUIRE(ws_bytes >= (wfl + bwd_slice_floats(d, TS)) * sizeof(float), "workspace too small (%zu bytes)", ws_bytes);
     // samples per slice that fit the workspace (multiple of TS)

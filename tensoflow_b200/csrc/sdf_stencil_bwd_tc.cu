@@ -13,7 +13,7 @@
 // Hand-offs are mbarriers (A ready / GEMM1 done / dA ready / dA consumed); weight slices (W0 by 8 features for GEMM1,
 // W0^T by 16 hidden units for GEMM-dA) stream through one 4-stage cp.async.bulk ring, each stage refilled by its own
 // issuing lane (bulk copies of one warp execute one after the other).  Weight gradients are finished by X^T Y passes
-// over the workspace (xty_tc.cu); the centre hidden activations come from the forward call when the caller kept them.
+// over the workspace (xty_tc.cu); the centre hidden activations come from the forward call, which kept them.
 #include <stdio.h>
 #include <stdlib.h>
 #include "common.cuh"
@@ -46,7 +46,6 @@ struct TcBwdParams {
     float* da_scratch;       // [gridDim][128][KT+4]: dA tiles handed from the math to the memory group through L2
     float* dpre;             // [tiles][H][128] (per tile: column-major, rows fastest)
     float* arow;             // [tiles*128][KT]
-    float* spc;              // [n][H] centre hidden activations (NULL = not needed)
     float* dW1r0; float* db1;
 #ifdef TF_TC_DEBUG_SWITCHES
     long long* prof;         // [3 roles][16] phase cycle totals of CTA 0 (TF_TC_BWD_PROF=1)
@@ -369,12 +368,6 @@ __global__ void __launch_bounds__(NTH, 1) sdf_stencil_bwd_tc_kernel(TcBwdParams 
                     tc::tmem_st_wait();
                 }
                 if (tid != 0) { PROF(13) }
-                if (centre && p.spc) {
-                    float4* sdst = reinterpret_cast<float4*>(p.spc + (size_t)n * H + col0);
-#pragma unroll
-                    for (int j = 0; j < 4; ++j) sdst[j] = make_float4(sp[4 * j], sp[4 * j + 1], sp[4 * j + 2], sp[4 * j + 3]);
-                }
-                if (tid != 0) { PROF(14) }
                 if (!TF_DBG(p, 8)) {
                     // 16 column sums over the warp's 32 rows with 16 shuffles: every exchange halves the columns a lane owns
                     float w8[8], w4[4], w2[2];
@@ -500,7 +493,7 @@ size_t tf_internal_bwd_tc_scratch_floats(int KT) { return (size_t)tf_num_sms() *
 // one slice of samples (n <= workspace capacity): activation-side backward
 int tf_internal_stencil_bwd_tc(const tf_vm_field_t* f, const tf_vm_mut_t* g, const tf_sdf_mlp_t* m, const float* wtc, const float* xyz,
                                const float* level, int64_t n, const float units[3], const float* sdf7, const float* g_sdf,
-                               const float* g_grad, const float* g_hess, const float* dHc, float* dpre, float* arow, float* spc,
+                               const float* g_grad, const float* g_hess, const float* dHc, float* dpre, float* arow,
                                float* da_scratch, float* dW1r0, float* db1, cudaStream_t stream) {
     const int C = f->n_comp, K = 3 * C + 3, KT = (K + KSL - 1) / KSL * KSL, H = m->hidden;
     TcBwdParams p = {};
@@ -509,7 +502,7 @@ int tf_internal_stencil_bwd_tc(const tf_vm_field_t* f, const tf_vm_mut_t* g, con
     p.sdf7 = sdf7; p.g_sdf = g_sdf; p.g_grad = g_grad; p.g_hess = g_hess; p.dHc = dHc;
     p.K = K; p.KT = KT; p.H = H; p.slot_floats = tf_internal_bwd_tc_slot_floats(KT, H);
     for (int k = 0; k < 3; ++k) p.units[k] = units[k];
-    p.dpre = dpre; p.arow = arow; p.spc = spc; p.da_scratch = da_scratch; p.dW1r0 = dW1r0; p.db1 = db1;
+    p.dpre = dpre; p.arow = arow; p.da_scratch = da_scratch; p.dW1r0 = dW1r0; p.db1 = db1;
 #ifdef TF_TC_DEBUG_SWITCHES
     { const char* e = getenv("TF_TC_BWD_DEBUG"); p.debug = e ? atoi(e) : 0; }
     static long long* prof_dev = nullptr;

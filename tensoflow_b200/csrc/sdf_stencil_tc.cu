@@ -331,11 +331,14 @@ __global__ void __launch_bounds__(NTH, 1) sdf_stencil_fwd_tc_kernel(TcParams p) 
     if (warp == 0) tc::tmem_dealloc<512>(tmem_base);
 }
 
-}  // namespace
-
-size_t tf_internal_tc_fwd_smem(int KT, int H) {
+size_t tc_fwd_smem(int KT, int H) {
     return (size_t)16 * (KT / 4) * site::A_LBO + (size_t)NST * 2 * H * KSL * 4 + (size_t)2 * H * 4 + (size_t)2 * NCG * TM * 4 + (2 * NST + 2) * 8 + 16;
 }
+}  // namespace
+
+// the decoder shapes this kernel takes: the GEMM1 accumulator holds at most 256 hidden columns of TMEM, and the tile must fit
+// shared memory.  sdf_stencil.cu dispatches on this predicate; the launcher below re-checks it.
+bool tf_internal_stencil_fwd_tc_ok(int KT, int H) { return H <= 256 && tc_fwd_smem(KT, H) <= 227 * 1024; }
 
 // workspace floats needed in front of spc: the pre-tiled W0
 size_t tf_internal_tc_w0_floats(int KT, int H) { return (size_t)KT * H * 2; }
@@ -353,9 +356,12 @@ int tf_internal_stencil_fwd_tc(const tf_vm_field_t* f, const tf_sdf_mlp_t* m, co
 #ifdef TF_TC_DEBUG_SWITCHES
     { const char* e = getenv("TF_TC_DEBUG"); p.debug = e ? atoi(e) : 0; }
 #endif
+    if (!tf_internal_stencil_fwd_tc_ok(KT, H) || f->n_levels > site::MAXL) {
+        tf_set_error("tensor-core stencil: tile does not fit shared / tensor memory (KT=%d, H=%d)", KT, H);
+        return 1;
+    }
     tc_prep_w0_kernel<<<64, 256, 0, stream>>>(m->W0, K, KT, H, w0tc);
-    const size_t smem = tf_internal_tc_fwd_smem(KT, H);
-    if (smem > 227 * 1024 || KT > 128 || H > 256 || f->n_levels > site::MAXL) { tf_set_error("tensor-core stencil: tile does not fit shared / tensor memory (KT=%d, H=%d)", KT, H); return 1; }
+    const size_t smem = tc_fwd_smem(KT, H);
     cudaFuncSetAttribute(sdf_stencil_fwd_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     const int spt = nq == NQ7 ? site::SPT : TM;
     const int64_t ntiles = (n + spt - 1) / spt;

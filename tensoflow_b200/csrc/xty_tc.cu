@@ -277,12 +277,12 @@ int tf_internal_xty_tc_tiled(const float* X, const float* Y, int64_t rows, int M
 int tf_internal_xty(const float* X, int ldx, const float* Y, int ldy, int64_t rows, int M, int N, float* out, int ldo, cudaStream_t stream);
 
 extern "C" TF_API int tf_xty_accumulate(const float* X, const float* Y, int64_t rows, int32_t M, int32_t N, float* out,
-                                        int32_t force_simt, tf_stream_t stream_) {
+                                        tf_stream_t stream_) {
     if (rows == 0) return 0;
     TF_REQUIRE(X && Y && out && M > 0 && N > 0, "tf_xty_accumulate: NULL pointer or bad shape (%d,%d)", M, N);
     cudaStream_t stream = (cudaStream_t)stream_;
-    if (!force_simt && tf_internal_xty_tc_ok(X, Y, M, N)) tf_internal_xty_tc(X, Y, rows, M, N, out, N, N, stream);
-    else tf_internal_xty(X, M, Y, N, rows, M, N, out, N, stream);
+    if (int e = tf_internal_xty_tc_ok(X, Y, M, N) ? tf_internal_xty_tc(X, Y, rows, M, N, out, N, N, stream)
+                                                  : tf_internal_xty(X, M, Y, N, rows, M, N, out, N, stream)) return e;
     TF_CHECK_LAUNCH("tf_xty_accumulate");
     return 0;
 }

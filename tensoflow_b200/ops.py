@@ -228,10 +228,6 @@ def _units_arr(units) -> C.Array:
     return (C.c_float * 3)(*u)
 
 
-# keep the forward's centre hidden activations for the backward (False: the backward recomputes them, 4 n H bytes less between the two)
-KEEP_HIDDEN = True
-
-
 class SdfStencilFunction(torch.autograd.Function):
     """TensoSDF.forward at x plus the six FD taps of TensoSDF.gradient
     (reference network/fields.py:262-299, 227-260) in one fused kernel.
@@ -268,10 +264,10 @@ class SdfStencilFunction(torch.autograd.Function):
         ctx.save_for_backward(xyz_c, lvl_c, sdf7, aabb, W0, b0, W1, b1, *factors)
         ctx.units = [float(x) for x in units]
         ctx.n_levels = n_levels
-        # the centre hidden activations sit in the forward workspace: keep it for the backward (4 n H bytes) so that the backward
-        # kernel does not recompute and store them again (they feed the weight gradient of the appearance head)
+        # the centre hidden activations sit in the forward workspace: keep it for the backward (4 n H bytes), which reads them
+        # (they feed the weight gradient of the appearance head)
         ctx.hidden = None
-        if KEEP_HIDDEN and any(ctx.needs_input_grad):
+        if any(ctx.needs_input_grad):
             off = lib.tf_sdf_stencil_fwd_hidden_offset(C.byref(vm.c), C.byref(m))
             if off != C.c_size_t(-1).value:
                 ctx.hidden = (ws, off)
@@ -297,9 +293,9 @@ class SdfStencilFunction(torch.autograd.Function):
         gs, gf, gg, gh = _f32c(g_sdf), _f32c(g_feat), _f32c(g_grad), _f32c(g_hess)
         hid = None if ctx.hidden is None else ctx.hidden[0].data_ptr() + ctx.hidden[1]
         with _timed("sdf_stencil_bwd"):
-            check(lib.tf_sdf_stencil_bwd_kept(C.byref(vm.c), C.byref(m), ptr(xyz_c), ptr(lvl_c), n, _units_arr(ctx.units), ptr(sdf7), hid,
-                                              ptr(gs), ptr(gf), ptr(gg), ptr(gh), C.byref(g), C.byref(mg), ptr(ws), wsb, stream_ptr()),
-                  "tf_sdf_stencil_bwd_kept")
+            check(lib.tf_sdf_stencil_bwd(C.byref(vm.c), C.byref(m), ptr(xyz_c), ptr(lvl_c), n, _units_arr(ctx.units), ptr(sdf7), hid,
+                                         ptr(gs), ptr(gf), ptr(gg), ptr(gh), C.byref(g), C.byref(mg), ptr(ws), wsb, stream_ptr()),
+                  "tf_sdf_stencil_bwd")
         ctx.hidden = None
         d_planes, d_lines = vm.finish_grads(g, gp, gl, with_mips)
         return (None, None, None, None, None, dW0, db0, dW1, db1, *d_planes, *d_lines)
@@ -327,14 +323,13 @@ def sdf_point(xyz, level, aabb, n_levels, W0, b0, W1, b1, planes, lines):
     """TensoSDF.forward (reference network/fields.py:262-299) without autograd and without the FD taps -> (sdf [N], feat [N,A]);
     None when the decoder shape is outside the tensor-core path (the caller then uses the stencil)."""
     lib = _lib.load()
-    H = int(W0.shape[0])
-    if H % 32 != 0 or H > 256 or __import__('os').environ.get('TF_STENCIL_SIMT') == '1':
-        return None
     xyz_c = _f32c(xyz.reshape(-1, 3))
     lvl_c = None if level is None else _f32c(level.reshape(-1))
     n = xyz_c.shape[0]
     vm = vm_desc(planes, lines, aabb, n_levels, lvl_c is not None)
     m, keep = _mlp_desc(W0, b0, W1, b1)
+    if lib.tf_sdf_stencil_fwd_hidden_offset(C.byref(vm.c), C.byref(m)) == C.c_size_t(-1).value:
+        return None
     sdf = torch.empty(n, device=xyz_c.device, dtype=torch.float32)
     feat = torch.empty(n, m.app_dim, device=xyz_c.device, dtype=torch.float32)
     if n == 0:
@@ -631,7 +626,7 @@ class FlowBlockFunction(torch.autograd.Function):
         lj_out = torch.empty(M, device=yc.device, dtype=torch.float32)
         # density direction with gradients: the tensor-core forward keeps h1, h2, h3 and the spline parameters (864 B per pair),
         # so that the backward is the adjoint chain alone
-        keep = (not inverse) and any(ctx.needs_input_grad) and lib.tf_flow_block_uses_tensor_cores() == 1
+        keep = (not inverse) and any(ctx.needs_input_grad)
         sh = torch.empty(M, 3, 64, device=yc.device, dtype=torch.float32) if keep else None
         sst = torch.empty(M, 24, device=yc.device, dtype=torch.float32) if keep else None
         with _timed("flow_block_fwd"):

@@ -27,9 +27,21 @@ def test_header_symbols_exported(lib):
     assert declared == set(_lib.exported_symbols()), declared ^ set(_lib.exported_symbols())
 
 
-def test_abi_version_and_error_string(lib):
-    assert lib.tf_abi_version() == 1
+def test_abi_version_2_and_error_string(lib):
+    """ABI 2: tf_sdf_stencil_bwd takes hidden_centre, tf_xty_accumulate has no force_simt, two entries are gone."""
+    assert lib.tf_abi_version() == 2
     assert isinstance(lib.tf_last_error(), bytes)
+
+
+def test_flow_block_bwd_requires_kept_activations(lib):
+    """tf_flow_block_bwd without the activations kept by the forward (saved_h / saved_st) returns an error before any launch.
+    The addresses are fake: the check fires before anything is dereferenced."""
+    fake, M, sn, F = ctypes.c_void_p(1 << 20), 64, 16, 8
+    launches = lib.tf_launch_count()
+    rc = lib.tf_flow_block_bwd(*(fake,) * 2, F, sn, *(fake,) * 8, 2.0, -1.0, 0, M, None, None, None, None, *(fake,) * 10, None)
+    assert rc != 0
+    assert b"saved_h" in lib.tf_last_error()
+    assert lib.tf_launch_count() == launches
 
 
 def test_no_cpu_fallback():

@@ -35,9 +35,11 @@ def test_tcgen05_gemm_matches_fp64(N, K, a_mode, a_lbo):
     assert e3 < 2e-6, e3          # split: fp32 level
 
 
-@pytest.mark.parametrize("rows,M,N", [(1000, 256, 112), (4099, 128, 256), (31, 128, 16), (20000, 256, 64), (9000, 256, 256), (5000, 48, 240)])
+@pytest.mark.parametrize("rows,M,N", [(1000, 256, 112), (4099, 128, 256), (31, 128, 16), (20000, 256, 64), (9000, 256, 256), (5000, 48, 240),
+                                      (5000, 40, 240), (3001, 96, 300)])
 def test_xty_tensor_core_matches_fp64(rows, M, N):
-    """dW = X^T Y on tcgen05 with MN-major operands straight from row-major HBM tensors."""
+    """dW = X^T Y on tcgen05 with MN-major operands straight from row-major HBM tensors; the last two shapes (M % 16 != 0,
+    N > 256) run on the FFMA kernel."""
     if not torch.cuda.is_available():
         pytest.skip("no CUDA device")
     from tensoflow_b200 import _lib
@@ -47,15 +49,12 @@ def test_xty_tensor_core_matches_fp64(rows, M, N):
     X = torch.randn(rows, M, generator=g).to(dev)
     Y = torch.randn(rows, N, generator=g).to(dev)
     ref = X.double().T @ Y.double()
-    outs = []
-    for force_simt in (0, 1):
-        out = torch.ones(M, N, device=dev)
-        check(_lib.load().tf_xty_accumulate(ptr(X), ptr(Y), rows, M, N, ptr(out), force_simt, stream_ptr()), "tf_xty_accumulate")
-        torch.cuda.synchronize()
-        outs.append(out)
-        e = float((out.double() - 1 - ref).abs().max() / ref.abs().max())
-        print(f"rows={rows} M={M} N={N} simt={force_simt}: {e:.2e}")
-        assert e < 5e-6, e
+    out = torch.ones(M, N, device=dev)
+    check(_lib.load().tf_xty_accumulate(ptr(X), ptr(Y), rows, M, N, ptr(out), stream_ptr()), "tf_xty_accumulate")
+    torch.cuda.synchronize()
+    e = float((out.double() - 1 - ref).abs().max() / ref.abs().max())
+    print(f"rows={rows} M={M} N={N}: {e:.2e}")
+    assert e < 5e-6, e
 
 
 @pytest.mark.parametrize("M,K,N,act", [(20000, 123, 256, "relu"), (9000, 256, 99, "exp"), (10000, 108, 128, "sigmoid"),
