@@ -214,6 +214,25 @@ TF_API void tf_bvh_destroy(tf_bvh_t* handle);
 TF_API int tf_bvh_trace(const tf_bvh_t* handle, const float* rays_o, const float* rays_d, int64_t n,
                         float* positions, float* face_normals, float* depth, tf_stream_t stream);
 
+/* ---- geometry evaluation (point-to-mesh distances, surface samples) ----------------------------
+ * tf_bvh_closest_point: for each of the n query points [n,3], the nearest point of the mesh behind `handle`:
+ *   out_points [n,3] (fp32), out_dist [n] (Euclidean, fp32), out_tri [n] (int64 index into the triangles given to
+ *   tf_bvh_create, in the caller's order).  Branch-and-bound over the BVH; per triangle Ericson's 7-region test
+ *   (Real-Time Collision Detection 5.1.5) in fp32; a triangle whose height is below 2^-24 of its longest edge (zero area,
+ *   collinear) is measured through its edges and vertices.  The smaller squared distance wins, an exact tie goes to the
+ *   smaller triangle index; no atomics, so two runs are bit-identical.  A query point with a NaN coordinate gives out_tri = -1.
+ * tf_mesh_sample_surface: n area-weighted samples of the mesh vertices [V,3] fp32 / triangles [n_tris,3] int32 (indices in
+ *   range, the caller checks).  cdf [n_tris] fp64 is the inclusive, normalised cumulative triangle area (last element 1);
+ *   uniforms [n,3] fp64 in [0,1): triangle t = the first with cdf[t] > u0 (binary search), point
+ *   (1 - sqrt(u1)) a + sqrt(u1)(1 - u2) b + sqrt(u1) u2 c evaluated in fp64 and rounded once; out_points [n,3] fp32,
+ *   out_tri [n] int64, out_normals [n,3] fp32 = unit (b - a) x (c - a).
+ * Both: n == 0 launches nothing; no allocation, no synchronisation. */
+TF_API int tf_bvh_closest_point(const tf_bvh_t* handle, const float* points, int64_t n, float* out_points, float* out_dist,
+                                int64_t* out_tri, tf_stream_t stream);
+TF_API int tf_mesh_sample_surface(const float* vertices, const int32_t* triangles, int64_t n_tris, const double* cdf,
+                                  const double* uniforms, int64_t n, float* out_points, int64_t* out_tri, float* out_normals,
+                                  tf_stream_t stream);
+
 /* ---- material-stage Monte-Carlo integral (network/fields.py:1075-1335) -----------------
  * tf_mc_directions builds one direction set per surface point and its pdf:
  *   mode 0: flow samples in the half-vector parametrisation (fields.py:1085-1108,1164-1188)

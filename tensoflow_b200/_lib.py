@@ -81,6 +81,8 @@ _OPTIONAL_SIGNATURES = {
     "tf_bvh_create": (C.c_int, [_P, C.c_int64, _P, C.c_int64, C.POINTER(C.c_void_p)]),
     "tf_bvh_destroy": (None, [_P]),
     "tf_bvh_trace": (C.c_int, [_P, _P, _P, C.c_int64, _P, _P, _P, _P]),
+    "tf_bvh_closest_point": (C.c_int, [_P, _P, C.c_int64, _P, _P, _P, _P]),
+    "tf_mesh_sample_surface": (C.c_int, [_P, _P, C.c_int64, _P, _P, C.c_int64, _P, _P, _P, _P]),
     "tf_mc_directions": (C.c_int, [C.c_int32, _P, _P, _P, _P, _P, C.c_int64, C.c_int32, _P, _P, C.c_int32, C.c_int32, _P]),
     "tf_cube_light_fwd": (C.c_int, [_P, C.c_int32, _P, _P, C.c_int64, _P, _P]),
     "tf_cube_light_bwd": (C.c_int, [C.c_int32, _P, _P, C.c_int64, _P, _P, _P, _P]),

@@ -12,7 +12,8 @@ struct BuildTri {
     int idx;
 };
 
-void build_bvh(const float* verts, const int32_t* tris, int64_t nt, std::vector<BvhNode>& nodes, std::vector<BvhTri>& out_tris) {
+void build_bvh(const float* verts, const int32_t* tris, int64_t nt, std::vector<BvhNode>& nodes, std::vector<BvhTri>& out_tris,
+               std::vector<int32_t>& perm) {
     std::vector<BuildTri> bt((size_t)nt);
     for (int64_t i = 0; i < nt; ++i) {
         const float* a = verts + 3 * (int64_t)tris[3 * i + 0];
@@ -65,8 +66,10 @@ void build_bvh(const float* verts, const int32_t* tris, int64_t nt, std::vector<
         jobs.push_back({left + 1, mid, j.hi});
     }
     out_tris.resize((size_t)nt);
+    perm.resize((size_t)nt);
     for (int64_t i = 0; i < nt; ++i) {
         const int t = bt[i].idx;
+        perm[i] = t;
         const float* a = verts + 3 * (int64_t)tris[3 * t + 0];
         const float* b = verts + 3 * (int64_t)tris[3 * t + 1];
         const float* c = verts + 3 * (int64_t)tris[3 * t + 2];
@@ -110,20 +113,26 @@ extern "C" TF_API int tf_bvh_create(const float* vertices_host, int64_t n_vertic
         TF_REQUIRE(triangles_host[i] >= 0 && triangles_host[i] < n_vertices, "tf_bvh_create: triangle index out of range");
     std::vector<BvhNode> nodes;
     std::vector<BvhTri> tris;
-    build_bvh(vertices_host, triangles_host, n_triangles, nodes, tris);
+    std::vector<int32_t> perm;
+    build_bvh(vertices_host, triangles_host, n_triangles, nodes, tris, perm);
     tf_bvh* h = new tf_bvh();
     h->n_nodes = (int)nodes.size();
     h->n_tris = (int)tris.size();
     cudaGetDevice(&h->device);
     cudaError_t e1 = cudaMalloc(&h->nodes, nodes.size() * sizeof(BvhNode));
     cudaError_t e2 = cudaMalloc(&h->tris, tris.size() * sizeof(BvhTri));
-    if (e1 != cudaSuccess || e2 != cudaSuccess) {
+    cudaError_t e3 = cudaMalloc(&h->perm, perm.size() * sizeof(int32_t));
+    if (e1 != cudaSuccess || e2 != cudaSuccess || e3 != cudaSuccess) {
         tf_set_error("tf_bvh_create: cudaMalloc failed");
+        if (e1 == cudaSuccess) cudaFree(h->nodes);
+        if (e2 == cudaSuccess) cudaFree(h->tris);
+        if (e3 == cudaSuccess) cudaFree(h->perm);
         delete h;
         return 2;
     }
     cudaMemcpy(h->nodes, nodes.data(), nodes.size() * sizeof(BvhNode), cudaMemcpyHostToDevice);
     cudaMemcpy(h->tris, tris.data(), tris.size() * sizeof(BvhTri), cudaMemcpyHostToDevice);
+    cudaMemcpy(h->perm, perm.data(), perm.size() * sizeof(int32_t), cudaMemcpyHostToDevice);
     *out = reinterpret_cast<tf_bvh_t*>(h);
     return 0;
 }
@@ -133,6 +142,7 @@ extern "C" TF_API void tf_bvh_destroy(tf_bvh_t* handle) {
     if (!h) return;
     cudaFree(h->nodes);
     cudaFree(h->tris);
+    cudaFree(h->perm);
     delete h;
 }
 

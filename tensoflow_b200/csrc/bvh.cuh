@@ -18,6 +18,7 @@ struct __align__(16) BvhTri {
 struct tf_bvh {
     BvhNode* nodes;
     BvhTri* tris;
+    int32_t* perm;   // perm[slot] = the caller's index of the triangle stored at tris[slot] (the build reorders them)
     int n_nodes, n_tris;
     int device;
 };

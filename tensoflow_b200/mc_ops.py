@@ -53,6 +53,26 @@ class RayTracer:
                   "tf_bvh_trace")
         return positions.reshape(*prefix, 3), normals.reshape(*prefix, 3), depth.reshape(*prefix)
 
+    def closest_point(self, points):
+        """Nearest point of the mesh to each of `points` [..., 3] -> (closest [..., 3] fp32, distance [...] fp32, triangle [...]
+        int64 indexing the constructor's `triangles`).  The smaller squared distance wins, an exact tie the smaller triangle
+        index; the result is bit-reproducible.  CUDA tensors only."""
+        if not torch.is_tensor(points) or not points.is_cuda:
+            raise RuntimeError("RayTracer.closest_point needs CUDA tensors (tensoflow_b200 has no CPU path)")
+        if points.shape[-1] != 3:
+            raise RuntimeError(f"RayTracer.closest_point needs points [..., 3], got {list(points.shape)}")
+        p = _f32c(points)
+        prefix = p.shape[:-1]
+        q = p.reshape(-1, 3)
+        n = q.shape[0]
+        closest = torch.empty_like(q)
+        dist = torch.empty(n, device=q.device, dtype=torch.float32)
+        tri = torch.empty(n, device=q.device, dtype=torch.int64)
+        with _timed("bvh_closest_point"):
+            check(_lib.load().tf_bvh_closest_point(self._h, ptr(q), n, ptr(closest), ptr(dist), ptr(tri), stream_ptr()),
+                  "tf_bvh_closest_point")
+        return closest.reshape(*prefix, 3), dist.reshape(prefix), tri.reshape(prefix)
+
 
 def mc_directions(mode: int, normals, view_dirs, src, aux, roughness, n_dirs: int, dirs_out, prob_out, offset: int):
     """Fill dirs_out[:, offset:offset+n_dirs], prob_out[:, offset:offset+n_dirs] (no autograd:
