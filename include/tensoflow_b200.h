@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define TF_ABI_VERSION 2
+#define TF_ABI_VERSION 3
 
 #if defined(__GNUC__)
 #define TF_API __attribute__((visibility("default")))
@@ -171,11 +171,13 @@ TF_API int tf_neus_composite_bwd(const float* sdf, const float* grad, const floa
  * act: 0 none, 1 ReLU, 2 LeakyReLU(0.01), 3 Softplus(beta=100), 4 Sigmoid,
  *      5 exp(min(x, act_param)) (ExpActivation, network/other_field.py:12-18).
  * Row-major contiguous X, W, Y.  b may be NULL.
- * `workspace` (tf_linear_workspace(K, N) bytes, 16-byte aligned, may be NULL) holds the pre-split weights of the
- * tensor-core path: with it, layers of >= 8192 rows and 96 <= K <= 1024, 96 <= N <= 256 run on tcgen05 (3xTF32,
- * fp32-level accuracy; K / N need not be aligned, padded inside); without it, for small batches and for narrow
- * layers the FFMA kernels run. */
-TF_API size_t tf_linear_workspace(int32_t K, int32_t N);
+ * The shape picks the kernel.  Layers of >= 8192 rows with 96 <= K <= 1024, 96 <= N <= 256 run the forward on
+ * tcgen05 (3xTF32, fp32-level accuracy; K / N need not be aligned, padded inside), and layers of >= 8192 rows with
+ * 96 <= K <= 256, 96 <= N <= 1024 run the data gradient dX there; smaller batches and narrower layers run on FFMA.
+ * tf_linear_workspace(M, K, N) is the size in bytes of the 16-byte aligned `workspace` that holds the pre-split
+ * weights of the tcgen05 path at that shape, for either direction, and 0 when neither direction uses it.  When a
+ * call takes the tcgen05 path, a NULL, smaller or unaligned workspace is an error. */
+TF_API size_t tf_linear_workspace(int64_t M, int32_t K, int32_t N);
 TF_API int tf_linear_fwd(const float* X, const float* W, const float* b, int64_t M, int32_t K,
                          int32_t N, int32_t act, float act_param, float* Y, void* workspace,
                          size_t ws_bytes, tf_stream_t stream);

@@ -68,11 +68,7 @@ _SIGNATURES = {
     "tf_iso_count": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, C.c_float, _P, _P, _P]),
     "tf_iso_vertices": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, C.c_float, _P, _P, _P, _P]),
     "tf_iso_triangles": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, C.c_float, _P, _P, _P, _P]),
-}
-
-# later sections of the ABI (small MLP layers, flow sampler, MC shading, BVH)
-_OPTIONAL_SIGNATURES = {
-    "tf_linear_workspace": (C.c_size_t, [C.c_int32, C.c_int32]),
+    "tf_linear_workspace": (C.c_size_t, [C.c_int64, C.c_int32, C.c_int32]),
     "tf_linear_fwd": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_float, _P, _P, C.c_size_t, _P]),
     "tf_linear_bwd": (C.c_int, [_P, _P, _P, _P, _P, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_float,
                                 _P, _P, _P, _P, C.c_size_t, _P]),
@@ -126,7 +122,7 @@ _OPTIONAL_SIGNATURES = {
 
 def exported_symbols():
     """Names every include/*.h entry point must resolve to (used by the CPU tests)."""
-    return sorted(list(_SIGNATURES) + list(_OPTIONAL_SIGNATURES))
+    return sorted(_SIGNATURES)
 
 
 def lib_path() -> Path:
@@ -143,11 +139,11 @@ def load():
             f"{_LIB_PATH} is missing: build it with `python -m tensoflow_b200.build` "
             "(tensoflow_b200 has no CPU / PyTorch fallback)")
     lib = C.CDLL(str(_LIB_PATH))
-    for name, (res, args) in {**_SIGNATURES, **_OPTIONAL_SIGNATURES}.items():
+    for name, (res, args) in _SIGNATURES.items():
         fn = getattr(lib, name)
         fn.restype = res
         fn.argtypes = args
-    if lib.tf_abi_version() != 2:
+    if lib.tf_abi_version() != 3:
         raise RuntimeError("libtensoflow_b200.so ABI version mismatch")
     _lib = lib
     return lib

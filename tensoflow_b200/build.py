@@ -80,7 +80,8 @@ def _build_into(LIB: Path, objdir: Path, NVCC_FLAGS, verbose: bool) -> Path:
         failed |= p.returncode != 0
     if failed:
         raise RuntimeError("nvcc failed")
-    cmd = [nvcc, "-shared", "-o", str(LIB), *objs, "-lcudart"]
+    # --no-undefined: a call into another translation unit without a definition fails here rather than when the library loads
+    cmd = [nvcc, "-shared", "-Xlinker", "--no-undefined", "-o", str(LIB), *objs, "-lcudart"]
     subprocess.run(cmd, check=True)
     return LIB
 

@@ -3,6 +3,7 @@
 // (reference network/flow.py:314-525) for K = 10 bins: st = 11 vertex heights + 10 widths.
 #include "common.cuh"
 #include "flow_spline.cuh"
+#include "internal.cuh"
 
 namespace {
 
@@ -72,15 +73,6 @@ extern "C" TF_API int tf_pwquad_bwd(const float* y, const float* st, int64_t M, 
     return 0;
 }
 
-// tensor-core kernels (flow_tc.cu)
-int tf_internal_flow_block_fwd_tc(const float* y_in, const float* logj_in, const float* feat, int feat_dim, int sn, const float* W1,
-                                  const float* b1, const float* W2, const float* b2, const float* W3, const float* b3, const float* W4,
-                                  const float* b4, float scale, float offset, int cond, int inverse, int64_t M, float* y_out, float* logj_out,
-                                  float* save_h, float* save_st, cudaStream_t stream);
-int tf_internal_flow_block_bwd_tc(const float* y_in, const float* feat, int feat_dim, int sn, const float* W1, const float* W2, const float* W3,
-                                  const float* W4, float scale, float offset, int cond, int64_t M, const float* saved_h, const float* saved_st,
-                                  const float* g_y_out, const float* g_logj, float* g_y_in, float* d_feat, float* dW1, float* db1, float* dW2,
-                                  float* db2, float* dW3, float* db3, float* dW4, float* db4, cudaStream_t stream);
 extern "C" TF_API int tf_flow_block_fwd(const float* y_in, const float* logj_in, const float* feat, int32_t feat_dim, int32_t sn,
                                         const float* W1, const float* b1, const float* W2, const float* b2, const float* W3, const float* b3,
                                         const float* W4, const float* b4, float scale, float offset, int32_t cond, int32_t inverse, int64_t M,

@@ -11,6 +11,7 @@
 #include "common.cuh"
 #include "tc_common.cuh"
 #include "flow_spline.cuh"
+#include "internal.cuh"
 
 namespace {
 

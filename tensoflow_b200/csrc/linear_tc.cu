@@ -14,6 +14,7 @@
 #include "common.cuh"
 #include "tc_common.cuh"
 #include "act.cuh"
+#include "internal.cuh"
 
 namespace {
 
@@ -304,11 +305,9 @@ int pad16(int n) { return (n + 15) / 16 * 16; }
 
 }  // namespace
 
-// shapes the tensor-core dense layer takes: contraction and output widths up to 256
-bool tf_internal_linear_tc_ok(const float* X, const float* Y, int K, int N, int act) {
-    (void)X; (void)Y;
+// shapes the tensor-core dense layer takes: contraction widths up to 1024, output widths up to 256
+bool tf_internal_linear_tc_ok(int K, int N) {
     if (N < 1 || N > 256 || K < 1 || K > 1024) return false;
-    if (act < 0 || act > 5) return false;
     return linear_tc_smem(pad16(N)) <= 227 * 1024;
 }
 size_t tf_internal_linear_tc_ws_floats(int K, int N) { return (size_t)2 * pad16(N) * ((K + KC - 1) / KC * KC); }

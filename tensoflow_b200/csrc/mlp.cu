@@ -7,6 +7,7 @@
 // v1 arithmetic is fp32 FFMA (128x64 CTA tile, 8x4 register tile); see DESIGN.md.
 #include "common.cuh"
 #include "act.cuh"
+#include "internal.cuh"
 
 namespace {
 
@@ -265,7 +266,6 @@ __global__ void __launch_bounds__(256, 2) small_linear_bwd_kernel(const float* _
 
 }  // namespace
 
-// internal entry points shared with the other translation units
 int tf_internal_xty(const float* X, int ldx, const float* Y, int ldy, int64_t rows, int M, int N, float* out, int ldo,
                     cudaStream_t stream) {
     if (rows == 0 || M == 0 || N == 0) return 0;
@@ -277,16 +277,6 @@ int tf_internal_xty(const float* X, int ldx, const float* Y, int ldy, int64_t ro
     if (rpc < 256) rpc = 256;
     grid.z = (unsigned)((rows + rpc - 1) / rpc);
     xty_kernel<<<grid, 256, 0, stream>>>(X, ldx, Y, ldy, rows, M, N, out, ldo, rpc);
-    tf_count_launches(1);
-    return 0;
-}
-
-// out[M][Nout] = A[M][Kred] * W[Kred][Nout] (row-major, no bias / activation)
-int tf_internal_matmul(const float* A, int lda, const float* W, int ldw, int64_t M, int Kred, int Nout, float* out, int ldo,
-                       cudaStream_t stream) {
-    if (M == 0 || Nout == 0) return 0;
-    dim3 grid((unsigned)((M + BM - 1) / BM), (Nout + BN - 1) / BN);
-    linear_kernel<true, false><<<grid, 256, 0, stream>>>(A, lda, nullptr, nullptr, W, ldw, nullptr, M, Kred, Nout, 0, 0.f, out, ldo);
     tf_count_launches(1);
     return 0;
 }
@@ -422,27 +412,24 @@ int head_grid(int64_t M) {
     return (int)(want < cap ? want : cap);
 }
 
-// tensor-core dense layer (linear_tc.cu) and weight-gradient kernel (xty_tc.cu)
-bool tf_internal_linear_tc_ok(const float* X, const float* Y, int K, int N, int act);
-size_t tf_internal_linear_tc_ws_floats(int K, int N);
-int tf_internal_linear_tc(const float* X, const float* W, int ldw, int trans, const float* bias, int64_t M, int K, int N, int act, float act_p,
-                          float* Y, float* wtc, cudaStream_t stream);
-int tf_internal_linear_tc_bwd(const float* dY, const float* Yact, float* dpre, const float* W, int64_t M, int K, int N, int act, float act_p,
-                              float* dX, float* wtc, cudaStream_t stream);
-bool tf_internal_xty_tc_ok(const float* X, const float* Y, int M, int N);
-int tf_internal_xty_tc(const float* X, const float* Y, int64_t rows, int M, int N, float* out, int ldo, int n_valid, cudaStream_t stream);
-
 // Tensor-core dispatch: at least 8192 rows and both widths >= 96.  Narrow layers (the coupling-layer conditioners,
 // 44 -> 64 -> 64 -> 21, and 1..3-wide heads) stay on the FFMA kernels: the tensor core would run mostly padding
 // there, and the spline parameters they produce are the one place where 3xTF32's ~22-bit products (vs 24) showed
 // up in the gradient tolerances.
 static const int64_t TC_MIN_ROWS = 8192;
 static bool tc_shape(int64_t M, int K, int N) { return M >= TC_MIN_ROWS && K >= 96 && N >= 96; }
+// Workspace bytes of the tcgen05 dense layer that contracts K into N outputs over M rows; 0 when that product runs on FFMA.
+// The forward is that product at (K, N), the data gradient at (N, K).
+static size_t tc_ws_bytes(int64_t M, int K, int N) {
+    return tc_shape(M, K, N) && tf_internal_linear_tc_ok(K, N) ? tf_internal_linear_tc_ws_floats(K, N) * sizeof(float) : 0;
+}
+static bool ws_ok(const void* workspace, size_t ws_bytes, size_t need) {
+    return workspace && ((uintptr_t)workspace & 15) == 0 && ws_bytes >= need;
+}
 
-extern "C" TF_API size_t tf_linear_workspace(int32_t K, int32_t N) {
-    if (K < 1 || N < 1) return 0;
-    const size_t a = tf_internal_linear_tc_ws_floats(K, N), b = tf_internal_linear_tc_ws_floats(N, K);
-    return (a > b ? a : b) * sizeof(float);
+extern "C" TF_API size_t tf_linear_workspace(int64_t M, int32_t K, int32_t N) {
+    const size_t fwd = tc_ws_bytes(M, K, N), bwd = tc_ws_bytes(M, N, K);
+    return fwd > bwd ? fwd : bwd;
 }
 
 extern "C" TF_API int tf_linear_fwd(const float* X, const float* W, const float* b, int64_t M, int32_t K, int32_t N, int32_t act,
@@ -457,8 +444,9 @@ extern "C" TF_API int tf_linear_fwd(const float* X, const float* W, const float*
         TF_CHECK_LAUNCH("tf_linear_fwd (head)");
         return 0;
     }
-    if (workspace && tc_shape(M, K, N) && tf_internal_linear_tc_ok(X, Y, K, N, act) && ((uintptr_t)workspace & 15) == 0 &&
-        ws_bytes >= tf_internal_linear_tc_ws_floats(K, N) * sizeof(float)) {
+    if (const size_t need = tc_ws_bytes(M, K, N)) {
+        TF_REQUIRE(ws_ok(workspace, ws_bytes, need), "tf_linear_fwd: the tcgen05 path needs a 16-byte aligned workspace of %zu bytes "
+                                                     "(tf_linear_workspace), got %zu at %p", need, ws_bytes, workspace);
         tf_internal_linear_tc(X, W, K, 0, b, M, K, N, act, act_param, Y, (float*)workspace, (cudaStream_t)stream);
         TF_CHECK_LAUNCH("tf_linear_fwd (tcgen05)");
         return 0;
@@ -498,8 +486,10 @@ extern "C" TF_API int tf_linear_bwd(const float* X, const float* W, const float*
     }
     // dPre = dY * act'(Y) and dX = dPre W.  dX may be NULL (first layer): then a one-column
     // launch still materialises dPre.
-    if (dX && workspace && tc_shape(M, K, N) && tf_internal_linear_tc_ok(dY, dX, N, K, act) && ((uintptr_t)workspace & 15) == 0 &&
-        ws_bytes >= tf_internal_linear_tc_ws_floats(N, K) * sizeof(float)) {
+    const size_t need = dX ? tc_ws_bytes(M, N, K) : 0;
+    if (need) {
+        TF_REQUIRE(ws_ok(workspace, ws_bytes, need), "tf_linear_bwd: the tcgen05 path needs a 16-byte aligned workspace of %zu bytes "
+                                                     "(tf_linear_workspace), got %zu at %p", need, ws_bytes, workspace);
         tf_internal_linear_tc_bwd(dY, Y, dpre, W, M, K, N, act, act_param, dX, (float*)workspace, stream);
     } else if (dX) {
         dim3 grid((unsigned)((M + BM - 1) / BM), (K + BN - 1) / BN);
@@ -512,7 +502,7 @@ extern "C" TF_API int tf_linear_bwd(const float* X, const float* W, const float*
     }
     if (dW) {
         // dW[n][k] += sum_m dPre[m][n] X[m][k]
-        if (tc_shape(M, K, N) && K % 16 == 0 && tf_internal_xty_tc_ok(dpre, X, N, K)) tf_internal_xty_tc(dpre, X, M, N, K, dW, K, K, stream);
+        if (tc_shape(M, K, N)) tf_internal_xty_auto(dpre, X, M, N, K, dW, stream);
         else tf_internal_xty(dpre, N, X, K, M, N, K, dW, K, stream);
     }
     if (db) tf_internal_colsum(dpre, N, M, N, db, stream);

@@ -12,6 +12,7 @@
 //              the 7 stencil rows of sample s x 2 hidden units -> the stencil is thread local
 //   GEMM2    : centre rows only ([16][NC] x [NC][A]); taps need output 0 only (a dot product)
 #include "common.cuh"
+#include "internal.cuh"
 
 namespace {
 
@@ -476,31 +477,6 @@ void fill_common(StencilParams& p, const tf_vm_field_t* f, const tf_sdf_mlp_t* m
 
 }  // namespace
 
-int tf_check_field(const tf_vm_field_t* f, bool need_mips);
-
-// tensor-core dense layer (linear_tc.cu)
-bool tf_internal_linear_tc_ok(const float* X, const float* Y, int K, int N, int act);
-size_t tf_internal_linear_tc_ws_floats(int K, int N);
-int tf_internal_linear_tc(const float* X, const float* W, int ldw, int trans, const float* bias, int64_t M, int K, int N, int act, float act_p,
-                          float* Y, float* wtc, cudaStream_t stream);
-// tensor-core forward (sdf_stencil_tc.cu)
-bool tf_internal_stencil_fwd_tc_ok(int KT, int H);
-size_t tf_internal_tc_w0_floats(int KT, int H);
-int tf_internal_stencil_fwd_tc(const tf_vm_field_t* f, const tf_sdf_mlp_t* m, const float* xyz, const float* level, int64_t n,
-                               const float units[3], int nq, float* sdf7, float* grad, float* hess, float* sdf1, float* spc,
-                               float* w0tc, cudaStream_t stream);
-// tensor-core backward (sdf_stencil_bwd_tc.cu)
-size_t tf_internal_bwd_tc_smem(int KT, int H);
-size_t tf_internal_bwd_tc_wtc_floats(int KT, int H);
-int tf_internal_bwd_tc_prep(const float* W0, int K, int KT, int H, float* wtc, cudaStream_t stream);
-int tf_internal_bwd_tc_samples_per_tile();
-int tf_internal_bwd_tc_fold(const float* tmp, int H, int K, int KT, float* dW0, float* db0, cudaStream_t stream);
-int tf_internal_stencil_bwd_tc(const tf_vm_field_t* f, const tf_vm_mut_t* g, const tf_sdf_mlp_t* m, const float* wtc, const float* xyz,
-                               const float* level, int64_t n, const float units[3], const float* sdf7, const float* g_sdf,
-                               const float* g_grad, const float* g_hess, const float* dHc, float* dpre, float* arow,
-                               float* da_scratch, float* dW1r0, float* db1, cudaStream_t stream);
-size_t tf_internal_bwd_tc_scratch_floats(int KT);
-
 // Which decoder shapes run on the tcgen05 kernels; the FFMA kernels above take the others (hidden > 256).  check_mlp and
 // tf_check_field already bound the rest: hidden % 32 == 0, n_comp % 4 == 0 and n_comp <= 36, so KT <= 112.
 static bool fwd_on_tc(const Dims& d) { return tf_internal_stencil_fwd_tc_ok(d.KT, d.H); }
@@ -539,9 +515,8 @@ static int stencil_fwd_impl(int mode, const tf_vm_field_t* f, const tf_sdf_mlp_t
         if (feat) {
             // appearance head: feat = hidden(centre) W1[1:,:]^T + b1[1:]
             float* wlin = spc + (size_t)n * d.H;
-            if (tf_internal_linear_tc_ok(spc, feat, d.H, d.A, 0))
-                tf_internal_linear_tc(spc, m->W1 + d.H, d.H, 0, m->b1 + 1, n, d.H, d.A, 0, 0.f, feat, wlin, stream);
-            else if (int e = tf_linear_fwd(spc, m->W1 + d.H, m->b1 + 1, n, d.H, d.A, 0, 0.f, feat, nullptr, 0, stream_)) return e;
+            // tf_internal_linear_tc_ok holds: K = H <= 256 (fwd_on_tc), N = A <= 128 (check_mlp)
+            tf_internal_linear_tc(spc, m->W1 + d.H, d.H, 0, m->b1 + 1, n, d.H, d.A, 0, 0.f, feat, wlin, stream);
         }
         TF_CHECK_LAUNCH("tf_sdf_stencil_fwd (tcgen05)");
         return 0;
@@ -599,15 +574,6 @@ static size_t bwd_slice_floats(const Dims& d, int64_t n_slice) {
     return (size_t)tiles * ((size_t)R * d.H + (size_t)R * d.KP + (size_t)TS * d.H);
 }
 
-int tf_internal_xty(const float* X, int ldx, const float* Y, int ldy, int64_t rows, int M, int N, float* out, int ldo, cudaStream_t stream);
-int tf_internal_colsum(const float* X, int ldx, int64_t rows, int cols, float* out, cudaStream_t stream);
-int tf_internal_matmul(const float* A, int lda, const float* W, int ldw, int64_t M, int Kred, int Nout, float* out, int ldo,
-                       cudaStream_t stream);
-bool tf_internal_xty_tc_ok(const float* X, const float* Y, int M, int N);
-int tf_internal_xty_tc(const float* X, const float* Y, int64_t rows, int M, int N, float* out, int ldo, int n_valid, cudaStream_t stream);
-int tf_internal_xty_tc_tiled(const float* X, const float* Y, int64_t rows, int M, int N, float* out, int ldo, int n_valid, int x_tiled,
-                             cudaStream_t stream);
-
 // tensor-core backward workspace: [W slices | dW0/db0 staging | per tile of 18 samples: dPre [128,H], A rows [128,KT],
 // dHidden(centre) [18,H]]
 static size_t bwd_tc_fixed_floats(const Dims& d) {
@@ -654,11 +620,8 @@ static int stencil_bwd_tc(const tf_vm_field_t* f, const tf_sdf_mlp_t* m, const D
         const int64_t s0 = t0 * spt;
         const int64_t ns = s0 + nt * spt < n ? nt * spt : n - s0;
         const float* gf = g_feat ? g_feat + s0 * d.A : nullptr;
-        // dHidden(centre) = g_feat W1[1:, :]
-        if (gf) {
-            if (tf_internal_linear_tc_ok(gf, dHc, d.A, H, 0)) tf_internal_linear_tc(gf, m->W1 + H, H, 1, nullptr, ns, d.A, H, 0, 0.f, dHc, wlin, stream);
-            else tf_internal_matmul(gf, d.A, m->W1 + H, H, ns, d.A, H, dHc, H, stream);
-        }
+        // dHidden(centre) = g_feat W1[1:, :]; tf_internal_linear_tc_ok holds: K = A <= 128 (check_mlp), N = H <= 256 (bwd_on_tc)
+        if (gf) tf_internal_linear_tc(gf, m->W1 + H, H, 1, nullptr, ns, d.A, H, 0, 0.f, dHc, wlin, stream);
         if (int e = tf_internal_stencil_bwd_tc(f, g_field, m, wtc, xyz + s0 * 3, level ? level + s0 : nullptr, ns, units, sdf7 + s0 * NQ,
                                                g_sdf ? g_sdf + s0 : nullptr, g_grad ? g_grad + s0 * 3 : nullptr,
                                                g_hess ? g_hess + s0 : nullptr, gf ? dHc : nullptr, dpre, arow,
@@ -669,10 +632,8 @@ static int stencil_bwd_tc(const tf_vm_field_t* f, const tf_sdf_mlp_t* m, const D
         TF_REQUIRE(tf_internal_xty_tc_ok(dpre, arow, H, KT), "tensor-core X^T Y does not take this decoder shape (H=%d, KT=%d)", H, KT);
         if (int e = tf_internal_xty_tc_tiled(dpre, arow, nt * 128, H, KT, tmp, KT, d.K + 1, 1, stream)) return e;
         if (gf) {
-            // centre hidden activations kept from the forward call
-            const float* hid = hidden_c + s0 * H;
-            if (tf_internal_xty_tc_ok(gf, hid, d.A, H)) tf_internal_xty_tc(gf, hid, ns, d.A, H, g_mlp->W1 + H, H, H, stream);
-            else tf_internal_xty(gf, d.A, hid, H, ns, d.A, H, g_mlp->W1 + H, H, stream);
+            // dW1[1:, :] += g_feat^T hidden(centre), from the centre hidden activations kept by the forward call
+            tf_internal_xty_auto(gf, hidden_c + s0 * H, ns, d.A, H, g_mlp->W1 + H, stream);
             tf_internal_colsum(gf, d.A, ns, d.A, g_mlp->b1 + 1, stream);
         }
     }

@@ -19,6 +19,7 @@
 #include "common.cuh"
 #include "tc_common.cuh"
 #include "stencil_site.cuh"
+#include "internal.cuh"
 
 namespace {
 

@@ -25,6 +25,7 @@
 #include "common.cuh"
 #include "tc_common.cuh"
 #include "stencil_site.cuh"
+#include "internal.cuh"
 
 namespace {
 

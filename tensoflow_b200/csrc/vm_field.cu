@@ -3,6 +3,7 @@
 // (network/fields.py:272-293, :786-806; network/flow.py:719-740).
 #include <stdarg.h>
 #include "common.cuh"
+#include "internal.cuh"
 
 // ---- error plumbing (thread-local; see include/tensoflow_b200.h) -------------
 static thread_local char g_err[512] = "";

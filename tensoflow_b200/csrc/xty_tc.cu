@@ -12,6 +12,7 @@
 #include <stdlib.h>
 #include "common.cuh"
 #include "tc_common.cuh"
+#include "internal.cuh"
 
 namespace {
 
@@ -236,11 +237,6 @@ bool tf_internal_xty_tc_ok(const float* X, const float* Y, int M, int N) {
 // X [rows][M] (ld = M), Y [rows][N] (ld = N); out[m][n] (ld = ldo) += X^T Y for n < n_valid
 // x_tiled: X is stored per 128-row tile as [tile][M][128] (rows must then be a multiple of 128)
 int tf_internal_xty_tc_tiled(const float* X, const float* Y, int64_t rows, int M, int N, float* out, int ldo, int n_valid, int x_tiled,
-                             cudaStream_t stream);
-int tf_internal_xty_tc(const float* X, const float* Y, int64_t rows, int M, int N, float* out, int ldo, int n_valid, cudaStream_t stream) {
-    return tf_internal_xty_tc_tiled(X, Y, rows, M, N, out, ldo, n_valid, 0, stream);
-}
-int tf_internal_xty_tc_tiled(const float* X, const float* Y, int64_t rows, int M, int N, float* out, int ldo, int n_valid, int x_tiled,
                              cudaStream_t stream) {
     if (rows == 0) return 0;
     // MMA N side = the wider operand; the M side is padded to whole 128-row MMAs (its extra rows are never read back)
@@ -274,15 +270,16 @@ int tf_internal_xty_tc_tiled(const float* X, const float* Y, int64_t rows, int M
     return 0;
 }
 
-int tf_internal_xty(const float* X, int ldx, const float* Y, int ldy, int64_t rows, int M, int N, float* out, int ldo, cudaStream_t stream);
+int tf_internal_xty_auto(const float* X, const float* Y, int64_t rows, int M, int N, float* out, cudaStream_t stream) {
+    return tf_internal_xty_tc_ok(X, Y, M, N) ? tf_internal_xty_tc_tiled(X, Y, rows, M, N, out, N, N, 0, stream)
+                                             : tf_internal_xty(X, M, Y, N, rows, M, N, out, N, stream);
+}
 
 extern "C" TF_API int tf_xty_accumulate(const float* X, const float* Y, int64_t rows, int32_t M, int32_t N, float* out,
-                                        tf_stream_t stream_) {
+                                        tf_stream_t stream) {
     if (rows == 0) return 0;
     TF_REQUIRE(X && Y && out && M > 0 && N > 0, "tf_xty_accumulate: NULL pointer or bad shape (%d,%d)", M, N);
-    cudaStream_t stream = (cudaStream_t)stream_;
-    if (int e = tf_internal_xty_tc_ok(X, Y, M, N) ? tf_internal_xty_tc(X, Y, rows, M, N, out, N, N, stream)
-                                                  : tf_internal_xty(X, M, Y, N, rows, M, N, out, N, stream)) return e;
+    if (int e = tf_internal_xty_auto(X, Y, rows, M, N, out, (cudaStream_t)stream)) return e;
     TF_CHECK_LAUNCH("tf_xty_accumulate");
     return 0;
 }

@@ -443,7 +443,6 @@ class NeusCompositeFunction(torch.autograd.Function):
         return d_sdf, d_grad, None, None, None, dv, None, d_vals, None
 
 
-LINEAR_TC_MIN_ROWS = 8192    # below this the library uses its FFMA kernel and needs no workspace
 ACT = {"none": 0, "relu": 1, "leaky": 2, "softplus100": 3, "sigmoid": 4, "exp": 5}
 
 
@@ -459,7 +458,7 @@ class LinearFunction(torch.autograd.Function):
         M, K = Xc.shape
         N = Wc.shape[0]
         Y = torch.empty(M, N, device=Xc.device, dtype=torch.float32)
-        wsb = int(lib.tf_linear_workspace(K, N)) if M >= LINEAR_TC_MIN_ROWS else 0
+        wsb = int(lib.tf_linear_workspace(M, K, N))
         ws = torch.empty(wsb // 4, device=Xc.device, dtype=torch.float32) if wsb else None
         with _timed(f"linear_fwd[{K}->{N}]"):
             check(lib.tf_linear_fwd(ptr(Xc), ptr(Wc), ptr(bc), M, K, N, ACT[act], float(act_param), ptr(Y), ptr(ws), wsb,
@@ -480,7 +479,7 @@ class LinearFunction(torch.autograd.Function):
         dX = torch.empty(M, K, device=Xc.device, dtype=torch.float32) if need_x else None
         dW = torch.zeros_like(Wc) if need_w else None
         db = torch.zeros(N, device=Xc.device, dtype=torch.float32) if need_b else None
-        wsb = int(lib.tf_linear_workspace(K, N)) if M >= LINEAR_TC_MIN_ROWS else 0
+        wsb = int(lib.tf_linear_workspace(M, K, N))
         ws = torch.empty(wsb // 4, device=Xc.device, dtype=torch.float32) if wsb else None
         with _timed(f"linear_bwd[{K}->{N}]"):
             check(lib.tf_linear_bwd(ptr(Xc), ptr(Wc), ptr(Y), ptr(gYc), ptr(dpre), M, K, N, ACT[ctx.act], ctx.act_param,
@@ -492,11 +491,11 @@ def linear(X, W, b=None, act="none", act_param=0.0):
     if X.shape[0] == 0:
         return X.new_zeros(0, W.shape[0])
     K = X.shape[1]
-    if X.shape[0] >= LINEAR_TC_MIN_ROWS and W.shape[0] >= 96 and K >= 80 and K % 16 != 0:
-        # wide layer with a ragged input width (the shader heads read 90 / 123 / 161 concatenated features): zero columns up to
-        # the next multiple of 16 put the layer, its data gradient and its weight gradient on the tensor-core kernels (16-byte
-        # aligned rows, K >= 96); the result is unchanged and autograd slices the padding off both gradients
-        pad = 16 - K % 16
+    pad = -K % 16
+    if pad and _lib.load().tf_linear_workspace(X.shape[0], K + pad, W.shape[0]) > 0:
+        # ragged input width (the shader heads read 90 / 123 / 161 concatenated features) of a layer that the tensor-core
+        # kernels take once it is padded: zero columns up to the next multiple of 16 put the layer, its data gradient and its
+        # weight gradient there (16-byte aligned rows); the result is unchanged and autograd slices the padding off both gradients
         X = torch.nn.functional.pad(X, (0, pad))
         W = torch.nn.functional.pad(W, (0, pad))
     return LinearFunction.apply(X, W, b, act, act_param)

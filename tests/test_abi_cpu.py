@@ -27,10 +27,49 @@ def test_header_symbols_exported(lib):
     assert declared == set(_lib.exported_symbols()), declared ^ set(_lib.exported_symbols())
 
 
-def test_abi_version_2_and_error_string(lib):
-    """ABI 2: tf_sdf_stencil_bwd takes hidden_centre, tf_xty_accumulate has no force_simt, two entries are gone."""
-    assert lib.tf_abi_version() == 2
+def test_abi_version_3_and_error_string(lib):
+    """ABI 3: tf_linear_workspace takes the row count, and the tcgen05 dense layer refuses to run without its workspace."""
+    assert lib.tf_abi_version() == 3
     assert isinstance(lib.tf_last_error(), bytes)
+
+
+def _linear_tc_bytes(K, N):
+    """Pre-split weights of the tcgen05 dense layer contracting K into N outputs: hi | lo, N padded to 16, K to 32."""
+    return 4 * 2 * (-(-N // 16) * 16) * (-(-K // 32) * 32)
+
+
+@pytest.mark.parametrize("M,K,N,fwd,bwd", [
+    (8191, 128, 128, False, False), (8192, 128, 128, True, True),       # rows
+    (8192, 95, 128, False, False), (8192, 96, 128, True, True),         # K >= 96
+    (8192, 1024, 128, True, False), (8192, 1025, 128, False, False),    # forward K <= 1024 (backward K <= 256)
+    (8192, 128, 95, False, False), (8192, 128, 96, True, True),         # N >= 96
+    (8192, 512, 256, True, False), (8192, 512, 257, False, False),      # forward N <= 256 (backward K <= 256)
+    (8192, 128, 512, False, True),                                      # only the data gradient (N into K) runs on tcgen05
+    (1 << 20, 64, 64, False, False),                                    # narrow layer: FFMA at any row count
+])
+def test_linear_workspace_follows_the_dispatch(lib, M, K, N, fwd, bwd):
+    """tf_linear_workspace(M, K, N) is what the tcgen05 forward (K into N) or data gradient (N into K) needs, 0 when neither runs."""
+    want = max(_linear_tc_bytes(K, N) if fwd else 0, _linear_tc_bytes(N, K) if bwd else 0)
+    assert lib.tf_linear_workspace(M, K, N) == want
+
+
+@pytest.mark.parametrize("bad", ["null", "small", "unaligned"])
+def test_linear_tc_requires_workspace(lib, bad):
+    """On a tcgen05 shape tf_linear_fwd / tf_linear_bwd return an error before any launch when the workspace is NULL, too
+    small or not 16-byte aligned, instead of falling back to the FFMA kernels.  The addresses are fake: the check fires before
+    anything is dereferenced."""
+    M, K, N = 8192, 128, 128
+    fake = lambda i: ctypes.c_void_p((1 << 20) * (i + 1))
+    need = lib.tf_linear_workspace(M, K, N)
+    ws, wsb = {"null": (None, need), "small": (fake(9), need - 4), "unaligned": (ctypes.c_void_p((1 << 20) * 10 + 4), need)}[bad]
+    launches = lib.tf_launch_count()
+    rc = lib.tf_linear_fwd(fake(0), fake(1), None, M, K, N, 0, 0.0, fake(2), ws, wsb, None)
+    assert rc != 0
+    assert b"workspace" in lib.tf_last_error()
+    rc = lib.tf_linear_bwd(fake(0), fake(1), fake(2), fake(3), fake(4), M, K, N, 0, 0.0, fake(5), fake(6), fake(7), ws, wsb, None)
+    assert rc != 0
+    assert b"workspace" in lib.tf_last_error()
+    assert lib.tf_launch_count() == launches
 
 
 def test_flow_block_bwd_requires_kept_activations(lib):
