@@ -479,6 +479,44 @@ TF_API int tf_iso_vertices(const float* u, int32_t nx, int32_t ny, int32_t nz, f
 TF_API int tf_iso_triangles(const float* u, int32_t nx, int32_t ny, int32_t nz, float threshold, const int64_t* tri_offsets,
                             const int32_t* index_volume, int32_t* triangles, tf_stream_t stream);
 
+/* ---- narrow-band isosurface extraction -------------------------------------------------------------
+ * The mesh of tf_iso_* (same vertex order, interpolation, triangle order and winding) on a lattice of nx, ny, nz points
+ * (2..4096 each; point, edge and cell indices are int64) whose values are known only in bricks around the surface.
+ * Bricks are 8^3 cells, brick (I, J, K) has id (I*by + J)*bz + K (bx = ceil((nx-1)/8), ...), covers the points 8I ..
+ * min(8I + 8, nx-1) per axis, and owns its cells and the points 8I .. 8I + 7 (the last brick on an axis also its end point).
+ * Band rule (tensoflow_b200.isosurface.marching_cubes_narrowband drives it):
+ *   1. coarse values u on the points min(8I, n-1) per axis, [bx+1][by+1][bz+1];
+ *   2. tf_iso_nb_classify: flags[brick] = 1 iff its 8 coarse corners straddle the threshold or one has
+ *      |u - threshold| < band (band = sqrt(3)*8*h_max rounded to fp32, h_max the largest axis spacing), else 0;
+ *   3. the values of the active bricks, values[slot][9][9][9] (z fastest; positions past the lattice's end are never read),
+ *      at the xyz tf_iso_nb_points writes ([n][729][3], from the axis tables; positions past the end repeat the last point);
+ *   4. tf_iso_nb_grow: for each crossed lattice edge in the closure of a listed brick, sets flags = 2 on every brick with
+ *      flag 0 whose closure holds the edge (face and edge neighbours).  The caller activates them and repeats from 3
+ *      until a round adds none.
+ * For a 1-Lipschitz field no brick holding a crossing is missed.  Otherwise every surface component that one active brick
+ * touches is still extracted whole; a component that no coarse corner sees (a steep, tiny closed surface between coarse
+ * points) is absent.  With the final active bricks in any slot order:
+ *   tf_iso_nb_count      per segment (slot*81 + 9*x + y: the row of local points (x, y, *)) the owned crossed edges, the
+ *                        triangles of its cells and the key (i*ny + j)*bz + K (INT64_MAX for a row the brick does not own);
+ *   the caller sorts the keys and takes exclusive int64 prefix sums of both counts in key order (totals < 2^31);
+ *   tf_iso_nb_vertices   vertices [V,3] and index[slot][729] (int32 id of the first vertex of each owned point);
+ *   tf_iso_nb_triangles  triangles [T,3] through slot_map[brick id] (int32 slot of every active brick).
+ * No atomics: the output is bit-reproducible.  It equals tf_iso_* on the dense lattice when every cell with a crossing lies
+ * in an active brick. */
+TF_API int tf_iso_nb_classify(const float* coarse, int32_t nx, int32_t ny, int32_t nz, float threshold, float band, uint8_t* flags,
+                              tf_stream_t stream);
+TF_API int tf_iso_nb_points(const float* ax, const float* ay, const float* az, int32_t nx, int32_t ny, int32_t nz,
+                            const int64_t* bricks, int64_t n_bricks, float* xyz, tf_stream_t stream);
+TF_API int tf_iso_nb_grow(const float* values, const int64_t* bricks, int64_t n_bricks, int32_t nx, int32_t ny, int32_t nz,
+                          float threshold, uint8_t* flags, tf_stream_t stream);
+TF_API int tf_iso_nb_count(const float* values, const int64_t* bricks, int64_t n_bricks, int32_t nx, int32_t ny, int32_t nz,
+                           float threshold, int32_t* vert_count, int32_t* tri_count, int64_t* keys, tf_stream_t stream);
+TF_API int tf_iso_nb_vertices(const float* values, const int64_t* bricks, int64_t n_bricks, int32_t nx, int32_t ny, int32_t nz,
+                              float threshold, const int64_t* vert_offsets, float* vertices, int32_t* index, tf_stream_t stream);
+TF_API int tf_iso_nb_triangles(const float* values, const int64_t* bricks, int64_t n_bricks, int32_t nx, int32_t ny, int32_t nz,
+                               float threshold, const int32_t* slot_map, const int64_t* tri_offsets, const int32_t* index,
+                               int32_t* triangles, tf_stream_t stream);
+
 /* ---- optimizer step ------------------------------------------------------------------------------
  * torch.optim.Adam(grad_vars, betas=(0.9, 0.99)).step() of the reference trainer (train/trainer_inv.py:112,212; one
  * learning rate per parameter group, :247-248) as ONE streaming pass: for tensor t (numel[t] fp32 elements in any

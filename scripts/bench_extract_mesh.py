@@ -1,5 +1,8 @@
 """Mesh extraction of the shape stage (ShapeRenderer.extract_geometry = extract_mesh.py's extract_fields + marching cubes) on a
-config-2-shaped field (G 512, C 36, H 256, A 128, 3 mip levels, seeded perturbation) at lattice resolutions 256, 512, 1024.
+config-2-shaped field (G 512, C 36, H 256, A 128, 3 mip levels, seeded perturbation): the dense path at lattice resolutions
+512 and 1024 (--res) and the narrow band (isosurface.marching_cubes_narrowband, --nb-res) at 512, 1024, 2048 and 4096.  Where
+both run at one resolution their repetitions alternate, so the two paths see the same machine state; 512 and 1024 are the two
+sizes on the dense side of extract_geometry's switch at 2^31 lattice points.
 
 Times, with CUDA events after a warm-up of every shape: the field evaluation (extract_fields) and each isosurface kernel
 (tf_iso_count, tf_iso_vertices, tf_iso_triangles; the host prefix sum + size read between count and vertices is reported as
@@ -7,7 +10,11 @@ Times, with CUDA events after a warm-up of every shape: the field evaluation (ex
 of the 7.7 TB/s HBM bound, V and T, the GPU name and power limit, and the CPU oracle (oracle/torch_oracle_iso.py) at 128^3 and
 256^3 as the host figure.  The 256^3 volume (64 MB) fits in the 126 MB L2; the 512^3 and 1024^3 volumes do not.
 
-    python scripts/bench_extract_mesh.py [--res 256 512 1024] [--reps 3] [--out results.json]
+Narrow band, per phase with CUDA events (best of --reps): coarse (coarse lattice queries + brick test), fine (brick-point
+queries, all rounds), grow (grow kernel + one host read per round), kernels (count, vertices, triangles), ordering (segment
+key sort, prefix sums, size read, slot map); SDF queries against R^3, grow rounds, active bricks, peak memory, V and T.
+
+    python scripts/bench_extract_mesh.py [--res 512 1024] [--nb-res 512 1024 2048 4096] [--reps 3] [--out results.json]
 """
 import argparse
 import json
@@ -78,6 +85,10 @@ def timed_iso(u, thr=0.0):
     return ms, n_verts, n_tris
 
 
+def best_scan(phases):
+    return min(p["scan_ms"] for p in phases)
+
+
 def kernel_bytes(R, V, T):
     """Compulsory HBM traffic per kernel: the volume is read once per kernel (4 B/point), row counts / offsets move 8 B per row,
     the index volume is written in full (4 B/point) and read back only around surface cells (not counted), vertices are 12 B,
@@ -86,9 +97,33 @@ def kernel_bytes(R, V, T):
     return {"count": 4 * N + 8 * rows, "vertices": 4 * N + 4 * N + 8 * rows + 12 * V, "triangles": 4 * N + 8 * rows + 12 * T}
 
 
+def timed_narrowband(shape, lo, hi, R):
+    """ShapeRenderer.extract_geometry's narrow band at resolution R -> row of phase times (ms), counts, peak memory"""
+    from tensoflow_b200.isosurface import marching_cubes_narrowband
+    torch.cuda.synchronize()
+    torch.cuda.reset_peak_memory_stats()
+    base = torch.cuda.memory_allocated()
+    stats = {}
+    a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    a.record()
+    with torch.no_grad():
+        v, t = marching_cubes_narrowband(shape._extract_values, shape._extract_axes(lo, hi, R), 0.0, stats=stats)
+    b.record()
+    torch.cuda.synchronize()
+    ms = {}
+    for name, e0, e1 in stats["events"]:
+        ms[f"{name}_ms"] = ms.get(f"{name}_ms", 0.0) + e0.elapsed_time(e1)
+    row = {"total_ms": a.elapsed_time(b), **ms, "grow_rounds": stats["grow_rounds"], "bricks": stats["bricks"],
+           "queries": stats["queries"], "queries_over_R3": stats["queries"] / R ** 3,
+           "peak_bytes": torch.cuda.max_memory_allocated() - base, "V": v.shape[0], "T": t.shape[0]}
+    del v, t
+    return row
+
+
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--res", type=int, nargs="+", default=[256, 512, 1024])
+    ap.add_argument("--res", type=int, nargs="+", default=[512, 1024])
+    ap.add_argument("--nb-res", type=int, nargs="+", default=[512, 1024, 2048, 4096])
     ap.add_argument("--reps", type=int, default=3)
     ap.add_argument("--host-res", type=int, nargs="+", default=[128, 256])
     ap.add_argument("--out", default=None)
@@ -100,14 +135,32 @@ def main():
     dev = torch.device("cuda:0")
     shape = make_shape(dev)
     lo, hi = [-1.0] * 3, [1.0] * 3
-    result = {"info": gpu_info(), "field": "G 512, C 36, H 256, A 128, 3 levels, perturbed (seed 1, 1e-2)", "gpu": [], "host": []}
-    for R in args.res:
+    result = {"info": gpu_info(), "field": "G 512, C 36, H 256, A 128, 3 levels, perturbed (seed 1, 1e-2)", "gpu": [], "host": [],
+              "narrowband": []}
+    for R in sorted(set(args.res) | set(args.nb_res)):
+        if R in args.nb_res:
+            timed_narrowband(shape, lo, hi, R)                          # warm-up
+            nb_rows = []
+        if R not in args.res:
+            for _ in range(args.reps):
+                nb_rows.append(timed_narrowband(shape, lo, hi, R))
+            best = {k: min(r[k] for r in nb_rows) for k in nb_rows[0] if k.endswith("_ms")}
+            row = {"res": R, **nb_rows[0], **best}
+            result["narrowband"].append(row)
+            print(json.dumps({"narrowband": row}), flush=True)
+            torch.cuda.empty_cache()
+            continue
         shape.extract_geometry(lo, hi, R)                              # warm-up of every shape of this resolution
         u = shape.extract_fields(lo, hi, R)
         timed_iso(u)
         torch.cuda.synchronize()
         field_ms, phases = [], []
         for _ in range(args.reps):
+            if R in args.nb_res:                                       # alternate with the dense repetitions
+                del u
+                torch.cuda.empty_cache()
+                nb_rows.append(timed_narrowband(shape, lo, hi, R))
+                u = torch.empty(0)
             del u
             a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             a.record()
@@ -127,6 +180,11 @@ def main():
                "hbm_share": {k: nbytes[k] / HBM_BYTES_PER_S / (best[f"{k}_ms"] * 1e-3) for k in nbytes}}
         result["gpu"].append(row)
         print(json.dumps(row), flush=True)
+        if R in args.nb_res:
+            best = {k: min(r[k] for r in nb_rows) for k in nb_rows[0] if k.endswith("_ms")}
+            nrow = {"res": R, **nb_rows[0], **best, "dense_total_ms": min(field_ms) + iso_ms + best_scan(phases)}
+            result["narrowband"].append(nrow)
+            print(json.dumps({"narrowband": nrow}), flush=True)
         if R in args.host_res:
             uc = u.cpu()
             t0 = time.perf_counter()

@@ -68,6 +68,12 @@ _SIGNATURES = {
     "tf_iso_count": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, C.c_float, _P, _P, _P]),
     "tf_iso_vertices": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, C.c_float, _P, _P, _P, _P]),
     "tf_iso_triangles": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, C.c_float, _P, _P, _P, _P]),
+    "tf_iso_nb_classify": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, C.c_float, C.c_float, _P, _P]),
+    "tf_iso_nb_points": (C.c_int, [_P, _P, _P, C.c_int32, C.c_int32, C.c_int32, _P, C.c_int64, _P, _P]),
+    "tf_iso_nb_grow": (C.c_int, [_P, _P, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_float, _P, _P]),
+    "tf_iso_nb_count": (C.c_int, [_P, _P, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_float, _P, _P, _P, _P]),
+    "tf_iso_nb_vertices": (C.c_int, [_P, _P, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_float, _P, _P, _P, _P]),
+    "tf_iso_nb_triangles": (C.c_int, [_P, _P, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_float, _P, _P, _P, _P, _P]),
     "tf_linear_workspace": (C.c_size_t, [C.c_int64, C.c_int32, C.c_int32]),
     "tf_linear_fwd": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_float, _P, _P, C.c_size_t, _P]),
     "tf_linear_bwd": (C.c_int, [_P, _P, _P, _P, _P, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_float,
