@@ -9,7 +9,7 @@
 //             d d       through the bilinear fractions (d S / d fu = sum_k dw_k/dfu (T_k - S) / W), u = (x/m + 1) R/2 - 1/2
 //             d level   = g . (S_l1 - S_l0) inside the clamp range
 // In round 1 this was ~150 tensor ops per lookup and level (about 3000 launches per ShapeRenderer step).
-#include "common.cuh"
+#include "shading.cuh"
 
 namespace {
 
@@ -21,92 +21,6 @@ struct CubeStack {
     int res[CS_MAX_LEVELS];
     int n;
 };
-
-// face convention of network/light_utils.py:24-31 / renderutils/c_src/cubemap.cu:32-60
-__device__ __forceinline__ void cs_cube_to_dir(int s, float x, float y, float c[3]) {
-    switch (s) {
-        case 0: c[0] = 1.f; c[1] = -y; c[2] = -x; break;
-        case 1: c[0] = -1.f; c[1] = -y; c[2] = x; break;
-        case 2: c[0] = x; c[1] = 1.f; c[2] = y; break;
-        case 3: c[0] = x; c[1] = -1.f; c[2] = -y; break;
-        case 4: c[0] = x; c[1] = -y; c[2] = 1.f; break;
-        default: c[0] = -x; c[1] = -y; c[2] = -1.f; break;
-    }
-}
-
-// x = sx d[ax] / m, y = sy d[ay] / m, m = sm d[am] > 0
-struct FaceMap { int face, ax, ay, am; float sx, sy, sm, m, x, y; };
-
-__device__ __forceinline__ FaceMap cs_face(const float d[3]) {
-    FaceMap f;
-    const float a0 = fabsf(d[0]), a1 = fabsf(d[1]), a2 = fabsf(d[2]);
-    if (a0 >= a1 && a0 >= a2) {
-        f.am = 0; f.ax = 2; f.ay = 1; f.sy = -1.f;
-        if (d[0] >= 0.f) { f.face = 0; f.sx = -1.f; f.sm = 1.f; } else { f.face = 1; f.sx = 1.f; f.sm = -1.f; }
-    } else if (a1 >= a2) {
-        f.am = 1; f.ax = 0; f.ay = 2; f.sx = 1.f;
-        if (d[1] >= 0.f) { f.face = 2; f.sy = 1.f; f.sm = 1.f; } else { f.face = 3; f.sy = -1.f; f.sm = -1.f; }
-    } else {
-        f.am = 2; f.ax = 0; f.ay = 1; f.sy = -1.f;
-        if (d[2] >= 0.f) { f.face = 4; f.sx = 1.f; f.sm = 1.f; } else { f.face = 5; f.sx = -1.f; f.sm = -1.f; }
-    }
-    f.m = fmaxf(fabsf(d[f.am]), 1e-30f);
-    f.x = f.sx * d[f.ax] / f.m;
-    f.y = f.sy * d[f.ay] / f.m;
-    return f;
-}
-
-struct LevelTaps {
-    int idx[4];
-    float w[4];        // raw bilinear weights (0 for the dropped corner tap)
-    float dwu[4], dwv[4];   // d w / d fu, d w / d fv
-    float wsum;
-};
-
-__device__ __forceinline__ LevelTaps cs_taps(const FaceMap& f, int R) {
-    const float u = (f.x + 1.f) * 0.5f * R - 0.5f, v = (f.y + 1.f) * 0.5f * R - 0.5f;
-    const float u0f = floorf(u), v0f = floorf(v);
-    const float fu = u - u0f, fv = v - v0f;
-    const int u0 = (int)u0f, v0 = (int)v0f;
-    LevelTaps t;
-    t.wsum = 0.f;
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-        const int du = k & 1, dv = k >> 1;
-        int iu = u0 + du, iv = v0 + dv;
-        const float a = du ? fu : 1.f - fu, b = dv ? fv : 1.f - fv;
-        float w = a * b, dwu = (du ? 1.f : -1.f) * b, dwv = (dv ? 1.f : -1.f) * a;
-        const bool ou = iu < 0 || iu >= R, ov = iv < 0 || iv >= R;
-        int f2 = f.face;
-        if (ou && ov) {
-            w = 0.f; dwu = 0.f; dwv = 0.f;
-            iu = min(max(iu, 0), R - 1); iv = min(max(iv, 0), R - 1);
-        } else if (ou || ov) {
-            const float fx = 2.f * ((float)iu + 0.5f) / R - 1.f, fy = 2.f * ((float)iv + 0.5f) / R - 1.f;
-            float c[3];
-            cs_cube_to_dir(f.face, fx, fy, c);
-            const int major = f.face >> 1;
-            float e = 0.f;
-            int over = -1;
-#pragma unroll
-            for (int a3 = 0; a3 < 3; ++a3)
-                if (a3 != major && fabsf(c[a3]) > 1.f) { e = fabsf(c[a3]) - 1.f; over = a3; }
-#pragma unroll
-            for (int a3 = 0; a3 < 3; ++a3) {
-                if (a3 == over) c[a3] = c[a3] > 0.f ? 1.f : -1.f;
-                if (a3 == major) c[a3] = (c[a3] > 0.f ? 1.f : -1.f) * (1.f - e);
-            }
-            const FaceMap g = cs_face(c);
-            f2 = g.face;
-            iu = min(max((int)floorf((g.x + 1.f) * 0.5f * R), 0), R - 1);
-            iv = min(max((int)floorf((g.y + 1.f) * 0.5f * R), 0), R - 1);
-        }
-        t.idx[k] = (f2 * R + iv) * R + iu;
-        t.w[k] = w; t.dwu[k] = dwu; t.dwv[k] = dwv;
-        t.wsum += w;
-    }
-    return t;
-}
 
 __device__ __forceinline__ void cs_levels(const float* level, int64_t i, int n, int& l0, int& l1, float& f, bool& inside) {
     l0 = 0; l1 = 0; f = 0.f; inside = false;
@@ -120,7 +34,7 @@ __device__ __forceinline__ void cs_levels(const float* level, int64_t i, int n, 
     l1 = min(l0 + 1, n - 1);
 }
 
-__device__ __forceinline__ void cs_fetch(const float* tex, const LevelTaps& t, float s[3]) {
+__device__ __forceinline__ void cs_fetch(const float* tex, const CubeTaps& t, float s[3]) {
     s[0] = s[1] = s[2] = 0.f;
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
@@ -136,14 +50,14 @@ __global__ void __launch_bounds__(256) cube_sample_fwd_kernel(const CubeStack st
     const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (i >= n) return;
     const float d[3] = {dirs[i * 3], dirs[i * 3 + 1], dirs[i * 3 + 2]};
-    const FaceMap fm = cs_face(d);
+    const CubeFace fm = cube_face(d);
     int l0, l1; float f; bool inside;
     cs_levels(level, i, st.n, l0, l1, f, inside);
     float s0[3];
-    cs_fetch(st.tex[l0], cs_taps(fm, st.res[l0]), s0);
+    cs_fetch(st.tex[l0], cube_taps(fm, st.res[l0]), s0);
     if (l1 != l0 && f != 0.f) {
         float s1[3];
-        cs_fetch(st.tex[l1], cs_taps(fm, st.res[l1]), s1);
+        cs_fetch(st.tex[l1], cube_taps(fm, st.res[l1]), s1);
 #pragma unroll
         for (int c = 0; c < 3; ++c) s0[c] = (1.f - f) * s0[c] + f * s1[c];
     }
@@ -151,9 +65,9 @@ __global__ void __launch_bounds__(256) cube_sample_fwd_kernel(const CubeStack st
 }
 
 // adjoint of one level's lookup: scatters g * scale into d_tex, returns S and accumulates (dS/dx, dS/dy) . g * scale
-__device__ __forceinline__ void cs_level_bwd(const float* tex, float* d_tex, const FaceMap& fm, int R, const float g[3], float scale,
+__device__ __forceinline__ void cs_level_bwd(const float* tex, float* d_tex, const CubeFace& fm, int R, const float g[3], float scale,
                                              float s[3], float& gx, float& gy) {
-    const LevelTaps t = cs_taps(fm, R);
+    const CubeTaps t = cube_taps(fm, R);
     cs_fetch(tex, t, s);
     const float inv = 1.f / t.wsum;
     float gu = 0.f, gv = 0.f;
@@ -181,7 +95,7 @@ __global__ void __launch_bounds__(256) cube_sample_bwd_kernel(const CubeStack st
     if (i >= n) return;
     const float d[3] = {dirs[i * 3], dirs[i * 3 + 1], dirs[i * 3 + 2]};
     const float g[3] = {g_out[i * 3], g_out[i * 3 + 1], g_out[i * 3 + 2]};
-    const FaceMap fm = cs_face(d);
+    const CubeFace fm = cube_face(d);
     int l0, l1; float f; bool inside;
     cs_levels(level, i, st.n, l0, l1, f, inside);
     float gx = 0.f, gy = 0.f, s0[3], s1[3] = {0.f, 0.f, 0.f};

@@ -4,25 +4,13 @@
 //   cube_light    : exp(seamless bilinear cube lookup) of the env light      (light.py:125-162) fwd + bwd
 //   mc_estimate   : Cook-Torrance BRDF weights + diffuse / specular estimators (fields.py:977-1033,1146-1234) fwd + bwd
 // One thread per (point, direction) pair for the first two, one warp per point for the estimator.
-#include "common.cuh"
+#include "shading.cuh"
 
 namespace {
 
 constexpr float PI_F = 3.14159265358979323846f;
 constexpr float EPSF = 1e-6f;   // fields.py:18
 
-struct V3 { float x, y, z; };
-__device__ __forceinline__ V3 v3(float x, float y, float z) { return V3{x, y, z}; }
-__device__ __forceinline__ V3 operator+(V3 a, V3 b) { return v3(a.x + b.x, a.y + b.y, a.z + b.z); }
-__device__ __forceinline__ V3 operator-(V3 a, V3 b) { return v3(a.x - b.x, a.y - b.y, a.z - b.z); }
-__device__ __forceinline__ V3 operator*(float s, V3 a) { return v3(s * a.x, s * a.y, s * a.z); }
-__device__ __forceinline__ float dot(V3 a, V3 b) { return a.x * b.x + a.y * b.y + a.z * b.z; }
-__device__ __forceinline__ V3 cross(V3 a, V3 b) { return v3(a.y * b.z - a.z * b.y, a.z * b.x - a.x * b.z, a.x * b.y - a.y * b.x); }
-__device__ __forceinline__ V3 normalize12(V3 a) {   // F.normalize: x / max(|x|, 1e-12)
-    const float n = fmaxf(sqrtf(dot(a, a)), 1e-12f);
-    return v3(a.x / n, a.y / n, a.z / n);
-}
-__device__ __forceinline__ V3 ld3(const float* p, int64_t i) { return v3(p[i * 3], p[i * 3 + 1], p[i * 3 + 2]); }
 __device__ __forceinline__ float clamp01(float x) { return fminf(fmaxf(x, 0.f), 1.f); }
 
 // tangent frame of fields.py:812-822 (x), y = z cross x
@@ -86,81 +74,13 @@ __global__ void __launch_bounds__(128) mc_directions_kernel(int mode, const floa
 }
 
 // ---- cube map --------------------------------------------------------------------------------
-// face convention of network/light_utils.py:24-31 / renderutils/c_src/cubemap.cu:32-60
-__device__ __forceinline__ V3 cube_to_dir(int s, float x, float y) {
-    switch (s) {
-        case 0: return v3(1.f, -y, -x);
-        case 1: return v3(-1.f, -y, x);
-        case 2: return v3(x, 1.f, y);
-        case 3: return v3(x, -1.f, -y);
-        case 4: return v3(x, -y, 1.f);
-        default: return v3(-x, -y, -1.f);
-    }
-}
-__device__ __forceinline__ void dir_to_face_xy(V3 d, int& face, float& x, float& y) {
-    const float ax = fabsf(d.x), ay = fabsf(d.y), az = fabsf(d.z);
-    if (ax >= ay && ax >= az) {
-        const float m = fmaxf(ax, 1e-30f);
-        if (d.x >= 0.f) { face = 0; x = -d.z / m; y = -d.y / m; } else { face = 1; x = d.z / m; y = -d.y / m; }
-    } else if (ay >= az) {
-        const float m = fmaxf(ay, 1e-30f);
-        if (d.y >= 0.f) { face = 2; x = d.x / m; y = d.z / m; } else { face = 3; x = d.x / m; y = -d.z / m; }
-    } else {
-        const float m = fmaxf(az, 1e-30f);
-        if (d.z >= 0.f) { face = 4; x = d.x / m; y = -d.y / m; } else { face = 5; x = -d.x / m; y = -d.y / m; }
-    }
-}
-
-struct CubeTaps { int idx[4]; float w[4]; };   // texel offsets (in texels) + normalised weights
-
-// seamless bilinear footprint: taps leaving the face fold onto the neighbouring face, the tap
-// leaving in both axes (cube corner) is dropped and the weights renormalised
-__device__ __forceinline__ CubeTaps cube_taps(V3 d, int R) {
-    int face;
-    float x, y;
-    dir_to_face_xy(d, face, x, y);
-    const float u = (x + 1.f) * 0.5f * R - 0.5f, v = (y + 1.f) * 0.5f * R - 0.5f;
-    const float u0f = floorf(u), v0f = floorf(v);
-    const float fu = u - u0f, fv = v - v0f;
-    const int u0 = (int)u0f, v0 = (int)v0f;
-    CubeTaps t;
-    float wsum = 0.f;
+// the footprint of dirs[i] with each weight normalised on its own (w_k / W) before the weighted sum; cube_sample.cu divides the
+// sum instead, which rounds differently
+__device__ __forceinline__ CubeTaps light_taps(const float* dirs, int64_t i, int R) {
+    const float d[3] = {dirs[i * 3], dirs[i * 3 + 1], dirs[i * 3 + 2]};
+    CubeTaps t = cube_taps(cube_face(d), R);
 #pragma unroll
-    for (int k = 0; k < 4; ++k) {
-        const int du = k & 1, dv = k >> 1;
-        int iu = u0 + du, iv = v0 + dv;
-        float w = (du ? fu : 1.f - fu) * (dv ? fv : 1.f - fv);
-        const bool ou = iu < 0 || iu >= R, ov = iv < 0 || iv >= R;
-        int f2 = face;
-        if (ou && ov) {
-            w = 0.f;
-            iu = min(max(iu, 0), R - 1); iv = min(max(iv, 0), R - 1);
-        } else if (ou || ov) {
-            const float fx = 2.f * ((float)iu + 0.5f) / R - 1.f, fy = 2.f * ((float)iv + 0.5f) / R - 1.f;
-            V3 pnt = cube_to_dir(face, fx, fy);
-            const int major = face >> 1;
-            float c[3] = {pnt.x, pnt.y, pnt.z};
-            float e = 0.f;
-            int over = -1;
-#pragma unroll
-            for (int a = 0; a < 3; ++a)
-                if (a != major && fabsf(c[a]) > 1.f) { e = fabsf(c[a]) - 1.f; over = a; }
-#pragma unroll
-            for (int a = 0; a < 3; ++a) {
-                if (a == over) c[a] = c[a] > 0.f ? 1.f : -1.f;
-                if (a == major) c[a] = (c[a] > 0.f ? 1.f : -1.f) * (1.f - e);
-            }
-            float x2, y2;
-            dir_to_face_xy(v3(c[0], c[1], c[2]), f2, x2, y2);
-            iu = min(max((int)floorf((x2 + 1.f) * 0.5f * R), 0), R - 1);
-            iv = min(max((int)floorf((y2 + 1.f) * 0.5f * R), 0), R - 1);
-        }
-        t.idx[k] = (f2 * R + iv) * R + iu;
-        t.w[k] = w;
-        wsum += w;
-    }
-#pragma unroll
-    for (int k = 0; k < 4; ++k) t.w[k] /= wsum;
+    for (int k = 0; k < 4; ++k) t.w[k] /= t.wsum;
     return t;
 }
 
@@ -171,7 +91,7 @@ __global__ void __launch_bounds__(256) cube_light_fwd_kernel(const float* __rest
     if (i >= P) return;
     float r = 0.f, g = 0.f, b = 0.f;
     if (!mask || mask[i]) {
-        const CubeTaps t = cube_taps(ld3(dirs, i), R);
+        const CubeTaps t = light_taps(dirs, i, R);
 #pragma unroll
         for (int k = 0; k < 4; ++k) {
             const float* px = base + (size_t)t.idx[k] * 3;
@@ -190,7 +110,7 @@ __global__ void __launch_bounds__(256) cube_light_bwd_kernel(int R, const float*
     if (mask && !mask[i]) return;
     const float gr = g_out[i * 3] * out[i * 3], gg = g_out[i * 3 + 1] * out[i * 3 + 1], gb = g_out[i * 3 + 2] * out[i * 3 + 2];
     if (gr == 0.f && gg == 0.f && gb == 0.f) return;
-    const CubeTaps t = cube_taps(ld3(dirs, i), R);
+    const CubeTaps t = light_taps(dirs, i, R);
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
         if (t.w[k] == 0.f) continue;
@@ -415,50 +335,22 @@ __global__ void __launch_bounds__(256) mc_estimate_bwd_kernel(const float* __res
 // X[i, 0:51] = posenc(p, 8), X[i, 51:123] = IDE(reflect(v, n)) with kappa_inv = 0 (utils/ref_utils.py:53-117, degree 5: 36 (m, l)
 // pairs), X[i, 123:ldx] = 0, for the i-th occluded (point, direction) pair: p = inters[idx[i]], v = -dirs[idx[i]],
 // n = normalize(hit_normals[idx[i]]).  One thread per hit; the IDE polynomial table mat[17, 36] sits in shared memory.
-constexpr int IDE_NP = 17, IDE_N = 36, PE_L = 8;
+constexpr int PE_L = 8;
 __global__ void __launch_bounds__(128) hit_encode_kernel(const float* __restrict__ inters, const float* __restrict__ dirs,
                                                          const float* __restrict__ hit_normals, const int64_t* __restrict__ idx, int64_t M,
                                                          const float* __restrict__ ide_mat, const int32_t* __restrict__ ide_m, int ldx,
                                                          float* __restrict__ X) {
     __shared__ float s_mat[IDE_NP * IDE_N];
     __shared__ int s_m[IDE_N];
-    for (int i = threadIdx.x; i < IDE_NP * IDE_N; i += blockDim.x) s_mat[i] = ide_mat[i];
-    for (int i = threadIdx.x; i < IDE_N; i += blockDim.x) s_m[i] = ide_m[i];
-    __syncthreads();
+    ide_load(ide_mat, ide_m, nullptr, s_mat, s_m, nullptr);
     const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (i >= M) return;
     const int64_t o = idx[i];
     const V3 p = ld3(inters, o), v = -1.f * ld3(dirs, o), n = normalize12(ld3(hit_normals, o));
     const V3 r = (dot(v, n) * 2.f) * n - v;
     float* x = X + i * ldx;
-    const float pc[3] = {p.x, p.y, p.z};
-#pragma unroll
-    for (int c = 0; c < 3; ++c) x[c] = pc[c];
-#pragma unroll
-    for (int k = 0; k < PE_L; ++k) {
-        const float f = (float)(1 << k);
-#pragma unroll
-        for (int c = 0; c < 3; ++c) { x[3 + k * 6 + c] = sinf(pc[c] * f); x[3 + k * 6 + 3 + c] = cosf(pc[c] * f); }
-    }
-    float zk[IDE_NP], re[IDE_NP], im[IDE_NP];
-    zk[0] = 1.f; re[0] = 1.f; im[0] = 0.f;
-#pragma unroll
-    for (int k = 1; k < IDE_NP; ++k) {
-        zk[k] = zk[k - 1] * r.z;
-        re[k] = re[k - 1] * r.x - im[k - 1] * r.y;
-        im[k] = re[k - 1] * r.y + im[k - 1] * r.x;
-    }
-    for (int j = 0; j < IDE_N; ++j) {
-        float poly = 0.f;
-#pragma unroll
-        for (int k = 0; k < IDE_NP; ++k) poly = fmaf(zk[k], s_mat[k * IDE_N + j], poly);
-        const int m = s_m[j];
-        float rm = 0.f, imm = 0.f;
-#pragma unroll
-        for (int k = 0; k < IDE_NP; ++k) if (k == m) { rm = re[k]; imm = im[k]; }
-        x[51 + j] = rm * poly;
-        x[51 + IDE_N + j] = imm * poly;
-    }
+    posenc3(x, p, PE_L);
+    ide_encode(x + 51, r, s_mat, s_m, nullptr, 0.f);
     for (int c = 51 + 2 * IDE_N; c < ldx; ++c) x[c] = 0.f;
 }
 

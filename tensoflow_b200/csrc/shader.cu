@@ -9,33 +9,11 @@
 //   shader_combine : material affine maps, split-sum FG LUT (bilinear, clamp), diffuse + specular combination with the
 //                    occlusion blend, linear -> sRGB, clamp
 // each with a hand-derived backward.  One thread per sample; HBM-bound (the encode writes ~1.6 KB per sample).
-#include "common.cuh"
+#include "shading.cuh"
 
 namespace {
 
-constexpr int IDE_NP = 17, IDE_N = 36;          // powers of z, (m, l) entries of the degree-5 encoding
 constexpr int PE_PTS = 8, PE_VIEW = 4, PE_REFL = 6;
-
-struct V3 { float x, y, z; };
-__device__ __forceinline__ V3 v3(float x, float y, float z) { return V3{x, y, z}; }
-__device__ __forceinline__ float dot(V3 a, V3 b) { return a.x * b.x + a.y * b.y + a.z * b.z; }
-__device__ __forceinline__ V3 ld3(const float* p, int64_t i) { return v3(p[i * 3], p[i * 3 + 1], p[i * 3 + 2]); }
-__device__ __forceinline__ V3 normalize12(V3 a, float& len) {   // F.normalize: x / max(|x|, 1e-12)
-    len = fmaxf(sqrtf(dot(a, a)), 1e-12f);
-    return v3(a.x / len, a.y / len, a.z / len);
-}
-
-// [v, sin(2^k v), cos(2^k v)]_{k < L} -> 3 + 6 L floats (utils/network_utils.py:38-50)
-__device__ __forceinline__ void posenc3(float* x, V3 v, int L) {
-    const float c[3] = {v.x, v.y, v.z};
-#pragma unroll
-    for (int a = 0; a < 3; ++a) x[a] = c[a];
-    for (int k = 0; k < L; ++k) {
-        const float f = (float)(1 << k);
-#pragma unroll
-        for (int a = 0; a < 3; ++a) { x[3 + k * 6 + a] = sinf(c[a] * f); x[3 + k * 6 + 3 + a] = cosf(c[a] * f); }
-    }
-}
 
 struct IdeTables { const float* mat; const int32_t* m; const float* sigma; };   // [17,36], [36], [36] (device)
 
@@ -77,9 +55,7 @@ __global__ void __launch_bounds__(128) shader_encode_fwd_kernel(EncParams p) {
     __shared__ float s_mat[IDE_NP * IDE_N];
     __shared__ float s_sig[IDE_N];
     __shared__ int s_m[IDE_N];
-    for (int i = threadIdx.x; i < IDE_NP * IDE_N; i += blockDim.x) s_mat[i] = p.ide.mat[i];
-    for (int i = threadIdx.x; i < IDE_N; i += blockDim.x) { s_m[i] = p.ide.m[i]; s_sig[i] = p.ide.sigma[i]; }
-    __syncthreads();
+    ide_load(p.ide.mat, p.ide.m, p.ide.sigma, s_mat, s_m, s_sig);
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     float* tile = enc_sm + warp * 32 * ENC_TS;
     float* x = tile + lane * ENC_TS;                 // this sample's staging row
@@ -99,26 +75,7 @@ __global__ void __launch_bounds__(128) shader_encode_fwd_kernel(EncParams p) {
         p.rough[i] = g.rough;
         // ---- [PE(points, 8) | IDE(mirror direction, roughness) | 0] into the staging row -------------------------------
         posenc3(x, pt, PE_PTS);
-        float zk[IDE_NP], re[IDE_NP], im[IDE_NP];
-        zk[0] = 1.f; re[0] = 1.f; im[0] = 0.f;
-#pragma unroll
-        for (int k = 1; k < IDE_NP; ++k) {
-            zk[k] = zk[k - 1] * g.r.z;
-            re[k] = re[k - 1] * g.r.x - im[k - 1] * g.r.y;
-            im[k] = re[k - 1] * g.r.y + im[k - 1] * g.r.x;
-        }
-        for (int j = 0; j < IDE_N; ++j) {
-            float poly = 0.f;
-#pragma unroll
-            for (int k = 0; k < IDE_NP; ++k) poly = fmaf(zk[k], s_mat[k * IDE_N + j], poly);
-            const float att = poly * expf(-s_sig[j] * g.rough);
-            const int m = s_m[j];
-            float rm = 0.f, imm = 0.f;
-#pragma unroll
-            for (int k = 0; k < IDE_NP; ++k) if (k == m) { rm = re[k]; imm = im[k]; }
-            x[51 + j] = rm * att;
-            x[51 + IDE_N + j] = imm * att;
-        }
+        ide_encode(x + 51, g.r, s_mat, s_m, s_sig, g.rough);
         for (int c = 51 + 2 * IDE_N; c < LD_IL; ++c) x[c] = 0.f;
     }
     __syncwarp();
@@ -160,9 +117,7 @@ __global__ void __launch_bounds__(128) shader_encode_bwd_kernel(EncBwdParams p) 
     __shared__ float s_mat[IDE_NP * IDE_N];
     __shared__ float s_sig[IDE_N];
     __shared__ int s_m[IDE_N];
-    for (int i = threadIdx.x; i < IDE_NP * IDE_N; i += blockDim.x) s_mat[i] = p.ide.mat[i];
-    for (int i = threadIdx.x; i < IDE_N; i += blockDim.x) { s_m[i] = p.ide.m[i]; s_sig[i] = p.ide.sigma[i]; }
-    __syncthreads();
+    ide_load(p.ide.mat, p.ide.m, p.ide.sigma, s_mat, s_m, s_sig);
     const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (i >= p.n) return;
     const Geo g = shader_geo(p.normals, p.view, p.mat, i);
@@ -182,13 +137,7 @@ __global__ void __launch_bounds__(128) shader_encode_bwd_kernel(EncBwdParams p) 
     if (p.g_Xil) {   // adjoint of the integrated directional encoding wrt the mirror direction and the roughness
         const float* gx = p.g_Xil + i * LD_IL + 51;
         float zk[IDE_NP], re[IDE_NP], im[IDE_NP], dre[IDE_NP], dim_[IDE_NP];
-        zk[0] = 1.f; re[0] = 1.f; im[0] = 0.f;
-#pragma unroll
-        for (int k = 1; k < IDE_NP; ++k) {
-            zk[k] = zk[k - 1] * g.r.z;
-            re[k] = re[k - 1] * g.r.x - im[k - 1] * g.r.y;
-            im[k] = re[k - 1] * g.r.y + im[k - 1] * g.r.x;
-        }
+        ide_powers(g.r, zk, re, im);
 #pragma unroll
         for (int k = 0; k < IDE_NP; ++k) { dre[k] = 0.f; dim_[k] = 0.f; }
         float dz = 0.f;
@@ -203,9 +152,8 @@ __global__ void __launch_bounds__(128) shader_encode_bwd_kernel(EncBwdParams p) 
             const float e = expf(-s_sig[j] * g.rough);
             const float att = poly * e;
             const int m = s_m[j];
-            float rm = 0.f, imm = 0.f;
-#pragma unroll
-            for (int k = 0; k < IDE_NP; ++k) if (k == m) { rm = re[k]; imm = im[k]; }
+            float rm, imm;
+            ide_pick(re, im, m, rm, imm);
             const float gre = gx[j], gim = gx[IDE_N + j];
             const float G = gre * rm + gim * imm;                 // d / d att
             dz += G * e * dpoly_dz;

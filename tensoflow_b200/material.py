@@ -50,7 +50,7 @@ def sample_sphere(num_samples, begin_elevation=0):
     return np.array(az), np.array(el)
 
 
-# ---- integrated directional encoding (reference utils/ref_utils.py:8-117), kappa_inv = 0 ----
+# ---- integrated directional encoding (reference utils/ref_utils.py:8-117) ----
 def _ide_tables(deg_view=5):
     ml = []
     for i in range(deg_view):
@@ -72,16 +72,25 @@ def _ide_tables(deg_view=5):
     return ml, mat.astype(np.float32)
 
 
-_IDE_CACHE = {}
+_IDE_DEV = {}
 
 
-def ide_encode(xyz: torch.Tensor) -> torch.Tensor:
-    """generate_ide_fn(5)(xyz, 0) -> [N,72] with real arithmetic: (x+iy)^m by recurrence."""
-    key = xyz.device
-    if key not in _IDE_CACHE:
+def _ide_device_tables(device):
+    """The degree-5 IDE tables on `device`: polynomial table mat [17,36] fp32, the order m of its 36 entries (int32) and
+    sigma = l (l + 1) / 2 [36] fp32.  tf_hit_encode takes (mat, m), tf_shader_encode_* all three."""
+    key = str(device)
+    if key not in _IDE_DEV:
         ml, mat = _ide_tables(5)
-        _IDE_CACHE[key] = (torch.from_numpy(ml[0].astype(np.int64)).to(xyz.device), torch.from_numpy(mat).to(xyz.device))
-    m_idx, mat = _IDE_CACHE[key]
+        _IDE_DEV[key] = (torch.from_numpy(np.ascontiguousarray(mat, dtype=np.float32)).to(device).contiguous(),
+                         torch.from_numpy(ml[0].astype(np.int32)).to(device).contiguous(),
+                         torch.from_numpy((0.5 * ml[1] * (ml[1] + 1)).astype(np.float32)).to(device).contiguous())
+    return _IDE_DEV[key]
+
+
+def ide_encode(xyz: torch.Tensor, kappa_inv: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """generate_ide_fn(5)(xyz, kappa_inv) -> [N,72] with real arithmetic: (x+iy)^m by recurrence.  kappa_inv [N,1] attenuates
+    entry (m, l) by exp(-l (l + 1) / 2 kappa_inv); None is kappa_inv = 0 and skips the multiply."""
+    mat, m_idx, sigma = _ide_device_tables(xyz.device)
     x, y, z = xyz[:, 0:1], xyz[:, 1:2], xyz[:, 2:3]
     n_pow = mat.shape[0]
     zs = [torch.ones_like(z)]
@@ -94,8 +103,10 @@ def ide_encode(xyz: torch.Tensor) -> torch.Tensor:
         im.append(im_n)
     vmz = torch.cat(zs, -1)
     re, im = torch.cat(re, -1).index_select(1, m_idx), torch.cat(im, -1).index_select(1, m_idx)   # backward = index_add, not a sorted index_put
-    poly = vmz @ mat
-    return torch.cat([re * poly, im * poly], -1)
+    att = vmz @ mat
+    if kappa_inv is not None:
+        att = att * torch.exp(-sigma * kappa_inv)
+    return torch.cat([re * att, im * att], -1)
 
 
 def make_predictor(n_layers, feats_dim, output_dim, run_dim=None):
@@ -109,19 +120,6 @@ def make_predictor(n_layers, feats_dim, output_dim, run_dim=None):
         last = run_dim
     layers += [wn(nn.Linear(last, output_dim)), nn.Identity()]
     return nn.Sequential(*layers)
-
-
-_IDE_DEV = {}
-
-
-def _ide_device_tables(device):
-    """IDE polynomial table [17,36] fp32 and the order m of its 36 entries (int32) on the device, for tf_hit_encode."""
-    key = str(device)
-    if key not in _IDE_DEV:
-        ml, mat = _ide_tables(5)
-        _IDE_DEV[key] = (torch.from_numpy(np.ascontiguousarray(mat, dtype=np.float32)).to(device).contiguous(),
-                         torch.from_numpy(ml[0].astype(np.int32)).to(device).contiguous())
-    return _IDE_DEV[key]
 
 
 def run_predictor_padded(seq: nn.Sequential, x_padded, k_valid: int, final_act: str, act_param: float = 0.0):
@@ -328,7 +326,7 @@ class MCShadingNetwork(nn.Module):
         if idx.numel() > 0:                                           # occluded directions: indirect-light MLP
             # [posenc(hit point, 8) | IDE(view mirrored at the hit normal)] of the hit records in one kernel, already padded to
             # the 128 columns the tensor-core first layer wants
-            ide_mat, ide_m = _ide_device_tables(pts.device)
+            ide_mat, ide_m, _ = _ide_device_tables(pts.device)
             enc = mc_ops.hit_encode(inters, dirs, hit_normals, idx, ide_mat, ide_m, 128)
             inner = run_predictor_padded(self.inner_light, enc, 123, "exp", self.cfg['inner_light_exp_max'])
             lights = lights.index_add(0, idx, inner)

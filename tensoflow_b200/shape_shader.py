@@ -1,11 +1,9 @@
 """Shape-stage shader (reference network/fields.py:320-575 ShapeShadingNetwork) and its
 prefiltered environment light (reference network/light.py:8-122).
 
-Round-1 structure: the MLP stacks (material / indirect light / occlusion / radiance heads) run
-on the fused linear kernels, the cubemap prefilter on the cached CSR operator kernel; the
-per-sample encodings and the (direction- and level-differentiable) cube / LUT lookups are
-tensor arithmetic on the device with autograd (next: fold them into one per-sample kernel,
-see DESIGN.md).
+The MLP heads (material / indirect light / occlusion / radiance) run on the fused linear kernels, the cubemap prefilter on
+the cached CSR operator kernel, the per-sample encodings and the combine on the tf_shader_* kernels, and the
+(direction- and level-differentiable) cube lookups on tf_cube_sample_*.
 """
 from __future__ import annotations
 
@@ -22,7 +20,7 @@ import torch.nn.functional as F
 from . import _lib, ops
 from ._lib import check, ptr, stream_ptr
 from .flow import posenc
-from .material import make_predictor, run_predictor, run_predictor_padded, linear_to_srgb, _ide_tables
+from .material import make_predictor, run_predictor, run_predictor_padded, linear_to_srgb, _ide_device_tables
 
 
 # ---- cube geometry (reference network/light_utils.py:24-31, renderutils/c_src/cubemap.cu:32-60) ----
@@ -35,72 +33,9 @@ def cube_to_dir_t(face: torch.Tensor, x: torch.Tensor, y: torch.Tensor) -> torch
     return out
 
 
-def dir_to_face_xy(d: torch.Tensor):
-    ax = d.abs()
-    dx, dy, dz = d[..., 0], d[..., 1], d[..., 2]
-    is_x = (ax[..., 0] >= ax[..., 1]) & (ax[..., 0] >= ax[..., 2])
-    is_y = (~is_x) & (ax[..., 1] >= ax[..., 2])
-    face = torch.where(is_x, torch.where(dx >= 0, 0, 1), torch.where(is_y, torch.where(dy >= 0, 2, 3), torch.where(dz >= 0, 4, 5)))
-    m = torch.where(is_x, ax[..., 0], torch.where(is_y, ax[..., 1], ax[..., 2])).clamp_min(1e-30)
-    xs = [-dz, dz, dx, dx, dx, -dx]
-    ys = [-dy, -dy, dz, -dz, -dy, -dy]
-    x, y = xs[5], ys[5]
-    for s in range(4, -1, -1):
-        x = torch.where(face == s, xs[s], x)
-        y = torch.where(face == s, ys[s], y)
-    return face, x / m, y / m
-
-
-def cube_taps(R: int, d: torch.Tensor):
-    """The four texel taps of a seamless bilinear cube lookup at directions d [N,3] on a [6,R,R,C] texture:
-    -> (idx [N,4] flat texel indices, w [N,4] normalised weights, differentiable in d).  Taps that leave the face fold onto
-    the neighbouring face, the tap leaving in both axes is dropped and the weights renormalised."""
-    face, x, y = dir_to_face_xy(d)
-    u = (x + 1.0) * 0.5 * R - 0.5
-    v = (y + 1.0) * 0.5 * R - 0.5
-    u0, v0 = torch.floor(u), torch.floor(v)
-    fu, fv = u - u0, v - v0
-    u0, v0 = u0.long(), v0.long()
-    major = face // 2
-    ar = torch.arange(3, device=d.device)
-    is_major = ar[None, :] == major[:, None]
-    idx, ws = [], []
-    for du, dv in ((0, 0), (1, 0), (0, 1), (1, 1)):
-        iu, iv = u0 + du, v0 + dv
-        w = (fu if du else 1 - fu) * (fv if dv else 1 - fv)
-        ou, ov = (iu < 0) | (iu >= R), (iv < 0) | (iv >= R)
-        fx = 2.0 * (iu.to(d.dtype) + 0.5) / R - 1.0
-        fy = 2.0 * (iv.to(d.dtype) + 0.5) / R - 1.0
-        p = cube_to_dir_t(face, fx, fy)
-        ex = (p.abs() - 1.0).clamp_min(0.0)
-        ex = torch.where(is_major, torch.zeros_like(ex), ex)
-        e = ex.sum(-1, keepdim=True)
-        q = torch.where(ex > 0, torch.sign(p), p)
-        q = torch.where(is_major, torch.sign(p) * (1.0 - e), q)
-        f2, x2, y2 = dir_to_face_xy(q)
-        iu2 = torch.floor((x2 + 1.0) * 0.5 * R).long().clamp(0, R - 1)
-        iv2 = torch.floor((y2 + 1.0) * 0.5 * R).long().clamp(0, R - 1)
-        fold = ou ^ ov
-        f_use = torch.where(fold, f2, face)
-        iu_use = torch.where(fold, iu2, iu.clamp(0, R - 1))
-        iv_use = torch.where(fold, iv2, iv.clamp(0, R - 1))
-        idx.append((f_use * R + iv_use) * R + iu_use)
-        ws.append(torch.where(ou & ov, torch.zeros_like(w), w))
-    w = torch.stack(ws, -1)
-    return torch.stack(idx, -1), w / w.sum(-1, keepdim=True)
-
-
-def cube_sample(tex: torch.Tensor, d: torch.Tensor) -> torch.Tensor:
-    """Seamless bilinear lookup (dr.texture(..., boundary_mode='cube'), reference light.py:107,135):
-    tex [6,R,R,C], d [N,3] -> [N,C]; differentiable in tex and d."""
-    idx, w = cube_taps(tex.shape[1], d)
-    return (tex.reshape(-1, tex.shape[-1])[idx] * w.unsqueeze(-1)).sum(1)
-
-
 class CubeSampleFunction(torch.autograd.Function):
     """Seamless (tri)linear cube lookup on `tf_cube_sample_fwd/bwd`, differentiable in the textures, the direction and the level:
-    (d [N,3], level [N] or None, *texs [6,R_l,R_l,3]) -> [N,3].  Same arithmetic as `cube_sample` / `cube_sample_mip` below (which
-    stay as the tensor formulation the kernel is tested against)."""
+    (d [N,3], level [N] or None, *texs [6,R_l,R_l,3]) -> [N,3]."""
 
     @staticmethod
     def forward(ctx, d, level, *texs):
@@ -144,22 +79,6 @@ def cube_lookup(texs: List[torch.Tensor], d: torch.Tensor, level: Optional[torch
     return CubeSampleFunction.apply(d, level, *texs)
 
 
-def cube_sample_mip(stack: List[torch.Tensor], d: torch.Tensor, level: torch.Tensor) -> torch.Tensor:
-    """linear-mipmap-linear over a user-supplied stack (reference light.py:111-118); differentiable in
-    the textures, the direction and the level."""
-    n = len(stack)
-    lv = level.reshape(-1).clamp(0.0, float(n - 1))
-    l0 = torch.floor(lv)
-    f = (lv - l0).unsqueeze(-1)
-    l0 = l0.long()
-    l1 = (l0 + 1).clamp(max=n - 1)
-    out = 0
-    for l in range(n):
-        w = (l0 == l).unsqueeze(-1) * (1 - f) + ((l1 == l) & (l0 != l)).unsqueeze(-1) * f
-        out = out + cube_sample(stack[l], d) * w
-    return out
-
-
 def texture2d_linear_clamp(tex: torch.Tensor, uv: torch.Tensor) -> torch.Tensor:
     """dr.texture(tex[None], uv, filter_mode='linear', boundary_mode='clamp') (reference fields.py:522):
     tex [H,W,C], uv [N,2]; differentiable in uv."""
@@ -171,29 +90,6 @@ def texture2d_linear_clamp(tex: torch.Tensor, uv: torch.Tensor) -> torch.Tensor:
     y0i, y1i = y0.long().clamp(0, H - 1), (y0.long() + 1).clamp(0, H - 1)
     return (tex[y0i, x0i] * (1 - fx) * (1 - fy) + tex[y0i, x1i] * fx * (1 - fy)
             + tex[y1i, x0i] * (1 - fx) * fy + tex[y1i, x1i] * fx * fy)
-
-
-_IDE = {}
-
-
-def ide_encode_rough(xyz: torch.Tensor, kappa_inv: torch.Tensor) -> torch.Tensor:
-    """Integrated directional encoding (reference utils/ref_utils.py:53-117) -> [N,72]."""
-    if xyz.device not in _IDE:
-        ml, mat = _ide_tables(5)
-        _IDE[xyz.device] = (torch.from_numpy(ml[0].astype(np.int64)).to(xyz.device), torch.from_numpy(mat).to(xyz.device),
-                            torch.from_numpy((0.5 * ml[1] * (ml[1] + 1)).astype(np.float32)).to(xyz.device))
-    m_idx, mat, sigma = _IDE[xyz.device]
-    x, y, z = xyz[:, 0:1], xyz[:, 1:2], xyz[:, 2:3]
-    zs, re, im = [torch.ones_like(z)], [torch.ones_like(x)], [torch.zeros_like(x)]
-    for _ in range(1, mat.shape[0]):
-        zs.append(zs[-1] * z)
-        re_n, im_n = re[-1] * x - im[-1] * y, re[-1] * y + im[-1] * x
-        re.append(re_n)
-        im.append(im_n)
-    vmz = torch.cat(zs, -1)
-    re, im = torch.cat(re, -1).index_select(1, m_idx), torch.cat(im, -1).index_select(1, m_idx)   # backward = index_add, not a sorted index_put
-    att = (vmz @ mat) * torch.exp(-sigma * kappa_inv)
-    return torch.cat([re * att, im * att], -1)
 
 
 # ---- cubemap prefilter operators (reference renderutils/c_src/cubemap.cu:17-60,110-350) ----------------
@@ -300,22 +196,15 @@ class CubemapMip(torch.autograd.Function):
     def forward(ctx, cubemap):
         return F.avg_pool2d(cubemap.permute(0, 3, 1, 2), (2, 2)).permute(0, 2, 3, 1).contiguous()
 
-    _taps = {}      # (res, device) -> taps of the fine texel centres: constant geometry, built once
+    _dirs = {}      # res, device -> the normalised fine texel centre directions: constant geometry, built once
 
     @staticmethod
     def backward(ctx, dout):
         res = dout.shape[1] * 2
         key = (res, str(dout.device))
-        if key not in CubemapMip._taps:
-            with torch.no_grad():
-                c = torch.linspace(-1.0 + 1.0 / res, 1.0 - 1.0 / res, res, device=dout.device)
-                gy, gx = torch.meshgrid(c, c, indexing="ij")
-                face = torch.arange(6, device=dout.device)[:, None, None].expand(6, res, res)
-                v = F.normalize(cube_to_dir_t(face, gx.expand(6, res, res), gy.expand(6, res, res)), dim=-1, eps=1e-20)
-                CubemapMip._taps[key] = cube_taps(dout.shape[1], v.reshape(-1, 3))
-        idx, w = CubemapMip._taps[key]
-        src = (dout * 0.25).reshape(-1, dout.shape[-1])
-        return (src[idx] * w.unsqueeze(-1)).sum(1).reshape(6, res, res, -1)
+        if key not in CubemapMip._dirs:
+            CubemapMip._dirs[key] = _texel_dirs(res, dout.device)
+        return cube_lookup([dout * 0.25], CubemapMip._dirs[key]).reshape(6, res, res, -1)
 
 
 class ShadingEnvLight(nn.Module):
@@ -352,27 +241,6 @@ class ShadingEnvLight(nn.Module):
         return torch.exp(cube_lookup(self.specular, l, self.get_mip(roughness)[..., 0]))
 
 
-_IDE_ROUGH_DEV = {}
-
-
-def _ide_rough_tables(device):
-    """device copies of the degree-5 IDE tables for tf_shader_encode_*: mat [17,36] fp32, m [36] int32, sigma = l (l + 1) / 2 [36]"""
-    key = str(device)
-    if key not in _IDE_ROUGH_DEV:
-        ml, mat = _ide_tables(5)
-        _IDE_ROUGH_DEV[key] = (torch.from_numpy(np.ascontiguousarray(mat, dtype=np.float32)).to(device).contiguous(),
-                               torch.from_numpy(ml[0].astype(np.int32)).to(device).contiguous(),
-                               torch.from_numpy((0.5 * ml[1] * (ml[1] + 1)).astype(np.float32)).to(device).contiguous())
-    return _IDE_ROUGH_DEV[key]
-
-
-def _c32(t):
-    t = t.detach()
-    if t.dtype != torch.float32:
-        t = t.float()
-    return t if t.is_contiguous() else t.contiguous()
-
-
 class ShaderEncodeFunction(torch.autograd.Function):
     """Normalised normal / view, mirror direction, N.V, roughness and the zero-padded inputs of the radiance, indirect-light
     and occlusion heads (reference fields.py:453-501) in one kernel; backward in one kernel (IDE / mirror / normalisation
@@ -382,12 +250,11 @@ class ShaderEncodeFunction(torch.autograd.Function):
     @staticmethod
     def forward(ctx, points, normals, view_dirs, mat, feat):
         lib = _lib.load()
-        pc, nc, vc, mc = _c32(points), _c32(normals), _c32(view_dirs), _c32(mat)
-        fc = None if feat is None else _c32(feat)
+        pc, nc, vc, mc, fc = (ops._f32c(t) for t in (points, normals, view_dirs, mat, feat))
         n, dev = pc.shape[0], pc.device
         fd = 0 if fc is None else int(fc.shape[1])
         ld_rad = 0 if fc is None else (fd + 33 + 15) // 16 * 16
-        ide = _ide_rough_tables(dev)
+        ide = _ide_device_tables(dev)
         f32 = dict(device=dev, dtype=torch.float32)
         nrm, vdir, refl = torch.empty(n, 3, **f32), torch.empty(n, 3, **f32), torch.empty(n, 3, **f32)
         nov, rough = torch.empty(n, **f32), torch.empty(n, **f32)
@@ -409,8 +276,8 @@ class ShaderEncodeFunction(torch.autograd.Function):
         nc, vc, mc = ctx.saved_tensors
         fd, ld_rad, has_feat = ctx.dims
         n, dev = nc.shape[0], nc.device
-        ide = _ide_rough_tables(dev)
-        gs = [None if g is None else _c32(g) for g in (g_nrm, g_refl, g_nov, g_rough, g_Xrad, g_Xil)]
+        ide = _ide_device_tables(dev)
+        gs = [ops._f32c(g) for g in (g_nrm, g_refl, g_nov, g_rough, g_Xrad, g_Xil)]
         d_normals = torch.empty(n, 3, device=dev, dtype=torch.float32)
         d_mat = torch.zeros(n, 5, device=dev, dtype=torch.float32)
         d_mat3 = torch.empty(n, device=dev, dtype=torch.float32)
@@ -433,7 +300,7 @@ class ShaderCombineFunction(torch.autograd.Function):
     @staticmethod
     def forward(ctx, mat, diffuse_light, direct_light, indirect_light, w_raw, nov, lut):
         lib = _lib.load()
-        t = [_c32(x) for x in (mat, diffuse_light, direct_light, indirect_light, w_raw.reshape(-1), nov.reshape(-1), lut)]
+        t = [ops._f32c(x) for x in (mat, diffuse_light, direct_light, indirect_light, w_raw.reshape(-1), nov.reshape(-1), lut)]
         n, dev = t[0].shape[0], t[0].device
         color = torch.empty(n, 3, device=dev, dtype=torch.float32)
         occ = torch.empty(n, device=dev, dtype=torch.float32)
@@ -450,8 +317,8 @@ class ShaderCombineFunction(torch.autograd.Function):
         lib = _lib.load()
         t = list(ctx.saved_tensors)
         n, dev = t[0].shape[0], t[0].device
-        gc = _c32(g_color) if g_color is not None else torch.zeros(n, 3, device=dev, dtype=torch.float32)
-        go = None if g_occ is None else _c32(g_occ.reshape(-1))
+        gc = ops._f32c(g_color) if g_color is not None else torch.zeros(n, 3, device=dev, dtype=torch.float32)
+        go = None if g_occ is None else ops._f32c(g_occ.reshape(-1))
         f32 = dict(device=dev, dtype=torch.float32)
         d_mat, d_dif, d_dir, d_ind = torch.empty(n, 5, **f32), torch.empty(n, 3, **f32), torch.empty(n, 3, **f32), torch.empty(n, 3, **f32)
         d_w, d_nov = torch.empty(n, **f32), torch.empty(n, **f32)

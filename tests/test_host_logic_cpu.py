@@ -102,7 +102,7 @@ def test_surface_refinement_helpers_match_reference():
     assert torch.equal(got, want)
 
 
-def test_alpha_mask_encodings_and_losses_match_reference():
+def test_alpha_mask_encodings_one_ide_and_losses_match_reference():
     golden_pins.check("test_host_logic_cpu", "encodings", PINS["encodings"]())
     if not ref_shim.available():
         return
@@ -113,7 +113,6 @@ def test_alpha_mask_encodings_and_losses_match_reference():
     from tensoflow_b200 import shape_renderer as P
     from tensoflow_b200.flow import posenc
     from tensoflow_b200.material import ide_encode
-    from tensoflow_b200.shape_shader import ide_encode_rough
     torch.manual_seed(3)
     aabb = torch.tensor([[-1.0, -0.8, -1.2], [1.0, 0.9, 1.1]])
     vol = (torch.rand(12, 10, 14) > 0.6).float()
@@ -132,7 +131,7 @@ def test_alpha_mask_encodings_and_losses_match_reference():
     want0, want1 = MC.ide_encode(d.double(), 0), MC.ide_encode(d.double(), rough.double())
     # fp32 evaluation of the degree-16 harmonics carries ~4e-3 of rounding in the reference as well
     assert rel_err(ide_encode(d), want0) < 4 * max(rel_err(ide(d, torch.zeros(400, 1)), want0), 1e-4)
-    assert rel_err(ide_encode_rough(d, rough), want1) < 4 * max(rel_err(ide(d, rough), want1), 1e-4)
+    assert rel_err(ide_encode(d, rough), want1) < 4 * max(rel_err(ide(d, rough), want1), 1e-4)
     pr, gt = torch.rand(64, 3), torch.rand(64, 3)
     assert torch.equal(P.charbonnier(pr, gt), torch.sqrt(torch.sum((gt - pr) ** 2, dim=-1) + 0.001))   # shapeRenderer.py:803-805
 
@@ -221,7 +220,6 @@ def _surface_values():
 def _encoding_values():
     from tensoflow_b200.flow import posenc
     from tensoflow_b200.material import ide_encode
-    from tensoflow_b200.shape_shader import ide_encode_rough
     from oracle import torch_oracle_renderer as OR
     torch.manual_seed(3)
     aabb = torch.tensor([[-1.0, -0.8, -1.2], [1.0, 0.9, 1.1]])
@@ -231,7 +229,7 @@ def _encoding_values():
     out += [(f"posenc{m}", posenc(x, m), 0) for m in (3, 4, 6, 8)]
     d = F.normalize(torch.randn(400, 3), dim=-1)
     rough = torch.rand(400, 1)
-    return out + [("ide", ide_encode(d), 0), ("ide_rough", ide_encode_rough(d, rough), 0)]
+    return out + [("ide", ide_encode(d), 0), ("ide_rough", ide_encode(d, rough), 0)]
 
 
 def _loss_values():

@@ -111,6 +111,35 @@ def test_cube_light_forward_backward():
     assert rel_err(b.grad, g64) < max(1e-4, 4 * rel_err(g32, g64))
 
 
+def test_hit_encode_matches_posenc_and_ide():
+    """tf_hit_encode, the inner-light MLP input of the occluded pairs, against fp64 posenc(p, 8) | IDE(reflect(v, n), kappa_inv = 0)
+    of the oracle, and the zero padding up to ldx."""
+    from tensoflow_b200 import mc_ops
+    from tensoflow_b200.flow import posenc
+    from tensoflow_b200.material import _ide_device_tables
+    dev = _cuda()
+    g = torch.Generator().manual_seed(2)
+    K, M = 20000, 6000
+    inters = torch.rand(K, 3, generator=g) * 2.4 - 1.2
+    dirs = F.normalize(torch.randn(K, 3, generator=g), dim=-1)
+    hit_normals = torch.randn(K, 3, generator=g) * (0.5 + torch.rand(K, 1, generator=g))     # the kernel normalises them
+    idx = torch.randperm(K, generator=g)[:M]
+    ide_mat, ide_m, _ = _ide_device_tables(dev)
+    X = mc_ops.hit_encode(inters.to(dev), dirs.to(dev), hit_normals.to(dev), idx.to(dev), ide_mat, ide_m, 128)
+
+    def ref(dt):
+        p, v, n = inters[idx].to(dt), -dirs[idx].to(dt), F.normalize(hit_normals[idx].to(dt), dim=-1)
+        r = 2.0 * (v * n).sum(-1, keepdim=True) * n - v
+        return posenc(p, 8), MC.ide_encode(r, 0)
+
+    pe64, ide64 = ref(torch.float64)
+    _, ide32 = ref(torch.float32)
+    assert rel_err(X[:, :51], pe64) < 1e-5
+    # the degree-16 entries lose ~5e-3 to cancellation in any fp32 evaluation, the fp32 oracle's included
+    assert rel_err(X[:, 51:123], ide64) < max(1e-5, 4 * rel_err(ide32, ide64))
+    assert float(X[:, 123:].abs().max()) == 0.0
+
+
 def _product_mc(g, dev):
     from tensoflow_b200.material import MCShadingNetwork
     cfg = dict(gridSize=[16, 16, 16], light_reso=16, mat_grid=24, device=dev)

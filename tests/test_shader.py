@@ -86,14 +86,15 @@ def test_cuda_shader_golden():
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("with_level", [False, True])
-def test_cube_lookup_kernel_matches_tensor_formulation(with_level):
-    """tf_cube_sample_fwd/bwd against cube_sample / cube_sample_mip (the tensor formulation pinned to the reference shader by the
-    golden test above) in fp64: values and the gradients wrt every texture level, the direction and the mip level."""
+def test_cube_lookup_kernel_matches_oracle_texture_cube(with_level):
+    """tf_cube_sample_fwd/bwd against the oracle's texture_cube / texture_cube_mip (the tensor formulation the oracle shader of
+    the golden test above runs on) in fp64: values and the gradients wrt every texture level, the direction and the mip level."""
     if not torch.cuda.is_available():
         pytest.skip("no CUDA device")
     import torch.nn.functional as F
     from conftest import rel_err
     from tensoflow_b200 import shape_shader as S
+    from oracle import torch_oracle_mat as OM
     dev = torch.device("cuda:0")
     g = torch.Generator().manual_seed(5)
     res = [32, 16, 8, 4] if with_level else [16]
@@ -113,7 +114,7 @@ def test_cube_lookup_kernel_matches_tensor_formulation(with_level):
         tx = [t.detach().clone().to(dt).requires_grad_() for t in texs]
         dd = d.detach().clone().to(dt).requires_grad_()
         lv = None if level is None else level.detach().clone().to(dt).requires_grad_()
-        out = S.cube_sample(tx[0], dd) if lv is None else S.cube_sample_mip(tx, dd, lv)
+        out = OM.texture_cube(tx[0], dd) if lv is None else OM.texture_cube_mip(tx, dd, lv)
         (out * u.to(dt)).sum().backward()
         return out, [t.grad for t in tx], dd.grad, None if lv is None else lv.grad
 
