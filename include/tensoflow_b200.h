@@ -204,8 +204,9 @@ TF_API int tf_pwquad_bwd(const float* y, const float* st, int64_t M, const float
 /* ---- triangle-mesh ray tracer ---------------------------------------------------------
  * Replaces the un-vendored `_raytracing` extension behind raytracing/raytracer.py:8-54
  * (`create_raytracer(vertices, triangles)` / `impl.trace(o, d, positions, normals, depth)`).
- * tf_bvh_create takes HOST arrays (like the reference, which builds from numpy) and uploads a
- * BVH to the current device; the handle owns that device memory until tf_bvh_destroy.
+ * tf_bvh_create takes HOST arrays (like the reference, which builds from numpy), builds the BVH on the
+ * host and uploads it to the current device; the handle owns that device memory until tf_bvh_destroy.
+ * It rejects an index out of range and a non-finite coordinate on a referenced vertex.
  * trace: closest hit with t > 0; writes position = o + t d, UNIT face normal (e1 x e2, the
  * reference renderer flips it: network/materialRenderer.py:256-257) and depth = t;
  * a miss writes depth = 10 (the sentinel of materialRenderer.py:261), normal = 0. */
@@ -215,6 +216,37 @@ TF_API int tf_bvh_create(const float* vertices_host, int64_t n_vertices, const i
 TF_API void tf_bvh_destroy(tf_bvh_t* handle);
 TF_API int tf_bvh_trace(const tf_bvh_t* handle, const float* rays_o, const float* rays_d, int64_t n,
                         float* positions, float* face_normals, float* depth, tf_stream_t stream);
+
+/* ---- BVH build on the device -----------------------------------------------------------
+ * The same tree as tf_bvh_create, node for node: nodes (32 B: bmin[3], first, bmax[3], count), triangles (48 B: v0, e1 = b - a,
+ * e2 = c - a, each padded with a 0) and perm [n_triangles] (caller index of each triangle slot) are byte-equal to the host
+ * build's.  The rule both follow: ranges split at lo + cnt/2 until cnt <= 4; the axis is that of the largest fp32 centroid
+ * extent, ties preferring x then y; the left half holds the cnt/2 smallest triangles by (centroid on that axis, caller index);
+ * centroids are ((a + b) + c) * (1/3) rounded per operation; -0 counts as +0; a leaf lists its triangles by caller index; the
+ * k-th inner node in right-first preorder has its children at 1 + 2k and 2 + 2k.
+ * tf_bvh_build_sizes: for 0 < n_triangles < 2^31, the node count of the tree and the bytes of scratch tf_bvh_build needs (this
+ *   includes the radix sort's temporary storage as CUB sizes it on the current device).
+ * tf_bvh_build: vertices [n_vertices,3] fp32 and triangles [n_triangles,3] int32 on the current device; every index must be in
+ *   [0, n_vertices) and every referenced coordinate finite (the kernels do not check: mc_ops.RayTracer validates with one host
+ *   read first).  workspace (>= the bytes above, 16-byte aligned) is caller-owned scratch; outputs nodes [n_nodes], tris
+ *   [n_triangles] (both 16-byte aligned) and perm [n_triangles].  Level by level: a segmented min / max, one kernel writing
+ *   64-bit keys, and one CUB radix sort, about ceil(log2(n / 4)) + 1 levels; everything on `stream`, no allocation, no host
+ *   synchronisation.  tf_launch_count counts the build's own kernels, not the sort's.
+ * tf_bvh_create_from_device: a handle from device nodes / tris / perm (layouts as above) on the current device.  It COPIES them
+ *   (cudaMemcpyAsync on `stream`) into memory the handle owns, so the sources may be released once those copies are ordered
+ *   before their reuse (the same stream); tf_bvh_destroy frees the handle's memory and never the sources.
+ * tf_bvh_export: the sizes of any handle (NULL to skip) and, for each non-NULL destination, a copy of its nodes [n_nodes]
+ *   (32 B each), tris [n_triangles] (48 B each) and perm [n_triangles] to host or device memory.  It synchronises the handle's
+ *   device first (so copies enqueued by tf_bvh_create_from_device on any stream are complete) and returns when the copies are.
+ * The first three return non-zero with tf_last_error() on a NULL pointer, an empty mesh or n_triangles >= 2^31;
+ * tf_bvh_export on a NULL handle or a failed copy. */
+TF_API int tf_bvh_build_sizes(int64_t n_triangles, int64_t* n_nodes, size_t* workspace_bytes);
+TF_API int tf_bvh_build(const float* vertices, int64_t n_vertices, const int32_t* triangles, int64_t n_triangles,
+                        void* workspace, size_t workspace_bytes, void* nodes, void* tris, int32_t* perm, tf_stream_t stream);
+TF_API int tf_bvh_create_from_device(const void* nodes, int64_t n_nodes, const void* tris, const int32_t* perm,
+                                     int64_t n_triangles, tf_stream_t stream, tf_bvh_t** out);
+TF_API int tf_bvh_export(const tf_bvh_t* handle, int64_t* n_nodes, int64_t* n_triangles, void* nodes, void* tris,
+                         int32_t* perm);
 
 /* ---- geometry evaluation (point-to-mesh distances, surface samples) ----------------------------
  * tf_bvh_closest_point: for each of the n query points [n,3], the nearest point of the mesh behind `handle`:

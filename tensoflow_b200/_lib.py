@@ -82,6 +82,10 @@ _SIGNATURES = {
     "tf_pwquad_bwd": (C.c_int, [_P, _P, C.c_int64, _P, _P, _P, _P, _P]),
     "tf_bvh_create": (C.c_int, [_P, C.c_int64, _P, C.c_int64, C.POINTER(C.c_void_p)]),
     "tf_bvh_destroy": (None, [_P]),
+    "tf_bvh_build_sizes": (C.c_int, [C.c_int64, C.POINTER(C.c_int64), C.POINTER(C.c_size_t)]),
+    "tf_bvh_build": (C.c_int, [_P, C.c_int64, _P, C.c_int64, _P, C.c_size_t, _P, _P, _P, _P]),
+    "tf_bvh_create_from_device": (C.c_int, [_P, C.c_int64, _P, _P, C.c_int64, _P, C.POINTER(C.c_void_p)]),
+    "tf_bvh_export": (C.c_int, [_P, C.POINTER(C.c_int64), C.POINTER(C.c_int64), _P, _P, _P]),
     "tf_bvh_trace": (C.c_int, [_P, _P, _P, C.c_int64, _P, _P, _P, _P]),
     "tf_bvh_closest_point": (C.c_int, [_P, _P, C.c_int64, _P, _P, _P, _P]),
     "tf_mesh_sample_surface": (C.c_int, [_P, _P, C.c_int64, _P, _P, C.c_int64, _P, _P, _P, _P]),

@@ -23,6 +23,11 @@ struct tf_bvh {
     int device;
 };
 
+// BVH build rule shared by the host build (bvh.cu) and the device build (bvh_build.cu): ranges split at lo + cnt/2 until
+// cnt <= TF_BVH_LEAF; values are compared and reduced with -0 mapped to +0.
+constexpr int TF_BVH_LEAF = 4;
+__host__ __device__ __forceinline__ float bvh_canon_zero(float x) { return x == 0.f ? 0.f : x; }
+
 struct BvhView {
     const BvhNode* nodes;
     const BvhTri* tris;

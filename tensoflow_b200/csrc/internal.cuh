@@ -59,3 +59,9 @@ int tf_internal_flow_block_bwd_tc(const float* y_in, const float* feat, int feat
                                   const float* W4, float scale, float offset, int cond, int64_t M, const float* saved_h, const float* saved_st,
                                   const float* g_y_out, const float* g_logj, float* g_y_in, float* d_feat, float* dW1, float* db1, float* dW2,
                                   float* db2, float* dW3, float* db3, float* dW4, float* db4, cudaStream_t stream);
+
+// ---- bvh.cu: BVH handles ----
+struct tf_bvh;
+// a handle with room for n_nodes nodes and n_tris triangles (perm included) on the current device; NULL after
+// tf_set_error("<who>: ...") when an allocation fails
+tf_bvh* tf_internal_bvh_alloc(int64_t n_nodes, int64_t n_tris, const char* who);

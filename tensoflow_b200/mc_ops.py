@@ -3,6 +3,7 @@ lookup and the BRDF / Monte-Carlo estimator (reference network/fields.py:824-133
 network/light.py:125-162, raytracing/raytracer.py)."""
 from __future__ import annotations
 
+import contextlib
 import ctypes as C
 
 import numpy as np
@@ -13,11 +14,25 @@ from ._lib import check, ptr, stream_ptr
 from .ops import _f32c, _timed
 
 
+class _TooFewTriangles(RuntimeError, AssertionError):
+    """A mesh of at most 8 triangles: a RuntimeError like every other refusal of the device build, and still the
+    AssertionError the host build raises for it."""
+
+
 class RayTracer:
     """Drop-in for the reference's raytracing.RayTracer (raytracing/raytracer.py:8-54):
-    RayTracer(vertices, triangles).trace(rays_o, rays_d) -> positions, face_normals, depth."""
+    RayTracer(vertices, triangles).trace(rays_o, rays_d) -> positions, face_normals, depth.
+
+    CUDA tensors (both on one device) are built into a BVH on that device (tf_bvh_build, no host copy); numpy arrays and CPU
+    tensors by the host build (tf_bvh_create).  Both builds give the same BVH node for node, so trace and closest_point return
+    the same bits either way.  A mesh of at most 8 triangles raises _TooFewTriangles on the device path: a RuntimeError like the
+    device path's other refusals, and also the AssertionError that callers of the host path (and of the reference) catch."""
 
     def __init__(self, vertices, triangles):
+        self._device = None
+        if torch.is_tensor(vertices) and torch.is_tensor(triangles) and vertices.is_cuda and vertices.device == triangles.device:
+            self._build_on_device(vertices.detach(), triangles.detach())
+            return
         if torch.is_tensor(vertices):
             vertices = vertices.detach().cpu().numpy()
         if torch.is_tensor(triangles):
@@ -30,6 +45,36 @@ class RayTracer:
         check(lib.tf_bvh_create(v.ctypes.data_as(C.c_void_p), v.shape[0], t.ctypes.data_as(C.c_void_p), t.shape[0],
                                 C.byref(self._h)), "tf_bvh_create")
         self.n_triangles = int(t.shape[0])
+
+    def _build_on_device(self, vertices, triangles):
+        """tf_bvh_build on the tensors' device after the checks below, which read back one small tensor and raise before any
+        launch of the library."""
+        self._h = None
+        nt, nv = validate_device_mesh(vertices, triangles)
+        dev = vertices.device
+        with torch.cuda.device(dev):
+            v = _f32c(vertices)
+            t = triangles.to(torch.int32).contiguous()
+            lib = _lib.load()
+            n_nodes, ws_bytes = C.c_int64(), C.c_size_t()
+            check(lib.tf_bvh_build_sizes(nt, C.byref(n_nodes), C.byref(ws_bytes)), "tf_bvh_build_sizes")
+            ws = torch.empty(ws_bytes.value, device=dev, dtype=torch.uint8)
+            nodes = torch.empty(n_nodes.value, 8, device=dev, dtype=torch.float32)
+            tris = torch.empty(nt, 12, device=dev, dtype=torch.float32)
+            perm = torch.empty(nt, device=dev, dtype=torch.int32)
+            s = stream_ptr()
+            with _timed("bvh_build"):
+                check(lib.tf_bvh_build(ptr(v), nv, ptr(t), nt, ptr(ws), ws_bytes.value, ptr(nodes), ptr(tris), ptr(perm), s),
+                      "tf_bvh_build")
+            h = C.c_void_p()
+            check(lib.tf_bvh_create_from_device(ptr(nodes), n_nodes.value, ptr(tris), ptr(perm), nt, s, C.byref(h)),
+                  "tf_bvh_create_from_device")
+        self._h = h
+        self._device = dev
+        self.n_triangles = nt
+
+    def _on_device(self):
+        return torch.cuda.device(self._device) if self._device is not None else contextlib.nullcontext()
 
     def __del__(self):
         try:
@@ -48,7 +93,7 @@ class RayTracer:
         positions = torch.empty_like(o)
         normals = torch.empty_like(d)
         depth = torch.empty(n, device=o.device, dtype=torch.float32)
-        with _timed("bvh_trace"):
+        with self._on_device(), _timed("bvh_trace"):
             check(_lib.load().tf_bvh_trace(self._h, ptr(o), ptr(d), n, ptr(positions), ptr(normals), ptr(depth), stream_ptr()),
                   "tf_bvh_trace")
         return positions.reshape(*prefix, 3), normals.reshape(*prefix, 3), depth.reshape(*prefix)
@@ -68,10 +113,41 @@ class RayTracer:
         closest = torch.empty_like(q)
         dist = torch.empty(n, device=q.device, dtype=torch.float32)
         tri = torch.empty(n, device=q.device, dtype=torch.int64)
-        with _timed("bvh_closest_point"):
+        with self._on_device(), _timed("bvh_closest_point"):
             check(_lib.load().tf_bvh_closest_point(self._h, ptr(q), n, ptr(closest), ptr(dist), ptr(tri), stream_ptr()),
                   "tf_bvh_closest_point")
         return closest.reshape(*prefix, 3), dist.reshape(prefix), tri.reshape(prefix)
+
+
+def validate_device_mesh(vertices, triangles):
+    """The checks RayTracer makes before building on the device: vertices [V,3] floating point, triangles [T,3] integer,
+    8 < T < 2^31, every index in [0, min(V, 2^31)) and every coordinate of a referenced vertex finite once rounded to fp32 (the
+    build's precision, so a float64 coordinate beyond the fp32 range is refused as the host build refuses it).  Reads one small tensor
+    back to the host and launches nothing of the library.  Returns (T, V); raises RuntimeError."""
+    if vertices.ndim != 2 or vertices.shape[1] != 3 or triangles.ndim != 2 or triangles.shape[1] != 3:
+        raise RuntimeError(f"RayTracer needs vertices [V, 3] and triangles [T, 3], got {list(vertices.shape)} and "
+                           f"{list(triangles.shape)}")
+    if not vertices.is_floating_point() or triangles.is_floating_point() or triangles.dtype in (torch.bool, torch.uint8):
+        raise RuntimeError(f"RayTracer needs floating-point vertices and int32 / int64 triangles, got {vertices.dtype} and "
+                           f"{triangles.dtype}")
+    nt, nv = int(triangles.shape[0]), int(vertices.shape[0])
+    if nt == 0 or nv == 0:
+        raise RuntimeError("RayTracer: empty mesh")
+    if nt <= 8:
+        raise _TooFewTriangles("BVH needs at least 8 triangles.")
+    if nt >= 1 << 31:
+        raise RuntimeError(f"RayTracer: {nt} triangles, the BVH holds fewer than 2^31")
+    flat = triangles.reshape(-1)
+    bad_vertex = ~torch.isfinite(vertices.to(torch.float32)).all(1)
+    idx = flat.clamp(0, nv - 1)
+    referenced = torch.index_select(bad_vertex, 0, idx if idx.dtype in (torch.int32, torch.int64) else idx.long())
+    tmin, tmax, n_bad = torch.stack([flat.min().to(torch.int64), flat.max().to(torch.int64),
+                                     referenced.sum().to(torch.int64)]).tolist()
+    if tmin < 0 or tmax >= min(nv, 1 << 31):
+        raise RuntimeError(f"RayTracer: triangle index out of range (indices span [{tmin}, {tmax}], {nv} vertices)")
+    if n_bad:
+        raise RuntimeError("RayTracer: non-finite vertex coordinate on a referenced vertex")
+    return nt, nv
 
 
 def mc_directions(mode: int, normals, view_dirs, src, aux, roughness, n_dirs: int, dirs_out, prob_out, offset: int):
