@@ -267,6 +267,19 @@ TF_API int tf_mesh_sample_surface(const float* vertices, const int32_t* triangle
                                   const double* uniforms, int64_t n, float* out_points, int64_t* out_tri, float* out_normals,
                                   tf_stream_t stream);
 
+/* ---- mesh clean-up: connected components ------------------------------------------------------------
+ * tf_mesh_components: connected components of the graph whose nodes are the n_vertices vertices and whose edges are the
+ *   edges of the n_tris triangles [n_tris,3] int32 (every index in [0, n_vertices): precondition, checked by the caller;
+ *   geometry.mesh_components does it with one host read).
+ *   root[v]      = the smallest vertex index in v's component (a vertex no triangle references is its own component);
+ *   tri_count[r] = the number of triangles whose vertices have root r (zero for every non-root v).
+ *   root and tri_count are [n_vertices] int32 outputs; tri_count is zeroed by the call.  0 < n_vertices < 2^31,
+ *   0 <= n_tris < 2^31.  Lock-free union-find (ECL-CC: hooks by atomicCAS of the larger root under the smaller, path halving),
+ *   then a flatten pass and integer atomics for the counts.  No workspace, no host synchronisation; the result does not
+ *   depend on scheduling.  Returns non-zero with tf_last_error() on a NULL pointer or a count out of range, before any launch. */
+TF_API int tf_mesh_components(const int32_t* triangles, int64_t n_tris, int64_t n_vertices, int32_t* root, int32_t* tri_count,
+                              tf_stream_t stream);
+
 /* ---- material-stage Monte-Carlo integral (network/fields.py:1075-1335) -----------------
  * tf_mc_directions builds one direction set per surface point and its pdf:
  *   mode 0: flow samples in the half-vector parametrisation (fields.py:1085-1108,1164-1188)

@@ -62,6 +62,59 @@ def sample_surface(vertices, triangles, n: int, seed: int = 0):
         return _sample_surface_from(v, t, cdf, uniforms)
 
 
+def _components(vertices, triangles, what):
+    """Checks, then tf_mesh_components -> (triangles [T,3] int32, root [V] int32, tri_count [V] int32) on the mesh's device.
+    Every refusal comes before any launch; the index range costs one host read."""
+    if torch.is_tensor(triangles) and (triangles.is_floating_point() or triangles.is_complex() or triangles.dtype == torch.bool):
+        raise RuntimeError(f"{what} needs integer triangles, got {triangles.dtype}")
+    if torch.is_tensor(vertices) and vertices.dim() == 2 and vertices.shape[0] >= 2 ** 31:
+        raise RuntimeError(f"{what}: {vertices.shape[0]} vertices, the kernel indexes fewer than 2^31")
+    v, t = _mesh(vertices, triangles, what)
+    V = v.shape[0]
+    with torch.cuda.device(v.device):
+        flat = triangles.detach().reshape(-1)
+        lo, hi = torch.stack([flat.min(), flat.max()]).to(torch.int64).tolist()           # the one host read
+        if lo < 0 or hi >= V:
+            raise RuntimeError(f"{what}: triangle index out of range (indices span [{lo}, {hi}], {V} vertices)")
+        root = torch.empty(V, device=v.device, dtype=torch.int32)
+        tri_count = torch.empty(V, device=v.device, dtype=torch.int32)
+        check(_lib.load().tf_mesh_components(ptr(t), t.shape[0], V, ptr(root), ptr(tri_count), stream_ptr()), "tf_mesh_components")
+    return t, root, tri_count
+
+
+def mesh_components(vertices, triangles):
+    """Connected components of a mesh (vertices joined by triangle edges) -> (root [V] int32, tri_count [V] int32) on the mesh's
+    device: root[v] is the smallest vertex index of v's component (a vertex no triangle references is a component of its own),
+    tri_count[r] the number of triangles of the component whose root is r, 0 for every vertex that is not a root.  Lock-free
+    union-find on the GPU (tf_mesh_components); the result does not depend on scheduling.  Raises RuntimeError, before any
+    launch, on CPU tensors, shapes other than [V,3] / [T,3], an empty mesh, non-integer triangles, 2^31 or more vertices, or a
+    triangle index out of range (one host read)."""
+    _, root, tri_count = _components(vertices, triangles, "mesh_components")
+    return root, tri_count
+
+
+def remove_small_components(vertices, triangles, min_fraction: float):
+    """Drop the small connected components of a mesh ("floaters") -> (vertices [V',3], triangles [T',3] int32) on its device.
+    A triangle is kept iff its component has tri_count >= min_fraction * (the largest component's tri_count), compared in
+    fp64; min_fraction = 1.0 keeps the largest component and every component tied with it.  Kept triangles keep their order,
+    the vertices they reference keep theirs (and their dtype), and the indices are renumbered.  Vertices that no triangle
+    references are dropped.  Raises ValueError for min_fraction outside (0, 1], and what mesh_components raises, before any
+    launch.  Two host reads: the index range before the union-find, the output sizes after it."""
+    f = float(min_fraction)
+    if not 0.0 < f <= 1.0:
+        raise ValueError(f"remove_small_components: min_fraction must lie in (0, 1], got {min_fraction}")
+    t, root, tri_count = _components(vertices, triangles, "remove_small_components")
+    with torch.cuda.device(t.device):
+        # an unreferenced vertex has tri_count 0 < f * max, so it goes; a component's vertices and triangles go together
+        keep_v = tri_count[root.long()].double() >= f * tri_count.max().double()
+        keep_t = keep_v[t[:, 0].long()]
+        new_index = torch.cumsum(keep_v, 0, dtype=torch.int32) - 1
+        n_v, n_t = torch.stack([keep_v.sum(), keep_t.sum()]).tolist()                      # the second host read
+        vi = torch.nonzero_static(keep_v, size=n_v).reshape(-1)
+        ti = torch.nonzero_static(keep_t, size=n_t).reshape(-1)
+        return vertices.detach()[vi], new_index[t[ti].long()]
+
+
 def evaluate_mesh(pred_vertices, pred_triangles, gt_vertices, gt_triangles, n_samples: int = 1_000_000,
                   thresholds=(0.005, 0.01, 0.02), seed: int = 0) -> dict:
     """Distance of a predicted mesh to a ground-truth mesh, from `n_samples` area-weighted samples of each (seeds `seed` for the

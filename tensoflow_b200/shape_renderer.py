@@ -531,14 +531,21 @@ class ShapeRenderer(torch.nn.Module):
         return u
 
     @torch.no_grad()
-    def extract_geometry(self, bound_min, bound_max, resolution: int, threshold: float = 0.0):
+    def extract_geometry(self, bound_min, bound_max, resolution: int, threshold: float = 0.0,
+                         min_component_fraction: float | None = None):
         """Zero level set of the SDF as a triangle mesh -> (vertices [V,3] world fp32, triangles [T,3] int32) on the device,
         winding out of the object, vertices rescaled as v / (R - 1) * (bound_max - bound_min) + bound_min.
         `MaterialRenderer(cfg, *shape.extract_geometry(...))` takes it.  Below 2^31 lattice points (R <= 1290): marching
         cubes (tensoflow_b200.isosurface) on extract_fields.  From there up to R = 4096, where the dense volume no longer fits
         the kernels' indices: the narrow band (marching_cubes_narrowband) on the same lattice values, which evaluates the
-        field only in bricks around the surface and gives the dense mesh wherever its band rule captures the surface."""
+        field only in bricks around the surface and gives the dense mesh wherever its band rule captures the surface.
+        min_component_fraction (None: every component) drops the small disconnected components ("floaters") with
+        geometry.remove_small_components: a component is kept iff it has at least that fraction of the triangles of the
+        largest one (1.0 keeps the largest); it must lie in (0, 1].  An empty mesh is returned as it is."""
+        from .geometry import remove_small_components
         from .isosurface import marching_cubes, marching_cubes_narrowband
+        if min_component_fraction is not None and not 0.0 < float(min_component_fraction) <= 1.0:
+            raise ValueError(f"extract_geometry: min_component_fraction must lie in (0, 1], got {min_component_fraction}")
         R = int(resolution)
         if R ** 3 < 2 ** 31:
             verts, tris = marching_cubes(self.extract_fields(bound_min, bound_max, R), threshold)
@@ -548,7 +555,10 @@ class ShapeRenderer(torch.nn.Module):
             verts, tris = marching_cubes_narrowband(self._extract_values, self._extract_axes(bound_min, bound_max, R), threshold)
         lo = torch.as_tensor(bound_min, dtype=torch.float32).reshape(1, 3).to(verts.device)
         hi = torch.as_tensor(bound_max, dtype=torch.float32).reshape(1, 3).to(verts.device)
-        return verts / (R - 1.0) * (hi - lo) + lo, tris
+        verts = verts / (R - 1.0) * (hi - lo) + lo
+        if min_component_fraction is not None and tris.shape[0] > 0:
+            verts, tris = remove_small_components(verts, tris, min_component_fraction)
+        return verts, tris
 
     # ---- alpha mask (reference shapeRenderer.py:257-325) --------------------------------------------
     @torch.no_grad()
