@@ -280,6 +280,44 @@ TF_API int tf_mesh_sample_surface(const float* vertices, const int32_t* triangle
 TF_API int tf_mesh_components(const int32_t* triangles, int64_t n_tris, int64_t n_vertices, int32_t* root, int32_t* tri_count,
                               tf_stream_t stream);
 
+/* ---- mesh simplification: quadric-error edge collapse in rounds -------------------------------------------
+ * Garland-Heckbert edge collapse, run in rounds of collapses whose closed 1-rings are vertex-disjoint.  The result is
+ * deterministic and bit-equal to oracle/torch_oracle_simplify.py, which restates every rule below in numpy.
+ *   quadrics   fp64, per vertex the sum of the unit-normal plane quadrics p p^T of its faces (no area weight, so sqrt(cost) is a
+ *              length), summed in face order; a face of zero-length cross product (b - a) x (c - a) adds nothing.  A collapse
+ *              gives the survivor Q_a + Q_b.  fp64 operations are rounded one by one (no FMA contraction).
+ *   placement  v minimises v^T Q v: with A the 3x3 block of Q, v = -A^-1 (Q_xd, Q_yd, Q_zd) from the adjugate when det(A) >
+ *              1e-6 trace(A)^3, else the cheapest of a, b and their midpoint (ties in that order).  v is rounded to fp32 and the
+ *              cost max(0, v^T Q v) is taken there; positions are fp32 throughout.  The survivor is the smaller index a.
+ *   validity   an edge {a, b} may collapse iff it has exactly two faces, with different apexes c0, c1; neither a nor b is locked
+ *              (a vertex is locked when an edge with a face count other than 2 ends there, or a face with a repeated index
+ *              holds it: open boundaries and non-manifold vertices stay bit-identical); c0 and c1 each have more than 3 faces;
+ *              a and b have no common neighbour but c0 and c1 (link condition); every other face of the two stars whose old
+ *              normal is not zero keeps a new normal at a positive dot product with it (no fold-over, no new degenerate face);
+ *              and sqrt(cost) <= max_error.
+ *   selection  valid edges are ranked by (fp32 cost, a, b); the first k = min(max(1, n_valid / 16), (T - target) / 2) are
+ *              candidates.  Candidate i has priority (splitmix64(a << 32 | b) >> 32) << 32 | i and wins iff it holds the minimum
+ *              priority claimed by every vertex of its closed 1-ring (the vertices of the faces of a and of b).  Priorities are
+ *              hashed, not costs: smooth costs have few local minima, so cost priorities would let a handful of edges win.
+ *   stopping   when T <= target + 1 or a round collapses nothing.  Each collapse removes two faces, so T' >= target.
+ *   output     surviving faces keep their relative order, referenced vertices keep theirs, indices are renumbered; with no
+ *              collapse and every vertex referenced the output equals the input byte for byte.
+ * tf_mesh_simplify_sizes: the bytes of scratch tf_mesh_simplify needs for n_vertices and n_triangles (including CUB's temporary
+ *   storage as sized on the current device), about 310 bytes per triangle.
+ * tf_mesh_simplify: vertices [n_vertices,3] fp32 and triangles [n_triangles,3] int32 on the current device (every index in
+ *   [0, n_vertices): precondition, geometry.simplify_mesh checks it with one host read), target >= 0 triangles, max_error >= 0
+ *   (+inf for no bound).  Writes out_vertices [V',3] and out_triangles [T',3] (buffers of the input sizes) and V', T' and the
+ *   number of rounds that collapsed something to the host pointers.  It runs every round on `stream` and, at the end of each
+ *   round, reads one count (the surviving faces) to the host with cudaMemcpyAsync and a stream synchronise; it returns after a
+ *   last such read of V'.  Each round re-sorts the (vertex, face) pairs and the half-edges with CUB radix sorts.
+ * Both return non-zero with tf_last_error() before any launch on a NULL pointer, 0 or >= 2^31 vertices, 0 or >= 2^31 triangles
+ * or 3 n_triangles >= 2^31 (the half-edge sorts count in int; at about 310 B of workspace per triangle no device holds that
+ * many), target < 0, max_error negative or NaN, or a workspace smaller than the sizes call gives. */
+TF_API int tf_mesh_simplify_sizes(int64_t n_vertices, int64_t n_triangles, size_t* workspace_bytes);
+TF_API int tf_mesh_simplify(const float* vertices, int64_t n_vertices, const int32_t* triangles, int64_t n_triangles, int64_t target,
+                            double max_error, void* workspace, size_t workspace_bytes, float* out_vertices, int32_t* out_triangles,
+                            int64_t* out_n_vertices, int64_t* out_n_triangles, int32_t* out_rounds, tf_stream_t stream);
+
 /* ---- material-stage Monte-Carlo integral (network/fields.py:1075-1335) -----------------
  * tf_mc_directions builds one direction set per surface point and its pdf:
  *   mode 0: flow samples in the half-vector parametrisation (fields.py:1085-1108,1164-1188)

@@ -90,6 +90,9 @@ _SIGNATURES = {
     "tf_bvh_closest_point": (C.c_int, [_P, _P, C.c_int64, _P, _P, _P, _P]),
     "tf_mesh_sample_surface": (C.c_int, [_P, _P, C.c_int64, _P, _P, C.c_int64, _P, _P, _P, _P]),
     "tf_mesh_components": (C.c_int, [_P, C.c_int64, C.c_int64, _P, _P, _P]),
+    "tf_mesh_simplify_sizes": (C.c_int, [C.c_int64, C.c_int64, C.POINTER(C.c_size_t)]),
+    "tf_mesh_simplify": (C.c_int, [_P, C.c_int64, _P, C.c_int64, C.c_int64, C.c_double, _P, C.c_size_t, _P, _P,
+                                   C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.POINTER(C.c_int32), _P]),
     "tf_mc_directions": (C.c_int, [C.c_int32, _P, _P, _P, _P, _P, C.c_int64, C.c_int32, _P, _P, C.c_int32, C.c_int32, _P]),
     "tf_cube_light_fwd": (C.c_int, [_P, C.c_int32, _P, _P, C.c_int64, _P, _P]),
     "tf_cube_light_bwd": (C.c_int, [C.c_int32, _P, _P, C.c_int64, _P, _P, _P, _P]),

@@ -1,7 +1,9 @@
-"""Geometry evaluation of a mesh against a reference mesh on the GPU: area-weighted surface samples (`tf_mesh_sample_surface`)
-and exact point-to-mesh distances on the BVH (`tf_bvh_closest_point`, through mc_ops.RayTracer), reduced in fp64.  There is
-no CPU path."""
+"""Mesh geometry on the GPU: evaluation against a reference mesh (area-weighted surface samples, `tf_mesh_sample_surface`, and
+exact point-to-mesh distances on the BVH, `tf_bvh_closest_point` through mc_ops.RayTracer, reduced in fp64), connected
+components (`tf_mesh_components`) and quadric-error simplification (`tf_mesh_simplify`).  There is no CPU path."""
 from __future__ import annotations
+
+import ctypes
 
 import torch
 
@@ -113,6 +115,58 @@ def remove_small_components(vertices, triangles, min_fraction: float):
         vi = torch.nonzero_static(keep_v, size=n_v).reshape(-1)
         ti = torch.nonzero_static(keep_t, size=n_t).reshape(-1)
         return vertices.detach()[vi], new_index[t[ti].long()]
+
+
+def _simplify_limits(target_triangles, max_error, what):
+    """-> (target int, max_error float, +inf for None); ValueError on a negative target or a negative / non-finite bound"""
+    if isinstance(target_triangles, bool) or int(target_triangles) != target_triangles or int(target_triangles) < 0:
+        raise ValueError(f"{what}: target_triangles must be an integer >= 0, got {target_triangles}")
+    err = float("inf") if max_error is None else float(max_error)
+    if max_error is not None and not (0.0 <= err < float("inf")):
+        raise ValueError(f"{what}: max_error must be finite and >= 0 (None for no bound), got {max_error}")
+    return int(target_triangles), err
+
+
+def simplify_mesh(vertices, triangles, target_triangles: int, max_error: float | None = None):
+    """Quadric-error edge collapse on the GPU (tf_mesh_simplify) -> (vertices [V',3] fp32, triangles [T',3] int32) on the mesh's
+    device.  Collapses run in rounds of edges with vertex-disjoint closed 1-rings until T' <= target_triangles + 1 or no edge
+    may collapse; T' is never below the target.  max_error (None: no bound) bounds sqrt of each collapse's quadric cost, which
+    bounds the distance of the new vertex to the plane of every input face merged into it.  Open boundaries and non-manifold
+    vertices are kept bit for bit, surviving triangles keep their order, and the referenced vertices keep theirs.  The result
+    is deterministic (bit-equal to oracle/torch_oracle_simplify.py).  Raises ValueError on a negative target or a negative or
+    non-finite max_error, and RuntimeError on CPU tensors, shapes other than [V,3] / [T,3], an empty mesh, non-integer
+    triangles, 2^31 or more vertices or triangles, or a triangle index out of range (one host read), all before any launch.
+    The rounds read one count each to the host."""
+    return _simplify(vertices, triangles, target_triangles, max_error)[:2]
+
+
+def _simplify(vertices, triangles, target_triangles, max_error):
+    """simplify_mesh -> (vertices, triangles, the number of rounds that collapsed something)"""
+    what = "simplify_mesh"
+    target, max_error = _simplify_limits(target_triangles, max_error, what)
+    if torch.is_tensor(triangles) and (triangles.is_floating_point() or triangles.is_complex() or triangles.dtype == torch.bool):
+        raise RuntimeError(f"{what} needs integer triangles, got {triangles.dtype}")
+    for x, name in ((vertices, "vertices"), (triangles, "triangles")):
+        if torch.is_tensor(x) and x.dim() == 2 and x.shape[0] >= 2 ** 31:
+            raise RuntimeError(f"{what}: {x.shape[0]} {name}, the kernel indexes fewer than 2^31")
+    v, t = _mesh(vertices, triangles, what)
+    V, T = v.shape[0], t.shape[0]
+    lib = _lib.load()
+    with torch.cuda.device(v.device):
+        flat = triangles.detach().reshape(-1)
+        lo, hi = torch.stack([flat.min(), flat.max()]).to(torch.int64).tolist()           # the one host read before the rounds
+        if lo < 0 or hi >= V:
+            raise RuntimeError(f"{what}: triangle index out of range (indices span [{lo}, {hi}], {V} vertices)")
+        ws_bytes = ctypes.c_size_t()
+        check(lib.tf_mesh_simplify_sizes(V, T, ctypes.byref(ws_bytes)), "tf_mesh_simplify_sizes")
+        ws = torch.empty(ws_bytes.value, device=v.device, dtype=torch.uint8)
+        out_v = torch.empty(V, 3, device=v.device, dtype=torch.float32)
+        out_t = torch.empty(T, 3, device=v.device, dtype=torch.int32)
+        n_v, n_t, rounds = ctypes.c_int64(), ctypes.c_int64(), ctypes.c_int32()
+        check(lib.tf_mesh_simplify(ptr(v), V, ptr(t), T, target, max_error, ptr(ws), ws_bytes.value, ptr(out_v), ptr(out_t),
+                                   ctypes.byref(n_v), ctypes.byref(n_t), ctypes.byref(rounds), stream_ptr()), "tf_mesh_simplify")
+        del ws
+        return out_v[:n_v.value].clone(), out_t[:n_t.value].clone(), rounds.value
 
 
 def evaluate_mesh(pred_vertices, pred_triangles, gt_vertices, gt_triangles, n_samples: int = 1_000_000,

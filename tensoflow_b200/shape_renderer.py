@@ -532,7 +532,8 @@ class ShapeRenderer(torch.nn.Module):
 
     @torch.no_grad()
     def extract_geometry(self, bound_min, bound_max, resolution: int, threshold: float = 0.0,
-                         min_component_fraction: float | None = None):
+                         min_component_fraction: float | None = None, target_triangles: int | None = None,
+                         max_error: float | None = None):
         """Zero level set of the SDF as a triangle mesh -> (vertices [V,3] world fp32, triangles [T,3] int32) on the device,
         winding out of the object, vertices rescaled as v / (R - 1) * (bound_max - bound_min) + bound_min.
         `MaterialRenderer(cfg, *shape.extract_geometry(...))` takes it.  Below 2^31 lattice points (R <= 1290): marching
@@ -541,11 +542,17 @@ class ShapeRenderer(torch.nn.Module):
         field only in bricks around the surface and gives the dense mesh wherever its band rule captures the surface.
         min_component_fraction (None: every component) drops the small disconnected components ("floaters") with
         geometry.remove_small_components: a component is kept iff it has at least that fraction of the triangles of the
-        largest one (1.0 keeps the largest); it must lie in (0, 1].  An empty mesh is returned as it is."""
-        from .geometry import remove_small_components
+        largest one (1.0 keeps the largest); it must lie in (0, 1].  When target_triangles or max_error is given, the mesh is
+        then simplified with geometry.simplify_mesh (quadric-error edge collapse down to target_triangles, 0 when None, with
+        each collapse's error at most max_error in world units, no bound when None); this runs after the floater removal, so
+        floaters spend none of the budget.  An empty mesh is returned as it is."""
+        from .geometry import _simplify_limits, remove_small_components, simplify_mesh
         from .isosurface import marching_cubes, marching_cubes_narrowband
         if min_component_fraction is not None and not 0.0 < float(min_component_fraction) <= 1.0:
             raise ValueError(f"extract_geometry: min_component_fraction must lie in (0, 1], got {min_component_fraction}")
+        simplify = target_triangles is not None or max_error is not None
+        if simplify:
+            _simplify_limits(0 if target_triangles is None else target_triangles, max_error, "extract_geometry")
         R = int(resolution)
         if R ** 3 < 2 ** 31:
             verts, tris = marching_cubes(self.extract_fields(bound_min, bound_max, R), threshold)
@@ -558,6 +565,8 @@ class ShapeRenderer(torch.nn.Module):
         verts = verts / (R - 1.0) * (hi - lo) + lo
         if min_component_fraction is not None and tris.shape[0] > 0:
             verts, tris = remove_small_components(verts, tris, min_component_fraction)
+        if simplify and tris.shape[0] > 0:
+            verts, tris = simplify_mesh(verts, tris, 0 if target_triangles is None else target_triangles, max_error)
         return verts, tris
 
     # ---- alpha mask (reference shapeRenderer.py:257-325) --------------------------------------------
