@@ -318,6 +318,61 @@ TF_API int tf_mesh_simplify(const float* vertices, int64_t n_vertices, const int
                             double max_error, void* workspace, size_t workspace_bytes, float* out_vertices, int32_t* out_triangles,
                             int64_t* out_n_vertices, int64_t* out_n_triangles, int32_t* out_rounds, tf_stream_t stream);
 
+/* ---- UV atlas of box-projection charts and texture baking -------------------------------------------------
+ * Deterministic and bit-equal to oracle/torch_oracle_atlas.py, which restates every rule below in numpy.  fp64 operations are
+ * rounded one by one (no FMA contraction) and summed in a fixed order; the only atomics are integer ones.
+ *   classes    n = (b - a) x (c - a) in fp64, len = |n|.  Class 2k + (n_k < 0), k the axis of the largest |n_k| (ties to the lower
+ *              axis).  Class c (axis c / 2, + for even c) is allowed iff +-n_k >= len / 2, i.e. |n^ . axis| >= 1/2 on the front
+ *              side.  4 Jacobi passes: per class, len of the face and of its edge neighbours (for each of its edges k = 0, 1, 2,
+ *              the other faces of that edge, ascending) summed in that order; the face takes the allowed class of the largest
+ *              sum, its own on ties, then the lower class.
+ *   charts     faces sharing an edge (two vertex indices) and a class, neither marked solo, are joined (union-find over faces as
+ *              in tf_mesh_components); a chart's root is its smallest face and charts are numbered by root.
+ *   projection chart axis k: (u, w) = (p[(k+1)%3], p[(k+2)%3]) for +k, swapped for -k (front faces stay counter-clockwise);
+ *              one density s (texels per world unit) for all charts.
+ *   packing    rect = max(1, ceil(extent * s)) + 2 padding per axis; rects sorted by (h desc, w desc, chart asc), next-fit
+ *              decreasing height into shelves of width R.  s0 = R / sqrt(projected area), the area summed in fixed point
+ *              (rint(|n_k| / max |n_k| * 2^32) in uint64); s = s0 if it fits, else the lo of 20 bisection steps on (0, s0].
+ *   texels     corner x = fp32((x0 + padding) + (u - umin) s), y likewise, in [0, R]; uv = (x / R, y / R) and texture row j spans
+ *              v in [j/R, (j+1)/R] (image writers with row 0 at the top flip v).  Texel (i, j) is covered when its centre
+ *              (i + 1/2, j + 1/2) is inside the triangle: fp64 edge functions taken from the endpoint smaller in (x, y) order
+ *              (so both faces of an edge see one value), > 0 or = 0 on a top-left edge; a face of negative signed area is taken
+ *              reversed, one of zero covers nothing.  Coverage runs over 8x8 tiles of each face's box (a prefix sum of tile
+ *              counts, one thread per tile), so a few huge faces do not stall.
+ *   conflicts  every face covering a centre that another face covers is marked solo (a chart of its own) and charts, density,
+ *              packing and coverage run again, until no centre is covered twice (single triangles never overlap, and rects are
+ *              disjoint).  A chart covering no centre gets the texel under its root face's texel centroid, clamped into its rect.
+ *   output     vertices are the unique (source vertex, chart) pairs in (vertex, chart) order (split along seams); triangles
+ *              keep their order.
+ * tf_uv_atlas_sizes: the scratch bytes of tf_uv_atlas (CUB temporary storage sized on the current device), about 250 B per
+ *   triangle.
+ * tf_uv_atlas: vertices [n_vertices,3] fp32, triangles [n_triangles,3] int32 (indices in range: precondition, geometry.uv_atlas
+ *   checks it), 16 <= resolution R <= 16384, 1 <= padding <= 16.  Writes out_chart [T] int32, out_triangles [T,3] int32 (output
+ *   vertex ids), out_vertex_index [V'] int64 and out_xy [V',2] fp32 (buffers of 3T rows), out_texel_tri [R,R] int32 (owner
+ *   face, -1 for none), out_rects [C,4] int32 (x0, y0, w, h; buffer of T rows), and to host pointers s, V', C, the conflict
+ *   rounds and the density trials.  Host reads: the chart count once, one (conflicts, next chart count) read per round and
+ *   V' at the end; the density search keeps its state on the device.  Returns 3 with tf_last_error() when the charts do not
+ *   fit at any density tried.
+ * tf_uv_texel_points: for n texels (j R + i) owned in texel_tri, the point at the barycentrics of the centre in the owner of
+ *   triangles [T,3] over vertices [V',3] and xy [V',2] (fp64, clamped at 0 and renormalised; the centroid for a zero-area
+ *   face), rounded once to fp32 -> out_points [n,3].
+ * tf_uv_fill_sizes / tf_uv_fill: values [n,channels] fp32 scattered to their texels of texture [R,R,channels] (zeroed), then
+ *   `padding` dilation passes: an empty texel inside the rect of a filled 8-neighbour's chart takes the fp32 mean of those
+ *   neighbours, summed in row order (dy, then dx, from -1).  Rects are disjoint, so bilinear lookups never mix charts.
+ * All return non-zero with tf_last_error() before any launch on a NULL pointer, 0 or >= 2^31 vertices or triangles, 3 T >= 2^31,
+ * R or padding out of range, or a workspace smaller than the sizes call gives. */
+TF_API int tf_uv_atlas_sizes(int64_t n_vertices, int64_t n_triangles, int32_t resolution, size_t* workspace_bytes);
+TF_API int tf_uv_atlas(const float* vertices, int64_t n_vertices, const int32_t* triangles, int64_t n_triangles, int32_t resolution,
+                       int32_t padding, void* workspace, size_t workspace_bytes, int32_t* out_chart, int32_t* out_triangles,
+                       int64_t* out_vertex_index, float* out_xy, int32_t* out_texel_tri, int32_t* out_rects, double* out_scale,
+                       int64_t* out_n_vertices, int64_t* out_n_charts, int32_t* out_rounds, int32_t* out_steps, tf_stream_t stream);
+TF_API int tf_uv_texel_points(const float* vertices, const int32_t* triangles, const float* xy, const int32_t* texel_tri,
+                              int32_t resolution, const int64_t* texels, int64_t n, float* out_points, tf_stream_t stream);
+TF_API int tf_uv_fill_sizes(int32_t resolution, int32_t channels, size_t* workspace_bytes);
+TF_API int tf_uv_fill(const float* values, const int64_t* texels, int64_t n, int32_t channels, const int32_t* texel_tri,
+                      const int32_t* chart, const int32_t* rects, int32_t resolution, int32_t padding, void* workspace,
+                      size_t workspace_bytes, float* out_texture, tf_stream_t stream);
+
 /* ---- material-stage Monte-Carlo integral (network/fields.py:1075-1335) -----------------
  * tf_mc_directions builds one direction set per surface point and its pdf:
  *   mode 0: flow samples in the half-vector parametrisation (fields.py:1085-1108,1164-1188)

@@ -2,59 +2,23 @@
 // Lock-free union-find in the style of ECL-CC (Jaiganesh and Burtscher, "A High-Performance Connected Components
 // Implementation for GPUs", HPDC 2018): init, link (a thread per triangle), flatten, count.
 //
-// root[] is the parent array.  Parents only ever decrease and stay inside their tree, so root[v] <= v, with equality exactly
-// for the roots:
-//   - a hook sets a root's parent to a smaller root with atomicCAS(&root[hi], hi, lo), so a vertex stops being a root once
-//     and never becomes one again;
-//   - path halving lowers a non-root's parent to what it read as its grandparent with atomicMin: smaller than the vertex, in
-//     its tree, and not its descendant (descendants have larger indices), so the write cannot form a cycle or split a tree.
-//     A plain store would not do: a halving store that read the parent before another thread flattened the vertex could land
-//     after it and raise the parent again, leaving a vertex of the flattened output pointing at an ancestor below its root.
-// Trees only ever merge, every finished union leaves both ends in one tree, and each tree's root is its smallest vertex.  So
-// concurrent halving needs no locks, and the final root of a component is its minimum vertex index whatever the scheduling.
-// Parents are read through relaxed device-scope atomic references: a plain load may be served from a stale L1 line written by
-// another SM.
+// root[] is the parent array; the find / unite rules and why they need no locks are in union_find.cuh.  The final root of a
+// component is its minimum vertex index whatever the scheduling.
 //
 // HBM per vertex: init writes root and tri_count (8 B), flatten reads and writes root (8 B); per triangle: link reads 12 B of
 // indices plus the parent loads of two unions, count reads 4 B of index and one gathered root (then one atomic per warp and
 // component).  The parent array is 4 B per vertex (128 MB at 32 M vertices), so the finds of the link pass hit L2 when it fits.
 #include <algorithm>
-#include <cuda/atomic>
 #include "common.cuh"
+#include "union_find.cuh"
 
 namespace {
 
 constexpr unsigned FULL = 0xffffffffu;
 
-using ParentRef = cuda::atomic_ref<int32_t, cuda::thread_scope_device>;
-
-__device__ __forceinline__ int32_t parent_of(int32_t* root, int32_t v) { return ParentRef(root[v]).load(cuda::memory_order_relaxed); }
-__device__ __forceinline__ void set_parent(int32_t* root, int32_t v, int32_t p) { ParentRef(root[v]).store(p, cuda::memory_order_relaxed); }
-
-// the root of v's tree; on the way every other vertex is pointed at its grandparent (path halving)
-__device__ __forceinline__ int32_t find(int32_t* root, int32_t v) {
-    int32_t p = parent_of(root, v);
-    while (p != v) {
-        const int32_t gp = parent_of(root, p);
-        if (gp == p) return p;
-        atomicMin(root + v, gp);
-        v = gp;
-        p = parent_of(root, v);
-    }
-    return v;
-}
-
-// hook the larger root under the smaller; a failed CAS returns the new parent of the vertex that is no longer a root, and the
-// loop carries on from there
-__device__ __forceinline__ void unite(int32_t* root, int32_t a, int32_t b) {
-    int32_t ra = find(root, a), rb = find(root, b);
-    while (ra != rb) {
-        const int32_t lo = min(ra, rb), hi = max(ra, rb);
-        const int32_t old = atomicCAS(root + hi, hi, lo);
-        if (old == hi) return;
-        if (ra == hi) ra = old; else rb = old;
-    }
-}
+using tf_uf::find;
+using tf_uf::set_parent;
+using tf_uf::unite;
 
 __global__ void __launch_bounds__(256) mesh_cc_init(int32_t* __restrict__ root, int32_t* __restrict__ tri_count, int64_t n_vertices) {
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;

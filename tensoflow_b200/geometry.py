@@ -1,9 +1,11 @@
 """Mesh geometry on the GPU: evaluation against a reference mesh (area-weighted surface samples, `tf_mesh_sample_surface`, and
 exact point-to-mesh distances on the BVH, `tf_bvh_closest_point` through mc_ops.RayTracer, reduced in fp64), connected
-components (`tf_mesh_components`) and quadric-error simplification (`tf_mesh_simplify`).  There is no CPU path."""
+components (`tf_mesh_components`), quadric-error simplification (`tf_mesh_simplify`), and UV atlases with texture baking
+(`tf_uv_atlas`, `tf_uv_texel_points`, `tf_uv_fill`).  There is no CPU path."""
 from __future__ import annotations
 
 import ctypes
+from dataclasses import dataclass
 
 import torch
 
@@ -167,6 +169,147 @@ def _simplify(vertices, triangles, target_triangles, max_error):
                                    ctypes.byref(n_v), ctypes.byref(n_t), ctypes.byref(rounds), stream_ptr()), "tf_mesh_simplify")
         del ws
         return out_v[:n_v.value].clone(), out_t[:n_t.value].clone(), rounds.value
+
+
+@dataclass
+class UVAtlas:
+    """A UV atlas from `uv_atlas`, on the mesh's device.  Vertices are split along chart seams: output vertex i is the pair
+    (vertex_index[i], chart) and sits at vertices[i] = the input position.
+
+      vertices [V',3] fp32, triangles [T,3] int32 (input order), uv [V',2] fp32 in [0,1], vertex_index [V'] int64
+      xy [V',2] fp32        texel-space coordinates in [0, R]: uv = xy / R; texture row j spans v in [j/R, (j+1)/R], column i
+                            spans u in [i/R, (i+1)/R] (row 0 at v = 0: image writers that put row 0 at the top flip v)
+      chart [T] int32       chart of each triangle, numbered by its smallest triangle
+      texel_tri [R,R] int32 the triangle owning each texel (its centre lies inside it), -1 for none; [j, i] is row j, column i
+      rects [C,4] int32     each chart's rectangle (x0, y0, w, h) in texels, padding included; rectangles are disjoint
+      scale                 texels per world unit, the same for every chart
+      resolution, padding, rounds (conflict rounds), steps (density trials)"""
+    vertices: torch.Tensor
+    triangles: torch.Tensor
+    uv: torch.Tensor
+    xy: torch.Tensor
+    vertex_index: torch.Tensor
+    chart: torch.Tensor
+    texel_tri: torch.Tensor
+    rects: torch.Tensor
+    scale: float
+    resolution: int
+    padding: int
+    rounds: int
+    steps: int
+
+
+def uv_atlas(vertices, triangles, resolution: int = 2048, padding: int = 2) -> UVAtlas:
+    """A UV atlas of box-projection charts on the GPU (tf_uv_atlas; rules in include/tensoflow_b200.h) -> UVAtlas.
+
+    Each triangle takes the axis direction (+-x, +-y, +-z) of its largest normal component, smoothed over edge neighbours in 4
+    passes among the directions within 60 degrees of its normal; a chart is an edge-connected set of triangles of one
+    direction, projected orthographically along it at one density for all charts (so stretch is at most 2 in one direction).
+    Charts are packed as rectangles with `padding` texels on every side into an R x R atlas, next-fit decreasing height, at
+    the largest density a bisection finds to fit.  A chart whose projection folds over itself (a texel centre covered twice)
+    is split into single triangles and the atlas is laid out again, until every texel centre has at most one triangle.  The
+    result is deterministic (bit-equal to oracle/torch_oracle_atlas.py).
+
+    Raises ValueError for resolution outside [16, 16384] or padding outside [1, 16], and RuntimeError on CPU tensors, shapes
+    other than [V,3] / [T,3], an empty mesh, non-integer triangles, 2^31 or more vertices or triangles, a triangle index out of
+    range, non-finite vertices or a zero total area (one host read), all before any launch; RuntimeError when the charts do
+    not fit in the atlas at any density (more charts than R x R holds)."""
+    what = "uv_atlas"
+    if isinstance(resolution, bool) or int(resolution) != resolution or not 16 <= int(resolution) <= 16384:
+        raise ValueError(f"{what}: resolution must be an integer in [16, 16384], got {resolution}")
+    if isinstance(padding, bool) or int(padding) != padding or not 1 <= int(padding) <= 16:
+        raise ValueError(f"{what}: padding must be an integer in [1, 16], got {padding}")
+    R, pad = int(resolution), int(padding)
+    if torch.is_tensor(triangles) and (triangles.is_floating_point() or triangles.is_complex() or triangles.dtype == torch.bool):
+        raise RuntimeError(f"{what} needs integer triangles, got {triangles.dtype}")
+    for x, name in ((vertices, "vertices"), (triangles, "triangles")):
+        if torch.is_tensor(x) and x.dim() == 2 and x.shape[0] >= 2 ** 31:
+            raise RuntimeError(f"{what}: {x.shape[0]} {name}, the kernel indexes fewer than 2^31")
+    if torch.is_tensor(triangles) and triangles.dim() == 2 and 3 * triangles.shape[0] >= 2 ** 31:
+        raise RuntimeError(f"{what}: {triangles.shape[0]} triangles, the sorts need 3 T < 2^31")
+    v, t = _mesh(vertices, triangles, what)
+    V, T = v.shape[0], t.shape[0]
+    lib = _lib.load()
+    dev = v.device
+    with torch.cuda.device(dev):
+        flat = triangles.detach().reshape(-1)
+        lo, hi = flat.min().to(torch.int64), flat.max().to(torch.int64)
+        finite = torch.isfinite(v).all()
+        area = 0.5 * _face_cross(v, t.clamp(0, V - 1)).norm(dim=-1).sum()
+        lo, hi, finite, area = torch.stack([lo.double(), hi.double(), finite.double(), area]).tolist()   # the one host read
+        if lo < 0 or hi >= V:
+            raise RuntimeError(f"{what}: triangle index out of range (indices span [{int(lo)}, {int(hi)}], {V} vertices)")
+        if not finite:
+            raise RuntimeError(f"{what}: non-finite vertex coordinates")
+        if not area > 0:
+            raise RuntimeError(f"{what}: total area {area} is not positive")
+        ws_bytes = ctypes.c_size_t()
+        check(lib.tf_uv_atlas_sizes(V, T, R, ctypes.byref(ws_bytes)), "tf_uv_atlas_sizes")
+        ws = torch.empty(ws_bytes.value, device=dev, dtype=torch.uint8)
+        chart = torch.empty(T, device=dev, dtype=torch.int32)
+        tri = torch.empty(T, 3, device=dev, dtype=torch.int32)
+        vidx = torch.empty(3 * T, device=dev, dtype=torch.int64)
+        xy = torch.empty(3 * T, 2, device=dev, dtype=torch.float32)
+        texel_tri = torch.empty(R, R, device=dev, dtype=torch.int32)
+        rects = torch.empty(T, 4, device=dev, dtype=torch.int32)
+        scale, n_v, n_c = ctypes.c_double(), ctypes.c_int64(), ctypes.c_int64()
+        rounds, steps = ctypes.c_int32(), ctypes.c_int32()
+        check(lib.tf_uv_atlas(ptr(v), V, ptr(t), T, R, pad, ptr(ws), ws_bytes.value, ptr(chart), ptr(tri), ptr(vidx), ptr(xy),
+                              ptr(texel_tri), ptr(rects), ctypes.byref(scale), ctypes.byref(n_v), ctypes.byref(n_c),
+                              ctypes.byref(rounds), ctypes.byref(steps), stream_ptr()), "tf_uv_atlas")
+        del ws
+        vidx, xy = vidx[:n_v.value].clone(), xy[:n_v.value].clone()
+        return UVAtlas(vertices=v[vidx], triangles=tri, uv=xy / R, xy=xy, vertex_index=vidx, chart=chart, texel_tri=texel_tri,
+                       rects=rects[:n_c.value].clone(), scale=scale.value, resolution=R, padding=pad, rounds=rounds.value,
+                       steps=steps.value)
+
+
+def texel_points(atlas: UVAtlas):
+    """-> (texels [n] int64, the covered texels j * R + i in row order, and points [n,3] fp32 on their owning triangles): the
+    point at the barycentric coordinates of each texel centre, evaluated in fp64 and rounded once (tf_uv_texel_points).  One
+    host read (the count)."""
+    R = atlas.resolution
+    with torch.cuda.device(atlas.texel_tri.device):
+        texels = torch.nonzero(atlas.texel_tri.reshape(-1) >= 0)[:, 0]
+        pts = torch.empty(texels.shape[0], 3, device=texels.device, dtype=torch.float32)
+        check(_lib.load().tf_uv_texel_points(ptr(atlas.vertices), ptr(atlas.triangles), ptr(atlas.xy), ptr(atlas.texel_tri), R,
+                                             ptr(texels), texels.shape[0], ptr(pts), stream_ptr()), "tf_uv_texel_points")
+    return texels, pts
+
+
+def bake_texture(atlas: UVAtlas, fn, channels: int, chunk: int = 2 ** 20):
+    """Bake fn over the atlas -> (texture [R,R,channels] fp32, mask [R,R] bool of the texels covered before dilation).
+
+    fn(points [n,3] fp32 CUDA) -> [n, channels] runs on the texel points of `texel_points`, at most `chunk` at a time.  The
+    values are scattered to their texels, then `atlas.padding` dilation passes fill each empty texel of a chart's rectangle
+    that touches filled ones with the mean of its filled 8-neighbours of that chart (tf_uv_fill), so bilinear lookups inside a
+    chart never read another chart.  Row j of the texture spans v in [j/R, (j+1)/R] (see UVAtlas).  Raises RuntimeError when
+    fn returns another shape or non-finite values, and ValueError for channels < 1 or chunk < 1."""
+    if isinstance(channels, bool) or int(channels) != channels or int(channels) < 1:
+        raise ValueError(f"bake_texture: channels must be an integer >= 1, got {channels}")
+    if int(chunk) < 1:
+        raise ValueError(f"bake_texture: chunk must be >= 1, got {chunk}")
+    C, R = int(channels), atlas.resolution
+    lib = _lib.load()
+    texels, pts = texel_points(atlas)
+    dev = pts.device
+    with torch.cuda.device(dev):
+        values = torch.empty(pts.shape[0], C, device=dev, dtype=torch.float32)
+        for s in range(0, pts.shape[0], int(chunk)):
+            out = fn(pts[s:s + int(chunk)])
+            if not torch.is_tensor(out) or tuple(out.shape) != (min(int(chunk), pts.shape[0] - s), C):
+                raise RuntimeError(f"bake_texture: fn must return [n, {C}], got "
+                                   f"{list(out.shape) if torch.is_tensor(out) else type(out).__name__}")
+            values[s:s + out.shape[0]] = out.detach()
+        if not bool(torch.isfinite(values).all()):
+            raise RuntimeError("bake_texture: fn returned a non-finite value")
+        ws_bytes = ctypes.c_size_t()
+        check(lib.tf_uv_fill_sizes(R, C, ctypes.byref(ws_bytes)), "tf_uv_fill_sizes")
+        ws = torch.empty(ws_bytes.value, device=dev, dtype=torch.uint8)
+        tex = torch.empty(R, R, C, device=dev, dtype=torch.float32)
+        check(lib.tf_uv_fill(ptr(values), ptr(texels), texels.shape[0], C, ptr(atlas.texel_tri), ptr(atlas.chart), ptr(atlas.rects),
+                             R, atlas.padding, ptr(ws), ws_bytes.value, ptr(tex), stream_ptr()), "tf_uv_fill")
+        return tex, atlas.texel_tri >= 0
 
 
 def evaluate_mesh(pred_vertices, pred_triangles, gt_vertices, gt_triangles, n_samples: int = 1_000_000,

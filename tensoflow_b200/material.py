@@ -458,6 +458,7 @@ class MaterialRenderer(nn.Module):
         super().__init__()
         self.cfg = {**self.default_cfg, **cfg}
         dev = self.cfg['device']
+        self.vertices, self.triangles = vertices, triangles      # the mesh predict_materials / bake_materials export onto
         self.aabb = torch.tensor(self.cfg['aabb'], device=dev)
         grid = torch.tensor(self.cfg['gridSize'], device=dev)
         self.unit_size = torch.mean((self.aabb[1] - self.aabb[0]) / (grid - 1))
@@ -605,6 +606,39 @@ class MaterialRenderer(nn.Module):
 
     def trace(self, rays_o, rays_d):
         return self.tracer.trace(rays_o, rays_d)
+
+    # ---- material export onto the mesh ------------------------------------------------------------------------------
+    def _materials_at(self, pts, batch_size):
+        """[n,3] -> [n,5] fp32: albedo (3), roughness (sqrt of the predicted roughness squared), metallic"""
+        out = []
+        for i in range(0, pts.shape[0], batch_size):
+            metallic, roughness, albedo = self.shader_network.predict_materials(pts[i:i + batch_size])
+            out.append(torch.cat([albedo, torch.sqrt(roughness), metallic], -1).float())
+        return torch.cat(out, 0) if out else torch.zeros(0, 5, device=pts.device)
+
+    @torch.no_grad()
+    def predict_materials(self, batch_size: int = 8192):
+        """Per-vertex materials of the mesh the renderer was built with -> {'metallic' [V,1], 'roughness' [V,1], 'albedo' [V,3]}
+        on the device, from the material stage at the vertex positions in batches of `batch_size`.  Roughness is reported as
+        sqrt of the network's squared roughness, as `nvs` reports it.  This is the export behind relighting with vertex colours;
+        the reference renderer has a method of this name, but its source is not part of this repository, so whether its return
+        form (keys, shapes, roughness convention) matches this one is unverified."""
+        dev = self.cfg['device']
+        v = torch.as_tensor(self.vertices).to(device=dev, dtype=torch.float32).contiguous()
+        m = self._materials_at(v, int(batch_size))
+        return {'metallic': m[:, 4:5], 'roughness': m[:, 3:4], 'albedo': m[:, 0:3]}
+
+    @torch.no_grad()
+    def bake_materials(self, resolution: int = 2048, padding: int = 2, batch_size: int = 8192):
+        """Materials baked into textures over a UV atlas of the renderer's mesh (geometry.uv_atlas, geometry.bake_texture) ->
+        {'atlas': UVAtlas (split vertices, triangles, uv, ...), 'albedo' [R,R,3], 'roughness' [R,R,1] (sqrt convention, as
+        predict_materials), 'metallic' [R,R,1] fp32, 'mask' [R,R] bool (texels covered before dilation)}.  Texture row j spans
+        v in [j/R, (j+1)/R]."""
+        from .geometry import bake_texture, uv_atlas
+        dev = self.cfg['device']
+        atlas = uv_atlas(torch.as_tensor(self.vertices).to(dev), torch.as_tensor(self.triangles).to(dev), resolution, padding)
+        tex, mask = bake_texture(atlas, lambda p: self._materials_at(p, int(batch_size)), 5)
+        return {'atlas': atlas, 'albedo': tex[..., 0:3], 'roughness': tex[..., 3:4], 'metallic': tex[..., 4:5], 'mask': mask}
 
     def get_train_opt_params(self, learning_rate_xyz, learning_rate_net, learning_rate_env):
         return self.shader_network.get_optparam_groups(learning_rate_xyz, learning_rate_net, learning_rate_env)
